@@ -2,6 +2,7 @@
 """Headline benchmark: train rays/s of the PreSight city-NeRF inner loop (BASELINE.json config 2).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c1] [--fp32] [--strong]
+                    [--dump-outputs DIR]
 
 One step = encode + MLP + sample + composite, forward and backward (update step: proposal nets get gradients),
 plus the gradient all-reduce for N > 1; the optimizer is excluded (SURVEY §8d).  Prints ONE JSON line.
@@ -12,6 +13,7 @@ plus the gradient all-reduce for N > 1; the optimizer is excluded (SURVEY §8d).
             peak; the kernel runs once per ray slice of the final level, concurrently with the field backward
   cpu_baseline  the oracle port of the reference's torch path, timed on this box's host cores on a bounded sample
 `--impl reference` times that CPU path alone (the reference arm of the harness).
+`--dump-outputs DIR` also writes what the last timed step computed (rank 0) as DIR/<name>.npy, see step_results().
 """
 from __future__ import annotations
 
@@ -27,11 +29,16 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
 METRIC = "train_rays_per_s"
 UNIT = "rays/s"
+
+DUMP_RAYS = 4096              # rays sampled from every per-ray output by --dump-outputs
+DUMP_GRAD_ENTRIES = 32768     # entries sampled from every larger parameter gradient
+DUMP_BYTES = 64 << 20
 
 
 # ------------------------------------------------------------------------------------------------ helpers
@@ -186,6 +193,35 @@ def step_loss(model, out, batch):
     for v in loss_dict.values():
         loss = v if loss is None else loss + v
     return loss
+
+
+def step_results(out, loss, model, n_rays: int) -> dict:
+    """What a training step hands its caller, as host float32 / float64 arrays: the loss, the model outputs (weights and
+    euclidean bin edges per sampler level) of a fixed seeded sample of DUMP_RAYS rays, and every parameter gradient (a
+    fixed seeded sample of DUMP_GRAD_ENTRIES entries of a larger one).  The samples depend on the shapes alone, so two
+    builds run with the same arguments write files that compare entry for entry."""
+    g = torch.Generator().manual_seed(0)
+    rows = torch.randperm(n_rays, generator=g)[:DUMP_RAYS].sort().values.to(loss.device)
+    res = {"loss": loss}
+    for k, v in out.items():
+        if k == "weights_list":
+            res.update({f"weights_{i}": w[rows] for i, w in enumerate(v)})
+        elif k == "ray_samples_list":
+            res.update({f"eu_bins_{i}": rs.frustums.eu_bins[rows] for i, rs in enumerate(v)})
+        else:
+            res[k] = v[rows]
+    for name, p in model.named_parameters():
+        if p.grad is None:
+            continue
+        gr = p.grad.reshape(-1)
+        if gr.numel() > DUMP_GRAD_ENTRIES:
+            gr = gr[torch.randint(gr.numel(), (DUMP_GRAD_ENTRIES,), generator=g).to(gr.device)]
+        res[f"grad.{name}"] = gr
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).numpy()
+              for k, v in res.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs would write {total} bytes (limit {DUMP_BYTES})"
+    return arrays
 
 
 # ------------------------------------------------------------------------------------------------ CPU reference arm
@@ -369,7 +405,12 @@ def main() -> None:
     ap.add_argument("--optimizer", default="none", choices=["none", "torch", "fused"],
                     help="also take an Adam step inside the timed step (SURVEY 8f-2; the headline metric excludes it): "
                          "torch.optim.Adam or presight_b200.optim.FusedAdam with PreSight's hyper-parameters")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's loss, sampled outputs and sampled gradients (rank 0) as DIR/<name>.npy, "
+                         "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "c5" or args.steps < 1):
+        ap.error("--dump-outputs needs the training step of the b200 arm (not --impl reference or --config c5) and --steps >= 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -454,7 +495,7 @@ def main() -> None:
     resident = {k: pinned[k].to(dev, non_blocking=True) for k in tensor_keys}
     h2d_bytes = sum(pinned[k].numel() * pinned[k].element_size() for k in tensor_keys)
 
-    def run_step(batch):
+    def run_step(batch, keep=None):
         for p in params:
             p.grad = None
         rb = RayBundle(origins=batch["origins"], directions=batch["directions"],
@@ -467,6 +508,8 @@ def main() -> None:
             sync.finish()
         if optimizer is not None:
             optimizer.step()
+        if keep is not None:
+            keep.update(out=out, loss=loss)
         return loss
 
     def barrier():
@@ -490,11 +533,16 @@ def main() -> None:
     run_step(resident)                               # one more warm-up step, timed on the HOST with an empty launch queue:
     t_host = time.perf_counter() - t_host0          # the Python / launch cost of a step (the GPU must exceed it to stay busy)
     barrier()
+    last_step = {} if args.dump_outputs else None
     ev0.record()
-    for _ in range(args.steps):
-        run_step(resident)
+    for i in range(args.steps):
+        run_step(resident, last_step if i == args.steps - 1 else None)
     ev1.record()
     barrier()
+    dump = None
+    if last_step is not None and rank == 0:          # read before the end-to-end leg replaces the gradients
+        dump = step_results(last_step["out"], last_step["loss"], model, rays_per_rank)
+    last_step = None
     launches = ops.launch_count() - launches0
     probe = ops.PROBE.summary()
     ops.PROBE = None
@@ -669,6 +717,10 @@ def main() -> None:
                                               f"cannot travel to this box), torch CPU fp32, {cores} threads, median of 3 "
                                               f"steps ({med:.2f} s/step)",
                                     "hash_only_points_per_s": cpu_hash_only(cfg)}
+        if dump is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
