@@ -384,6 +384,33 @@ int ps_prop_level_bwd(const ps_prop_net* net, const float* origins, const float*
                       const void* feat_bf16, const float* d_weights, float* dtable, void* stream);
 
 /* ---------------------------------------------------------------------------------------
+ * Density level of the main field, forward only (bf16 parity class): the same kernels as the fused proposal level,
+ * instantiated for the density head of iNGPField (fields/PreSight/ingp_field.py:168-191): base0 [64, L*F] + ReLU, then
+ * row 0 of base1 [80, 64] plus base1.bias[0], trunc_exp, selector.  Pass net->W1 = &base1.weight[0][0] and
+ * net->b1 = &base1.bias[0]; the backward members are ignored.  Supported: hidden 64, L*F <= 48 with F in {1,2,4},
+ * S in {32,64,96,128} (ray mode).  Used to find the threshold depth of eval rays (prior extraction).
+ *   ps_density_level_fwd     origins/dirs [N,3], eu_bins [N,S+1] -> weights [N,S], exactly as ps_prop_level_fwd
+ *   ps_density_level_fwd_ms  routed rows (see the sub-field section below) -> density [P] at each point's own index,
+ *                            exactly as ps_prop_level_fwd_ms
+ */
+int ps_density_level_fwd(const ps_prop_net* net, const float* origins, const float* dirs, const float* eu_bins, int64_t N,
+                         int S, const float* aabb_host, int contract, const float* table, const float* scalings_host,
+                         int L, int F, int log2_T, float* weights, void* stream);
+struct ps_prop_net_dev;
+int ps_density_level_fwd_ms(const struct ps_prop_net_dev* nets_dev, int hidden, const float* x01_sorted,
+                            const uint8_t* sel_sorted, const int32_t* perm, const uint8_t* tile_sf, int64_t rows,
+                            const float* const* tables_dev, const float* scalings_host, int L, int F, int log2_T,
+                            float* density, void* stream);
+
+/* Surface hits of rays at their threshold depth (scripts/extract_priors.py:100-126), one thread per ray:
+ *   points_scaled [N,3] = fmaf(d, depth, o) per component; points_m [N,3] = points_scaled / pose_scale (IEEE division);
+ *   keep [N] u8 = depth / pose_scale <= max_range_m && z_min_m <= points_m.z <= z_max_m, a non-finite bound not applied.
+ * origins / dirs [N,3], depth [N]; pose_scale > 0. */
+int ps_surface_hits(const float* origins, const float* dirs, const float* depth, int64_t N, float pose_scale,
+                    float max_range_m, float z_min_m, float z_max_m, float* points_scaled, float* points_m, uint8_t* keep,
+                    void* stream);
+
+/* ---------------------------------------------------------------------------------------
  * Sub-field routing and the sub-field mode of the fused levels (SURVEY §8 a10).  Replace the nearest-centroid routers
  * fields/PreSight/ingp_field_ms.py:80-126, prop_density_field_ms.py:86-105 (cdist().argmin, then per sub-field a
  * boolean-mask gather, a field call, a masked scatter and a `torch.any` host sync) without any host synchronisation:

@@ -91,6 +91,9 @@ SIGNATURES = {
     "ps_prop_level_feat_stride": [_i, _i],
     "ps_prop_level_fwd": [_p, _p, _p, _p, _i64, _i, _fp, _i, _p, _fp, _i, _i, _i, _p, _p, _p],
     "ps_prop_level_bwd": [_p, _p, _p, _p, _i64, _i, _fp, _i, _fp, _i, _i, _i, _p, _p, _p, _p],
+    "ps_density_level_fwd": [_p, _p, _p, _p, _i64, _i, _fp, _i, _p, _fp, _i, _i, _i, _p, _p],
+    "ps_density_level_fwd_ms": [_p, _i, _p, _p, _p, _p, _i64, _p, _fp, _i, _i, _i, _p, _p],
+    "ps_surface_hits": [_p, _p, _p, _i64, _f, _f, _f, _f, _p, _p, _p, _p],
 }
 _RESTYPES = {"ps_last_error": C.c_char_p, "ps_abi_version": C.c_int, "ps_launch_count": C.c_int64}
 

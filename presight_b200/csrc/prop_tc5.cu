@@ -9,6 +9,18 @@
 // per-thread dot product over the bf16-rounded hidden row; in the backward the input-gradient GEMM, both weight-gradient
 // GEMMs and the hidden bias gradient (a GEMM against a ones tile) run on the tensor core with accumulators resident in
 // TMEM for the whole kernel.  The scatter-add keeps the warp pre-aggregation and x-pair merge of the stand-alone kernel.
+//
+// The forward kernels also serve the density head of the main field (ps_density_level_fwd / _ms: base0 [64, L*F] + ReLU,
+// row 0 of base1, trunc_exp * selector — the same network shape with a wider input), instantiated for hidden 64,
+// F in {1, 2, 4} and the padded input width K0 = 16 / 32 / 48; they write each pair of levels straight into the bf16 X0
+// tile (gather_to_tile).  The proposal instantiations (K0 = 16, F <= 2) keep their register path and compile to the same
+// SASS as before the widening (prop_fwd_kernel<64, 1> up to register numbering).  ptxas -v, sm_100a, CUDA 12.9, forward
+// only, no spills in any of them; registers (ray mode / routed mode) and dynamic shared memory:
+//   F = 1  K0 = 32: 62 / 52 regs     F = 2  K0 = 32: 68 / 72 regs     F = 4  K0 = 16: 92 / 94 regs
+//          K0 = 48: 62 / 52 regs            K0 = 48: 67 / 72 regs            K0 = 32: 92 / 94 regs
+//                                                                            K0 = 48: 96 / 94 regs
+//   shared memory 21.1 KB (K0 = 32) / 27.2 KB (K0 = 48); resident CTAs per SM (registers / shared memory / 64 TMEM
+//   columns): 8 up to 64 registers, 7 up to 72, 5 for the F = 4 kernels.
 #include <cuda_bf16.h>
 #include <stdlib.h>
 
@@ -46,16 +58,18 @@ struct PropArgs {
     const float* d_w;       // [N,S]
 };
 
-template <int H>
+// K0: padded input width of the first layer.  The backward kernels exist for K0 = 16 only; the forward kernels are
+// also instantiated for K0 = 32 / 48 (the main field's density head, ps_density_level_fwd*).
+template <int H, int K0 = kK0>
 struct Smem {
     // tiles used as the M = 128 "X" operand of a weight-gradient GEMM (H1, DZ0) are followed by >= 32 KB - own size
     static constexpr uint32_t h1 = 0;                                  // [128 x H]   (backward)
     static constexpr uint32_t dz0 = h1 + cm_bytes(kRows, H);           // [128 x H]   (backward)
-    static constexpr uint32_t x0 = dz0 + cm_bytes(kRows, H);           // [128 x 16]
-    static constexpr uint32_t dz1 = x0 + cm_bytes(kRows, kK0);         // [128 x 16]  (backward)
+    static constexpr uint32_t x0 = dz0 + cm_bytes(kRows, H);           // [128 x K0]
+    static constexpr uint32_t dz1 = x0 + cm_bytes(kRows, K0);          // [128 x 16]  (backward)
     static constexpr uint32_t ones = dz1 + cm_bytes(kRows, kK0);       // [128 x 16] of 1.0 (backward)
-    static constexpr uint32_t w0 = ones + cm_bytes(kRows, kK0);        // [H x 16]
-    static constexpr uint32_t fl = w0 + cm_bytes(H, kK0);              // float: b0[H] | w1[H] (bf16-rounded) | b1
+    static constexpr uint32_t w0 = ones + cm_bytes(kRows, kK0);        // [H x K0]
+    static constexpr uint32_t fl = w0 + cm_bytes(H, K0);              // float: b0[H] | w1[H] (bf16-rounded) | b1
     static constexpr uint32_t tails = fl + (2 * H + 4) * 4;            // double [4][2]
     static constexpr uint32_t bars = ((tails + 64 + 15) / 16) * 16;
     static constexpr uint32_t used = bars + 32;
@@ -94,11 +108,11 @@ __device__ __forceinline__ RowCtx make_row(const PropArgs& a, int64_t tile, int 
     return c;
 }
 
-template <int H>
+template <int H, int K0 = kK0>
 __device__ __forceinline__ void load_net_raw(const float* W0, const float* b0, const float* W1, const float* b1, int in_dim,
                                              unsigned char* smem, int tid) {
-    using SM = Smem<H>;
-    load_weight_cm(W0, H, in_dim, H, kK0, smem + SM::w0, nullptr, tid, kThreads);
+    using SM = Smem<H, K0>;
+    load_weight_cm(W0, H, in_dim, H, K0, smem + SM::w0, nullptr, tid, kThreads);
     float* fl = reinterpret_cast<float*>(smem + SM::fl);
     for (int i = tid; i < H; i += kThreads) {
         fl[i] = b0 ? __ldg(b0 + i) : 0.f;
@@ -106,9 +120,9 @@ __device__ __forceinline__ void load_net_raw(const float* W0, const float* b0, c
     }
     if (tid == 0) fl[2 * H] = b1 ? __ldg(b1) : 0.f;
 }
-template <int H>
+template <int H, int K0 = kK0>
 __device__ __forceinline__ void load_net(const PropArgs& a, unsigned char* smem, int tid) {
-    load_net_raw<H>(a.W0, a.b0, a.W1, a.b1, a.in_dim, smem, tid);
+    load_net_raw<H, K0>(a.W0, a.b0, a.W1, a.b1, a.in_dim, smem, tid);
 }
 
 // hidden row of this thread: accumulator -> +bias -> ReLU; returns raw = b1 + <h, w1> (fp32 h) and the ReLU mask.
@@ -138,10 +152,64 @@ __device__ __forceinline__ float hidden_row(uint32_t trow, const float* fl, unsi
     return raw;
 }
 
+// Hash features of one point for the density-head instantiations (bit-exact encodings.py:343-384, two levels per loop trip as in the K0 = 16
+// code): every pair of levels goes straight into row r of the bf16 X0 tile as one 2F-wide store (16 / 8 / 4 bytes for
+// F = 4 / 2 / 1), so no K0-entry feature array is held in registers; the padding columns [L*F, K0) are zeroed.
+template <int F, int K0>
+constexpr bool kRegFeat = K0 == kK0 && F <= 2;     // the proposal levels' instantiations: features in registers
+
+template <int F, int K0>
+__device__ __forceinline__ void gather_to_tile(const float* table, const float (&x)[3], const HashParams& hp,
+                                               uint32_t mask_t, unsigned char* X0, int r) {
+    static_assert(K0 % (2 * F) == 0, "level pairs tile the padded width");
+    const int L = hp.L;
+#pragma unroll 1
+    for (int l0 = 0; l0 < L; l0 += 2) {
+        float v[2][8][F];
+        Corner8 cr[2];
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            const int l = min(l0 + j, L - 1);
+            cr[j] = hash_corners(x[0], x[1], x[2], hp.scale[l], mask_t);
+            const float* lt = table + ((size_t)l << hp.log2_T) * F;
+#pragma unroll
+            for (int k = 0; k < 8; ++k) gather_row<F>(lt, cr[j].row[k], v[j][k]);
+        }
+        float pair[2 * F];
+#pragma unroll
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+            for (int f = 0; f < F; ++f) {
+                const float t[8] = {v[j][0][f], v[j][1][f], v[j][2][f], v[j][3][f],
+                                    v[j][4][f], v[j][5][f], v[j][6][f], v[j][7][f]};
+                pair[j * F + f] = l0 + j < L ? trilerp_ref(t, cr[j].ox, cr[j].oy, cr[j].oz) : 0.f;
+            }
+        unsigned char* dst = X0 + cm_off(kRows, r, l0 * F);
+        if constexpr (F == 4) {
+            *reinterpret_cast<uint4*>(dst) = pack8(pair);
+        } else if constexpr (F == 2) {
+            *reinterpret_cast<uint2*>(dst) = make_uint2(pack_bf16x2(pair[0], pair[1]), pack_bf16x2(pair[2], pair[3]));
+        } else {
+            *reinterpret_cast<uint32_t*>(dst) = pack_bf16x2(pair[0], pair[1]);
+        }
+    }
+#pragma unroll 1
+    for (int c = (L + 1) / 2 * 2 * F; c < K0; c += 2 * F) {
+        unsigned char* dst = X0 + cm_off(kRows, r, c);
+        if constexpr (F == 4) {
+            *reinterpret_cast<uint4*>(dst) = make_uint4(0u, 0u, 0u, 0u);
+        } else if constexpr (F == 2) {
+            *reinterpret_cast<uint2*>(dst) = make_uint2(0u, 0u);
+        } else {
+            *reinterpret_cast<uint32_t*>(dst) = 0u;
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------------------------------
-template <int H, int F>
+template <int H, int F, int K0 = kK0>
 __global__ void __launch_bounds__(kThreads) prop_fwd_kernel(PropArgs a) {
-    using SM = Smem<H>;
+    using SM = Smem<H, K0>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     unsigned char* smem = smem_raw - SM::fwd_base;     // forward allocates only [fwd_base, used)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -152,7 +220,7 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_kernel(PropArgs a) {
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + SM::bars + 16);
     constexpr uint32_t kCols = H < 32 ? 32 : H;
 
-    load_net<H>(a, smem, tid);
+    load_net<H, K0>(a, smem, tid);
     if (warp == 0) tmem_alloc(tmem_slot, kCols);
     if (tid == 0) {
         mbar_init(smem_u32(bar_ptr), 1);
@@ -174,48 +242,52 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_kernel(PropArgs a) {
 
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const RowCtx c = make_row(a, tile, tid, rpt, rows_used);
-        // ---- hash gather: bit-exact encodings.py:343-384 -----------------------------------------------------
-        // (two levels per loop trip: 16 independent gathers in flight per thread, compact code)
-        float feat[kK0];
-#pragma unroll
-        for (int i = 0; i < kK0; ++i) feat[i] = 0.f;
-#pragma unroll 1
-        for (int l0 = 0; l0 < L; l0 += 2) {
-            float v[2][8][F];
-            Corner8 cr[2];
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                const int l = min(l0 + j, L - 1);
-                cr[j] = hash_corners(c.x[0], c.x[1], c.x[2], a.hp.scale[l], mask_t);
-                const float* lt = a.table + ((size_t)l << a.hp.log2_T) * F;
-#pragma unroll
-                for (int k = 0; k < 8; ++k) gather_row<F>(lt, cr[j].row[k], v[j][k]);
-            }
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                if (l0 + j < L) {
-#pragma unroll
-                    for (int f = 0; f < F; ++f) {
-                        const float t[8] = {v[j][0][f], v[j][1][f], v[j][2][f], v[j][3][f],
-                                            v[j][4][f], v[j][5][f], v[j][6][f], v[j][7][f]};
-                        const float val = trilerp_ref(t, cr[j].ox, cr[j].oy, cr[j].oz);
-                        // feat[(l0 + j) * F + f] with a compile-time register index
-#pragma unroll
-                        for (int i = 0; i < kK0; ++i)
-                            if (i == (l0 + j) * F + f) feat[i] = val;
+        if constexpr (kRegFeat<F, K0>) {
+            // ---- hash gather: bit-exact encodings.py:343-384 -----------------------------------------------------
+            // (two levels per loop trip: 16 independent gathers in flight per thread, compact code)
+            float feat[kK0];
+    #pragma unroll
+            for (int i = 0; i < kK0; ++i) feat[i] = 0.f;
+    #pragma unroll 1
+            for (int l0 = 0; l0 < L; l0 += 2) {
+                float v[2][8][F];
+                Corner8 cr[2];
+    #pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    const int l = min(l0 + j, L - 1);
+                    cr[j] = hash_corners(c.x[0], c.x[1], c.x[2], a.hp.scale[l], mask_t);
+                    const float* lt = a.table + ((size_t)l << a.hp.log2_T) * F;
+    #pragma unroll
+                    for (int k = 0; k < 8; ++k) gather_row<F>(lt, cr[j].row[k], v[j][k]);
+                }
+    #pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    if (l0 + j < L) {
+    #pragma unroll
+                        for (int f = 0; f < F; ++f) {
+                            const float t[8] = {v[j][0][f], v[j][1][f], v[j][2][f], v[j][3][f],
+                                                v[j][4][f], v[j][5][f], v[j][6][f], v[j][7][f]};
+                            const float val = trilerp_ref(t, cr[j].ox, cr[j].oy, cr[j].oz);
+                            // feat[(l0 + j) * F + f] with a compile-time register index
+    #pragma unroll
+                            for (int i = 0; i < kK0; ++i)
+                                if (i == (l0 + j) * F + f) feat[i] = val;
+                        }
                     }
                 }
             }
-        }
-        {
-            const uint4 lo = pack8(feat), hi = pack8(feat + 8);
-            *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 0)) = lo;
-            *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 8)) = hi;
-            if (a.feat && c.valid) {
-                uint4* dst = reinterpret_cast<uint4*>(a.feat + c.p * a.feat_stride);
-                dst[0] = lo;
-                if (a.feat_stride > 8) dst[1] = hi;
+            {
+                const uint4 lo = pack8(feat), hi = pack8(feat + 8);
+                *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 0)) = lo;
+                *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 8)) = hi;
+                if (a.feat && c.valid) {
+                    uint4* dst = reinterpret_cast<uint4*>(a.feat + c.p * a.feat_stride);
+                    dst[0] = lo;
+                    if (a.feat_stride > 8) dst[1] = hi;
+                }
             }
+        } else {
+            gather_to_tile<F, K0>(a.table, c.x, a.hp, mask_t, X0, tid);
         }
         fence_async_smem();
         fence_before();
@@ -223,7 +295,7 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_kernel(PropArgs a) {
         if (warp_u == 0) {
             if (elect_one()) {
                 fence_after();
-                gemm_kk(tmem, smem_u32(X0), kRows, smem_u32(smem + SM::w0), H, H, kK0, false);
+                gemm_kk(tmem, smem_u32(X0), kRows, smem_u32(smem + SM::w0), H, H, K0, false);
                 umma_commit(bar);
             }
             __syncwarp();
@@ -465,15 +537,26 @@ __global__ void __launch_bounds__(kThreads) prop_bwd_kernel(PropArgs a) {
     if (warp == 0) tmem_dealloc(tmem, TM::alloc);
 }
 
-template <int H, int F>
-static int launch(const PropArgs& a, bool bwd, cudaStream_t stream) {
-    using SM = Smem<H>;
+// kHasBwd<H, F, K0>: a backward kernel exists (K0 = 16, F <= 2); the other instantiations are forward only, and
+// referencing prop_bwd_kernel for them would instantiate a backward nobody calls.
+template <int F, int K0>
+constexpr bool kHasBwd = K0 == kK0 && F <= 2;
+
+template <int H, int F, int K0 = kK0>
+static int launch(const PropArgs& a, bool bwd, cudaStream_t stream, const char* what_fwd = "prop_level_fwd") {
+    using SM = Smem<H, K0>;
+    const void* fwd_kernel = reinterpret_cast<const void*>(prop_fwd_kernel<H, F, K0>);
+    const void* kernel = fwd_kernel;
+    if constexpr (kHasBwd<F, K0>) {
+        if (bwd) kernel = reinterpret_cast<const void*>(prop_bwd_kernel<H, F>);
+    } else {
+        bwd = false;
+    }
     const size_t smem = bwd ? SM::bwd_total : SM::fwd_total;
     static int ctas_fwd = 0, ctas_bwd = 0;
     int& ctas = bwd ? ctas_bwd : ctas_fwd;
     if (ctas == 0) {
-        cudaError_t e = bwd ? cudaFuncSetAttribute(prop_bwd_kernel<H, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                            : cudaFuncSetAttribute(prop_fwd_kernel<H, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) {
             set_error("prop_level: cannot reserve %zu bytes of shared memory", smem);
             return 2;
@@ -482,7 +565,7 @@ static int launch(const PropArgs& a, bool bwd, cudaStream_t stream) {
         // memory (it cannot know the column count), so the limit is derived here: registers, shared memory (+1 KB
         // reserved per CTA), tensor-memory columns, and a cap of 8 (the hardware blocks in tcgen05.alloc otherwise).
         cudaFuncAttributes fa{};
-        e = bwd ? cudaFuncGetAttributes(&fa, prop_bwd_kernel<H, F>) : cudaFuncGetAttributes(&fa, prop_fwd_kernel<H, F>);
+        e = cudaFuncGetAttributes(&fa, kernel);
         const int regs = (e == cudaSuccess && fa.numRegs > 0) ? fa.numRegs : 128;
         const int regs_alloc = ((regs + 7) / 8) * 8;
         const int by_regs = 65536 / (regs_alloc * kThreads);
@@ -500,18 +583,21 @@ static int launch(const PropArgs& a, bool bwd, cudaStream_t stream) {
             if (c >= 1 && c < ctas) ctas = c;
         }
         if (getenv("PS_DEBUG"))
-            fprintf(stderr, "[prop_level %s H=%d F=%d] smem %zu occ %d (%s) by_tmem %d -> %d CTAs/SM\n", bwd ? "bwd" : "fwd", H,
-                    F, smem, occ, cudaGetErrorString(e), by_tmem, ctas);
+            fprintf(stderr, "[prop_level %s H=%d F=%d K0=%d] smem %zu occ %d (%s) by_tmem %d -> %d CTAs/SM\n",
+                    bwd ? "bwd" : "fwd", H, F, K0, smem, occ, cudaGetErrorString(e), by_tmem, ctas);
     }
     const int rpt = kRows / a.S;
     const int64_t ntiles = (a.N + rpt - 1) / rpt;
     const int64_t cap = (int64_t)kNumSMs * ctas;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
-    if (bwd)
-        prop_bwd_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
-    else
-        prop_fwd_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
-    return check_launch(bwd ? "prop_level_bwd" : "prop_level_fwd");
+    if constexpr (kHasBwd<F, K0>) {
+        if (bwd) {
+            prop_bwd_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
+            return check_launch("prop_level_bwd");
+        }
+    }
+    prop_fwd_kernel<H, F, K0><<<grid, kThreads, smem, stream>>>(a);
+    return check_launch(what_fwd);
 }
 
 static int dispatch(const PropArgs& a, int H, bool bwd, cudaStream_t s) {
@@ -555,9 +641,9 @@ struct PropMsArgs {
     const float* d_density;     // [P]
 };
 
-template <int H, int F>
+template <int H, int F, int K0 = kK0>
 __global__ void __launch_bounds__(kThreads) prop_fwd_ms_kernel(PropMsArgs a) {
-    using SM = Smem<H>;
+    using SM = Smem<H, K0>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     unsigned char* smem = smem_raw - SM::fwd_base;
     const int tid = threadIdx.x, warp = tid >> 5;
@@ -592,7 +678,7 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_ms_kernel(PropMsArgs a) {
         if (sf != cur) {
             __syncthreads();                                    // everybody is done with the previous network's constants
             const PropNetDev n = a.nets[sf];
-            load_net_raw<H>(n.W0, n.b0, n.W1, n.b1, a.in_dim, smem, tid);
+            load_net_raw<H, K0>(n.W0, n.b0, n.W1, n.b1, a.in_dim, smem, tid);
             cur = sf;                                           // (published by the barrier in front of the MMA below)
         }
         const int64_t i = tile * kRows + tid;
@@ -602,45 +688,49 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_ms_kernel(PropMsArgs a) {
                             valid ? __ldg(a.x01s + 3 * i + 2) : 0.f};
         const bool inside = valid && a.sels[i] != 0;
         const float* table = a.tables[sf];
-        float feat[kK0];
-#pragma unroll
-        for (int k = 0; k < kK0; ++k) feat[k] = 0.f;
-#pragma unroll 1
-        for (int l0 = 0; l0 < L; l0 += 2) {
-            float v[2][8][F];
-            Corner8 cr[2];
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                const int l = min(l0 + j, L - 1);
-                cr[j] = hash_corners(x[0], x[1], x[2], a.hp.scale[l], mask_t);
-                const float* lt = table + ((size_t)l << a.hp.log2_T) * F;
-#pragma unroll
-                for (int k = 0; k < 8; ++k) gather_row<F>(lt, cr[j].row[k], v[j][k]);
-            }
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                if (l0 + j < L) {
-#pragma unroll
-                    for (int f = 0; f < F; ++f) {
-                        const float t[8] = {v[j][0][f], v[j][1][f], v[j][2][f], v[j][3][f],
-                                            v[j][4][f], v[j][5][f], v[j][6][f], v[j][7][f]};
-                        const float val = trilerp_ref(t, cr[j].ox, cr[j].oy, cr[j].oz);
-#pragma unroll
-                        for (int k = 0; k < kK0; ++k)
-                            if (k == (l0 + j) * F + f) feat[k] = val;
+        if constexpr (kRegFeat<F, K0>) {
+            float feat[kK0];
+    #pragma unroll
+            for (int k = 0; k < kK0; ++k) feat[k] = 0.f;
+    #pragma unroll 1
+            for (int l0 = 0; l0 < L; l0 += 2) {
+                float v[2][8][F];
+                Corner8 cr[2];
+    #pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    const int l = min(l0 + j, L - 1);
+                    cr[j] = hash_corners(x[0], x[1], x[2], a.hp.scale[l], mask_t);
+                    const float* lt = table + ((size_t)l << a.hp.log2_T) * F;
+    #pragma unroll
+                    for (int k = 0; k < 8; ++k) gather_row<F>(lt, cr[j].row[k], v[j][k]);
+                }
+    #pragma unroll
+                for (int j = 0; j < 2; ++j) {
+                    if (l0 + j < L) {
+    #pragma unroll
+                        for (int f = 0; f < F; ++f) {
+                            const float t[8] = {v[j][0][f], v[j][1][f], v[j][2][f], v[j][3][f],
+                                                v[j][4][f], v[j][5][f], v[j][6][f], v[j][7][f]};
+                            const float val = trilerp_ref(t, cr[j].ox, cr[j].oy, cr[j].oz);
+    #pragma unroll
+                            for (int k = 0; k < kK0; ++k)
+                                if (k == (l0 + j) * F + f) feat[k] = val;
+                        }
                     }
                 }
             }
-        }
-        {
-            const uint4 lo = pack8(feat), hi = pack8(feat + 8);
-            *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 0)) = lo;
-            *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 8)) = hi;
-            if (a.feat) {
-                uint4* dst = reinterpret_cast<uint4*>(a.feat + i * a.feat_stride);
-                dst[0] = lo;
-                if (a.feat_stride > 8) dst[1] = hi;
+            {
+                const uint4 lo = pack8(feat), hi = pack8(feat + 8);
+                *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 0)) = lo;
+                *reinterpret_cast<uint4*>(X0 + cm_off(kRows, tid, 8)) = hi;
+                if (a.feat) {
+                    uint4* dst = reinterpret_cast<uint4*>(a.feat + i * a.feat_stride);
+                    dst[0] = lo;
+                    if (a.feat_stride > 8) dst[1] = hi;
+                }
             }
+        } else {
+            gather_to_tile<F, K0>(table, x, a.hp, mask_t, X0, tid);
         }
         fence_async_smem();
         fence_before();
@@ -648,7 +738,7 @@ __global__ void __launch_bounds__(kThreads) prop_fwd_ms_kernel(PropMsArgs a) {
         if (warp_u == 0) {
             if (elect_one()) {
                 fence_after();
-                gemm_kk(tmem, smem_u32(X0), kRows, smem_u32(smem + SM::w0), H, H, kK0, false);
+                gemm_kk(tmem, smem_u32(X0), kRows, smem_u32(smem + SM::w0), H, H, K0, false);
                 umma_commit(bar);
             }
             __syncwarp();
@@ -849,15 +939,20 @@ __global__ void __launch_bounds__(kThreads) prop_bwd_ms_kernel(PropMsArgs a) {
     if (warp == 0) tmem_dealloc(tmem, TM::alloc);
 }
 
-template <int H, int F>
-static int launch_ms(const PropMsArgs& a, bool bwd, cudaStream_t stream) {
-    using SM = Smem<H>;
+template <int H, int F, int K0 = kK0>
+static int launch_ms(const PropMsArgs& a, bool bwd, cudaStream_t stream, const char* what_fwd = "prop_level_fwd_ms") {
+    using SM = Smem<H, K0>;
+    const void* kernel = reinterpret_cast<const void*>(prop_fwd_ms_kernel<H, F, K0>);
+    if constexpr (kHasBwd<F, K0>) {
+        if (bwd) kernel = reinterpret_cast<const void*>(prop_bwd_ms_kernel<H, F>);
+    } else {
+        bwd = false;
+    }
     const size_t smem = bwd ? SM::bwd_total : SM::fwd_total;
     static bool conf_f = false, conf_b = false;
     bool& conf = bwd ? conf_b : conf_f;
     if (!conf) {
-        cudaError_t e = bwd ? cudaFuncSetAttribute(prop_bwd_ms_kernel<H, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                            : cudaFuncSetAttribute(prop_fwd_ms_kernel<H, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) {
             set_error("prop_level_ms: cannot reserve %zu bytes of shared memory", smem);
             return 2;
@@ -868,11 +963,28 @@ static int launch_ms(const PropMsArgs& a, bool bwd, cudaStream_t stream) {
     const int64_t ntiles = a.rows / kRows;
     const int64_t cap = (int64_t)kNumSMs * ctas;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
-    if (bwd)
-        prop_bwd_ms_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
-    else
-        prop_fwd_ms_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
-    return check_launch(bwd ? "prop_level_bwd_ms" : "prop_level_fwd_ms");
+    if constexpr (kHasBwd<F, K0>) {
+        if (bwd) {
+            prop_bwd_ms_kernel<H, F><<<grid, kThreads, smem, stream>>>(a);
+            return check_launch("prop_level_bwd_ms");
+        }
+    }
+    prop_fwd_ms_kernel<H, F, K0><<<grid, kThreads, smem, stream>>>(a);
+    return check_launch(what_fwd);
+}
+
+// Density head of the main field (ps_density_level_fwd*): hidden width 64, F in {1, 2, 4}, K0 = L*F rounded up to 16.
+template <int F>
+static int dispatch_density_f(const PropArgs* a, const PropMsArgs* m, int in_dim, cudaStream_t s) {
+    const int k0 = (in_dim + 15) / 16 * 16;
+    if (k0 == 16) return a ? launch<64, F, 16>(*a, false, s, "density_level_fwd") : launch_ms<64, F, 16>(*m, false, s, "density_level_fwd_ms");
+    if (k0 == 32) return a ? launch<64, F, 32>(*a, false, s, "density_level_fwd") : launch_ms<64, F, 32>(*m, false, s, "density_level_fwd_ms");
+    return a ? launch<64, F, 48>(*a, false, s, "density_level_fwd") : launch_ms<64, F, 48>(*m, false, s, "density_level_fwd_ms");
+}
+static int dispatch_density(const PropArgs* a, const PropMsArgs* m, int F, int in_dim, cudaStream_t s) {
+    if (F == 1) return dispatch_density_f<1>(a, m, in_dim, s);
+    if (F == 2) return dispatch_density_f<2>(a, m, in_dim, s);
+    return dispatch_density_f<4>(a, m, in_dim, s);
 }
 
 static int dispatch_ms(const PropMsArgs& a, int H, bool bwd, cudaStream_t s) {
@@ -884,13 +996,25 @@ static int dispatch_ms(const PropMsArgs& a, int H, bool bwd, cudaStream_t s) {
     return 3;
 }
 
-static int fill(PropArgs& a, const ps_prop_net* net, const float* origins, const float* dirs, const float* eu_bins, int64_t N,
-                int S, const float* aabb_host, int contract, const float* scalings_host, int L, int F, int log2_T,
-                const char* what) {
-    PS_REQUIRE(net && net->W0 && net->W1, "%s: network is null", what);
-    PS_REQUIRE(net->hidden == 16 || net->hidden == 64, "%s: hidden width %d not in {16, 64}", what, net->hidden);
+// density = true: the main field's density head (ps_density_level_fwd*): hidden 64, F in {1, 2, 4}, L*F <= 48
+static int check_shape(int hidden, int L, int F, bool density, const char* what) {
+    if (density) {
+        PS_REQUIRE(hidden == 64, "%s: hidden width %d is not 64", what, hidden);
+        PS_REQUIRE(F == 1 || F == 2 || F == 4, "%s: features_per_level %d not in {1,2,4}", what, F);
+        PS_REQUIRE(L >= 1 && L * F <= 48 && L <= PS_MAX_LEVELS, "%s: L*F = %d exceeds %d", what, L * F, 48);
+        return 0;
+    }
+    PS_REQUIRE(hidden == 16 || hidden == 64, "%s: hidden width %d not in {16, 64}", what, hidden);
     PS_REQUIRE(F == 1 || F == 2, "%s: features_per_level %d not in {1,2}", what, F);
     PS_REQUIRE(L >= 1 && L * F <= kK0 && L <= PS_MAX_LEVELS, "%s: L*F = %d exceeds %d", what, L * F, kK0);
+    return 0;
+}
+
+static int fill(PropArgs& a, const ps_prop_net* net, const float* origins, const float* dirs, const float* eu_bins, int64_t N,
+                int S, const float* aabb_host, int contract, const float* scalings_host, int L, int F, int log2_T,
+                const char* what, bool density = false) {
+    PS_REQUIRE(net && net->W0 && net->W1, "%s: network is null", what);
+    if (int e = check_shape(net->hidden, L, F, density, what)) return e;
     PS_REQUIRE(log2_T >= 1 && log2_T <= 31, "%s: log2_hashmap_size %d out of range", what, log2_T);
     PS_REQUIRE(S >= 32 && S <= 128 && S % 32 == 0, "%s: samples per ray %d must be 32, 64, 96 or 128", what, S);
     PS_REQUIRE(N > 0 && N * (int64_t)S < (1ll << 31), "%s: too many points", what);
@@ -947,11 +1071,9 @@ static_assert(sizeof(ps_prop_net_dev) == sizeof(ps::ptc5::PropNetDev), "ps_prop_
 
 static int fill_ms(PropMsArgs& a, const ps_prop_net_dev* nets, int hidden, const float* x01s, const uint8_t* sels,
                    const int32_t* perm, const uint8_t* tile_sf, int64_t rows, const float* scalings_host, int L, int F,
-                   int log2_T, const char* what) {
+                   int log2_T, const char* what, bool density = false) {
     PS_REQUIRE(nets != nullptr, "%s: nets is null", what);
-    PS_REQUIRE(hidden == 16 || hidden == 64, "%s: hidden width %d not in {16, 64}", what, hidden);
-    PS_REQUIRE(F == 1 || F == 2, "%s: features_per_level %d not in {1,2}", what, F);
-    PS_REQUIRE(L >= 1 && L * F <= kK0 && L <= PS_MAX_LEVELS, "%s: L*F = %d exceeds %d", what, L * F, kK0);
+    if (int e = check_shape(hidden, L, F, density, what)) return e;
     PS_REQUIRE(log2_T >= 1 && log2_T <= 31, "%s: log2_hashmap_size %d out of range", what, log2_T);
     PS_REQUIRE(rows > 0 && rows % kRows == 0 && rows < (1ll << 31), "%s: rows must be a positive multiple of 128", what);
     PS_REQUIRE(x01s && sels && perm && tile_sf && scalings_host, "%s: null pointer", what);
@@ -990,4 +1112,31 @@ extern "C" int ps_prop_level_bwd_ms(const ps_prop_net_dev* nets_dev, int hidden,
     a.dtables = dtables_dev; a.d_density = d_density;
     a.feat = reinterpret_cast<__nv_bfloat16*>(const_cast<void*>(feat_bf16));
     return dispatch_ms(a, hidden, true, (cudaStream_t)stream);
+}
+
+// ---- density head of the main field (forward only) -----------------------------------------------------------------
+extern "C" int ps_density_level_fwd(const ps_prop_net* net, const float* origins, const float* dirs, const float* eu_bins,
+                                    int64_t N, int S, const float* aabb_host, int contract, const float* table,
+                                    const float* scalings_host, int L, int F, int log2_T, float* weights, void* stream) {
+    if (N == 0) return 0;
+    PropArgs a{};
+    if (int e = fill(a, net, origins, dirs, eu_bins, N, S, aabb_host, contract, scalings_host, L, F, log2_T,
+                     "density_level_fwd", true))
+        return e;
+    PS_REQUIRE(table && weights, "density_level_fwd: null pointer");
+    a.table = table; a.weights = weights;
+    return dispatch_density(&a, nullptr, F, a.in_dim, (cudaStream_t)stream);
+}
+
+extern "C" int ps_density_level_fwd_ms(const ps_prop_net_dev* nets_dev, int hidden, const float* x01_sorted,
+                                       const uint8_t* sel_sorted, const int32_t* perm, const uint8_t* tile_sf, int64_t rows,
+                                       const float* const* tables_dev, const float* scalings_host, int L, int F, int log2_T,
+                                       float* density, void* stream) {
+    PropMsArgs a{};
+    if (int e = fill_ms(a, nets_dev, hidden, x01_sorted, sel_sorted, perm, tile_sf, rows, scalings_host, L, F, log2_T,
+                        "density_level_fwd_ms", true))
+        return e;
+    PS_REQUIRE(tables_dev && density, "density_level_fwd_ms: null pointer");
+    a.tables = tables_dev; a.density = density;
+    return dispatch_density(nullptr, &a, F, a.in_dim, (cudaStream_t)stream);
 }

@@ -138,6 +138,29 @@ class iNGPField(Field):
             fused.GridMeta(enc._scalings_host, enc.log2_hashmap_size, enc.features_per_level), base_m, sem_m, rgb_m,
             self.geo_feat_dim, self.mlp_base_mlp.precision, threshold, base_p, sem_p, rgb_p)
 
+    def _grid_meta(self):
+        from .. import fused
+        enc = self.mlp_base_grid
+        return fused.GridMeta(enc._scalings_host, enc.log2_hashmap_size, enc.features_per_level)
+
+    def supports_level_depth(self, S: int) -> bool:
+        """True when `level_depth` serves this field with S samples per ray: a 2-layer base MLP with biases whose density
+        head fits the fused density kernels (fused.tc5_density_supported: bf16 class, hidden 64, L*F <= 48)."""
+        from .. import fused
+        ls = list(self.mlp_base_mlp.layers)
+        return (fused.USE_TC5_FIELD and len(ls) == 2 and all(l.bias is not None for l in ls)
+                and fused.tc5_density_supported(self._grid_meta(), ls[0].weight.shape[0], self.mlp_base_mlp.precision, S))
+
+    def level_depth(self, origins: Tensor, directions: Tensor, eu_bins: Tensor, threshold: float = 0.5) -> Tensor:
+        """Threshold depth [N,1] of the final level from its bins (the depth of `get_depth`), forward only, on the fused
+        density kernels: hash gather, base0 + ReLU and the density column of base1 only (no features or 80-wide output
+        written to memory).  Callers check `supports_level_depth` first."""
+        from .. import fused
+        l0, l1 = list(self.mlp_base_mlp.layers)
+        return fused.density_level_depth(origins, directions, eu_bins, self.mlp_base_grid.hash_table, self.aabb_host(),
+                                         self.spatial_distortion is not None, self._grid_meta(), l0.weight, l0.bias,
+                                         l1.weight, l1.bias, threshold)
+
     def semantic_fn(self, positions: Tensor) -> Tensor:
         """ingp_field.py:253-267."""
         assert self.use_semantics, "Cannot query semantics when `self.use_semantics` is set to False"

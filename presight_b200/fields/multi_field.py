@@ -121,6 +121,32 @@ class iNGPFieldMS(nn.Module):
                                     self._aabbs_host(), self.fields[0].spatial_distortion is not None, grid, threshold,
                                     params)
 
+    def supports_level_depth(self, S: int) -> bool:
+        """`level_depth` serves these sub-fields: the first one fits the fused density kernels and all share its grid,
+        base-MLP shapes and contraction (the semantic and colour heads play no part in the depth)."""
+        f0 = self.fields[0]
+        if not f0.supports_level_depth(S):
+            return False
+        g0 = f0._grid_meta()
+        shapes = [l.weight.shape for l in f0.mlp_base_mlp.layers]
+        return all(f._grid_meta() == g0 and [l.weight.shape for l in f.mlp_base_mlp.layers] == shapes
+                   and all(l.bias is not None for l in f.mlp_base_mlp.layers)
+                   and (f.spatial_distortion is None) == (f0.spatial_distortion is None) for f in self.fields[1:])
+
+    def level_depth(self, origins: Tensor, directions: Tensor, eu_bins: Tensor, threshold: float = 0.5) -> Tensor:
+        """Threshold depth [N,1] of the final level: iNGPField.level_depth for one sub-field, the routed mode of the fused
+        density kernels + one compositing pass for several.  Callers check `supports_level_depth` first."""
+        if len(self.fields) == 1:
+            return self.fields[0].level_depth(origins, directions, eu_bins, threshold)
+        from .. import fused
+        params = []
+        for f in self.fields:
+            l0, l1 = list(f.mlp_base_mlp.layers)
+            params.append((f.mlp_base_grid.hash_table, l0.weight, l0.bias, l1.weight, l1.bias))
+        return fused.density_level_depth_ms(origins, directions, eu_bins, self.centroids, self._aabbs_host(),
+                                            self.fields[0].spatial_distortion is not None, self.fields[0]._grid_meta(),
+                                            params, threshold)
+
     def _aabbs_host(self):
         key = tuple(f.aabb.data_ptr() for f in self.fields) + tuple(f.aabb._version for f in self.fields)
         if getattr(self, "_aabbs_cache", None) is None or self._aabbs_cache[0] != key:

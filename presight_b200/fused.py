@@ -938,3 +938,61 @@ def query_priors(points_scaled: Tensor, prop_fields, field) -> Tuple[Tensor, Ten
     feats = torch.empty(M, smeta.dims[-1], device=dev, dtype=torch.float16)
     call("ps_prior_finalize", host_ptrs(dens), len(dens), ptr(sem), M, smeta.dims[-1], ptr(mean), ptr(feats), stream())
     return mean, feats
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# Density level of the main field, forward only (prior extraction): the final level of `get_depth` as the fused proposal
+# kernels instantiated for the field's density head (csrc/prop_tc5.cu, ps_density_level_fwd*), then the threshold depth.
+# No autograd node and no saved state: these run under torch.no_grad().
+# ---------------------------------------------------------------------------------------------------------------
+def tc5_density_supported(grid: GridMeta, hidden: int, prec, S: int) -> bool:
+    """The fused density level covers the bf16 parity class, hidden width 64, L*F <= 48 with F in {1,2,4} and
+    S in {32,64,96,128}; anything else (fp32 class, S = 48, ...) keeps the per-operator path."""
+    return (prec == ops.PREC_BF16 and hidden == 64 and grid.F in (1, 2, 4) and grid.L * grid.F <= 48
+            and S in (32, 64, 96, 128))
+
+
+@torch.no_grad()
+def density_level_depth(origins, dirs, eu_bins, table, aabb, contract, grid: GridMeta, w0, b0, w1, b1,
+                        threshold: float = 0.5) -> Tensor:
+    """Threshold depth [N,1] of one sub-field's final level: ps_density_level_fwd -> ps_depth_threshold.
+    w0 / b0: base0 weight [64, L*F] / bias; w1 / b1: base1 weight [80, 64] / bias (row 0 and bias[0] are read)."""
+    import ctypes as C
+    from ._lib import host_prop_net
+    o, d, eu = _f32c(origins), _f32c(dirs), _f32c(eu_bins)
+    N, S = eu.shape[0], eu.shape[1] - 1
+    w = torch.empty(N, S, device=eu.device, dtype=torch.float32)
+    net = host_prop_net([w0.detach(), w1.detach()], [b0.detach(), b1.detach()])
+    with ops._probe(f"density_level_fwd_S{S}"):
+        call("ps_density_level_fwd", C.byref(net), ptr(o), ptr(d), ptr(eu), N, S, host_floats(aabb), 1 if contract else 0,
+             ptr(table.detach()), host_floats(grid.scalings), grid.L, grid.F, grid.log2_T, ptr(w), stream())
+    depth = torch.empty(N, 1, device=eu.device, dtype=torch.float32)
+    call("ps_depth_threshold", ptr(w), ptr(eu), N, S, float(threshold), ptr(depth), None, stream())
+    return depth
+
+
+@torch.no_grad()
+def density_level_depth_ms(origins, dirs, eu_bins, centroids, aabbs_host, contract, grid: GridMeta, fields_params,
+                           threshold: float = 0.5) -> Tensor:
+    """Threshold depth [N,1] of a final level routed to nf sub-fields: route_points -> ps_density_level_fwd_ms ->
+    ps_composite_fwd (threshold depth only).  fields_params: per sub-field (table, w0, b0, w1, b1) as in
+    density_level_depth."""
+    from ._lib import PropNetDev, device_ptr_array, device_struct_array
+    o, d, eu = _f32c(origins), _f32c(dirs), _f32c(eu_bins)
+    N, S = eu.shape[0], eu.shape[1] - 1
+    dev = eu.device
+    subs = [[t.detach() for t in fp] for fp in fields_params]
+    rt = route_points(centroids, aabbs_host, contract, o, d, eu)
+    slot = ("density", subs[0][0].data_ptr())
+    tables = device_ptr_array([s[0] for s in subs], dev, (slot, "tables"))
+    nets = device_struct_array([PropNetDev(s[1].data_ptr(), s[2].data_ptr(), s[3].data_ptr(), s[4].data_ptr(), 0, 0, 0, 0)
+                                for s in subs], dev, (slot, "nets_fwd"))
+    density = torch.zeros(N * S, device=dev, dtype=torch.float32)
+    with ops._probe(f"density_level_fwd_ms_S{S}"):
+        call("ps_density_level_fwd_ms", ptr(nets), subs[0][1].shape[0], ptr(rt.x01), ptr(rt.sel), ptr(rt.perm),
+             ptr(rt.tile_sf), rt.rows, ptr(tables), host_floats(grid.scalings), grid.L, grid.F, grid.log2_T, ptr(density),
+             stream())
+    depth = torch.empty(N, 1, device=dev, dtype=torch.float32)
+    call("ps_composite_fwd", ptr(eu), ptr(density), None, None, N, S, 0, float(threshold), None, None, None, None,
+         ptr(depth), None, None, stream())
+    return depth

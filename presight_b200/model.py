@@ -426,6 +426,21 @@ class NerfactoNuscMSModel(nn.Module):
         return outputs
 
     @torch.no_grad()
+    def get_surface_hits(self, ray_bundle: RayBundle, threshold: float = 0.5) -> Dict[str, Tensor]:
+        """The threshold depth of `get_depth` for prior extraction (scripts/extract_priors.py:100-113) -> {"depth": [N,1]}.
+        Same collider and proposal sampling as `get_depth`; the final level runs on the fused density kernels
+        (iNGPFieldMS.level_depth) when the field fits them, else exactly `get_depth`'s computation."""
+        ray_bundle = self.collider(ray_bundle)
+        ray_samples, _, _ = self.proposal_sampler(ray_bundle, density_fns=self.density_fns)
+        N, S = ray_samples.shape
+        eu = ray_samples.frustums.eu_bins
+        if self.use_fused and self.field.supports_level_depth(S):
+            return {"depth": self.field.level_depth(ray_bundle.origins, ray_bundle.directions, eu, threshold)}
+        density, _ = self.field.get_density(ray_samples)
+        _, _, _, _, depth, _, _ = ops.composite(eu, density.reshape(N, S), None, None, threshold)
+        return {"depth": depth}
+
+    @torch.no_grad()
     def get_depth_for_camera_ray_bundle(self, camera_ray_bundle: RayBundle, threshold: float = 0.5) -> Dict[str, Tensor]:
         """nerfacto_nusc_ms.py:710-734: chunked evaluation."""
         chunk = self.config.eval_num_rays_per_chunk

@@ -158,3 +158,13 @@ def step_bytes_per_ray(cfg: NerfactoNuscMSModelConfig, update_step: bool = True)
     total += cfg.num_nerf_samples_per_ray * (hash_bytes_fwd(cfg.num_levels, cfg.features_per_level)
                                              + hash_bytes_bwd(cfg.num_levels, cfg.features_per_level))
     return total
+
+
+def depth_pass_bytes_per_ray(cfg: NerfactoNuscMSModelConfig) -> int:
+    """Algorithmic bytes of the eval depth pass per ray (get_depth / get_surface_hits): sum over the sampling levels of
+    S_k x hash fwd bytes (C2 = 132 096, PreSight's shipped shape = 150 528)."""
+    total = 0
+    for i, S in enumerate(cfg.num_proposal_samples_per_ray):
+        a = cfg.proposal_net_args_list[min(i, len(cfg.proposal_net_args_list) - 1)]
+        total += S * hash_bytes_fwd(a["num_levels"], a["features_per_level"])
+    return total + cfg.num_nerf_samples_per_ray * hash_bytes_fwd(cfg.num_levels, cfg.features_per_level)
