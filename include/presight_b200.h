@@ -410,6 +410,21 @@ int ps_surface_hits(const float* origins, const float* dirs, const float* depth,
                     float max_range_m, float z_min_m, float z_max_m, float* points_scaled, float* points_m, uint8_t* keep,
                     void* stream);
 
+/* Image metrics of rendered images: replace the torchmetrics calls of the reference model's `get_metrics_dict` and
+ * `get_image_metrics_and_images` (models/PreSight/nerfacto_nusc_ms.py, as nerfstudio's models/nerfacto.py):
+ * `PeakSignalNoiseRatio(data_range=1.0)` and `structural_similarity_index_measure` with its defaults, one image at a time.
+ *   pred, gt [B,H,W,3] fp32 channels-last, per image:
+ *   sse [B] f64 = sum (pred - gt)^2;  psnr [B] f32 = 10 log10(data_range_psnr^2 / (sse / 3HW)), +inf for equal images
+ *   ssim [B] f64: 11-tap Gaussian window (sigma 1.5), data range max(max - min of pred, of gt) over the image, mean over
+ *                 channels and the (H-10) x (W-10) windows inside the image (what torchmetrics keeps after its reflect pad
+ *                 and crop); NaN for two constant images.  Definitions in presight_b200/csrc/metrics_core.h.
+ * ssim == NULL computes sse / psnr only, for any H, W (a ray batch as B = 1, H = 1, W = N); else H, W >= 11 (status 1
+ * otherwise).  sse may be NULL.  workspace: device memory of ps_image_metrics_workspace(B, H, W) bytes.  No host
+ * synchronisation and no floating-point atomics: repeated calls give bit-identical results. */
+int ps_image_metrics_workspace(int B, int H, int W, int64_t* bytes);
+int ps_image_metrics(const float* pred, const float* gt, int B, int H, int W, float data_range_psnr, void* workspace,
+                     double* sse, float* psnr, double* ssim, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Sub-field routing and the sub-field mode of the fused levels (SURVEY §8 a10).  Replace the nearest-centroid routers
  * fields/PreSight/ingp_field_ms.py:80-126, prop_density_field_ms.py:86-105 (cdist().argmin, then per sub-field a

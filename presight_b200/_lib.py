@@ -94,6 +94,8 @@ SIGNATURES = {
     "ps_density_level_fwd": [_p, _p, _p, _p, _i64, _i, _fp, _i, _p, _fp, _i, _i, _i, _p, _p],
     "ps_density_level_fwd_ms": [_p, _i, _p, _p, _p, _p, _i64, _p, _fp, _i, _i, _i, _p, _p],
     "ps_surface_hits": [_p, _p, _p, _i64, _f, _f, _f, _f, _p, _p, _p, _p],
+    "ps_image_metrics_workspace": [_i, _i, _i, _p],
+    "ps_image_metrics": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p, _p],
 }
 _RESTYPES = {"ps_last_error": C.c_char_p, "ps_abi_version": C.c_int, "ps_launch_count": C.c_int64}
 

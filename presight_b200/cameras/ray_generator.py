@@ -54,3 +54,18 @@ class RayGenerator(nn.Module):
              ptr(pixel_area), ptr(norm), stream())
         return RayBundle(origins=origins, directions=directions, pixel_area=pixel_area, camera_indices=idx[:, :1],
                          metadata={"directions_norm": norm})
+
+    def image_rays(self, camera_index: int, H: int, W: int) -> RayBundle:
+        """Every pixel of one H x W camera image -> a RayBundle whose fields are [H,W,.] (camera_indices included), as
+        `Cameras.generate_rays(camera_indices=i)` hands it to `get_outputs_for_camera_ray_bundle`.  The (camera, row, col)
+        indices are built on the device in row-major order and go through `forward`."""
+        dev = self.camera_to_worlds.device
+        rows = torch.arange(H, device=dev, dtype=torch.int64)[:, None].expand(H, W)
+        cols = torch.arange(W, device=dev, dtype=torch.int64)[None, :].expand(H, W)
+        idx = torch.stack([torch.full((H, W), int(camera_index), device=dev, dtype=torch.int64), rows, cols], dim=-1)
+        rb = self.forward(idx.view(H * W, 3))
+
+        def img(t: Tensor) -> Tensor:
+            return t.view(H, W, -1)
+        return RayBundle(origins=img(rb.origins), directions=img(rb.directions), pixel_area=img(rb.pixel_area),
+                         camera_indices=img(rb.camera_indices), metadata={k: img(v) for k, v in rb.metadata.items()})

@@ -456,6 +456,50 @@ class NerfactoNuscMSModel(nn.Module):
         return {k: torch.cat(v) for k, v in lists.items()}
 
     @torch.no_grad()
+    def get_outputs_for_camera_ray_bundle(self, camera_ray_bundle: RayBundle) -> Dict[str, Tensor]:
+        """nerfstudio's Model.get_outputs_for_camera_ray_bundle (models/base_model.py): a bundle whose fields are
+        [H,W,.] is flattened row-major and rendered by `forward` in consecutive slices of `eval_num_rays_per_chunk` rays;
+        the tensor outputs are concatenated and viewed as [H,W,-1].  Per-chunk statistics stay per chunk as in the
+        reference: `expected_depth` is clipped to its own chunk's min / max (renderers.py:379)."""
+        H, W = camera_ray_bundle.origins.shape[:2]
+        n = H * W
+        names = ("origins", "directions", "pixel_area", "camera_indices", "nears", "fars", "times")
+        flat = {k: getattr(camera_ray_bundle, k) for k in names}
+        flat = {k: None if v is None else v.reshape(n, -1) for k, v in flat.items()}
+        metadata = {k: v.reshape(n, -1) for k, v in camera_ray_bundle.metadata.items()}
+        chunk = self.config.eval_num_rays_per_chunk
+        lists: Dict[str, List[Tensor]] = {}
+        for i in range(0, n, chunk):
+            s = slice(i, i + chunk)
+            chunk_rb = RayBundle(**{k: None if v is None else v[s] for k, v in flat.items()},
+                                 metadata={k: v[s] for k, v in metadata.items()})
+            for k, v in self.forward(chunk_rb).items():
+                if torch.is_tensor(v):
+                    lists.setdefault(k, []).append(v)
+        return {k: torch.cat(v).view(H, W, -1) for k, v in lists.items()}
+
+    def get_metrics_dict(self, outputs: Dict[str, object], batch: Dict[str, Tensor]) -> Dict[str, Tensor]:
+        """nerfacto's get_metrics_dict: {"psnr": PSNR of the ray batch's rgb against batch["rgb"]}, a CUDA scalar (no host
+        read, so the training step stays free of synchronisations)."""
+        from . import metrics
+        return {"psnr": metrics.psnr(outputs["rgb"], batch["rgb"])}
+
+    def get_image_metrics_and_images(self, outputs: Dict[str, Tensor], batch: Dict[str, Tensor]
+                                     ) -> Tuple[Dict[str, float], Dict[str, Tensor]]:
+        """nerfacto's get_image_metrics_and_images for one rendered image: outputs of `get_outputs_for_camera_ray_bundle`,
+        batch["rgb"] [H,W,3] in [0,1] -> ({"psnr", "ssim"} as floats, {"img": gt and prediction side by side [H,2W,3],
+        "accumulation" [H,W,1], "depth" [H,W,1]}).  One host read for the two numbers.  The images are raw: the reference's
+        colormaps (matplotlib) are not applied, and LPIPS is not computed (it needs pretrained AlexNet weights)."""
+        from . import metrics
+        gt, pred = batch["rgb"].to(outputs["rgb"].device), outputs["rgb"]
+        psnr, ssim, _ = metrics.image_metrics(pred, gt)
+        vals = torch.stack([psnr[0].double(), ssim[0]]).tolist()
+        metrics_dict = {"psnr": float(vals[0]), "ssim": float(vals[1])}
+        images_dict = {"img": torch.cat([gt, pred], dim=1), "accumulation": outputs["accumulation"],
+                       "depth": outputs["depth"]}
+        return metrics_dict, images_dict
+
+    @torch.no_grad()
     def query_priors(self, points_scaled: Tensor) -> Tuple[Tensor, Tensor]:
         """scripts/extract_priors.py:130-138: mean density over proposal nets + field, clipped fp16 semantics."""
         if self.use_fused and len(self.field.fields) == 1 and self.field.supports_fused() and self.config.use_semantics:

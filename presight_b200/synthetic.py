@@ -19,14 +19,19 @@ CAM_YAWS_DEG = (0.0, 55.0, -55.0, 110.0, -110.0, 180.0)
 W, H, FX, FY, CX, CY = 1600, 900, 1266.0, 1266.0, 800.0, 450.0
 
 
-def make_rays(n_rays: int, seed: int = 42, n_frames: int = 200, n_videos: int = 10) -> Dict[str, torch.Tensor]:
-    """Host-side (CPU) batch: origins/directions [N,3], camera / video indices [N,1], and loss targets."""
-    g = torch.Generator().manual_seed(seed)
-    # ego trajectory: 2-D random walk, 2 m steps, wrapped into the 400 m tile; z ~ 1.5 m
+def _trajectory(g: torch.Generator, n_frames: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Ego trajectory: 2-D random walk, 2 m steps, wrapped into the 400 m tile -> (xy [F,2] metres, yaw [F])."""
     steps = torch.randn(n_frames, 2, generator=g) * 2.0
     xy = torch.cumsum(steps, dim=0)
     xy = (xy + 200.0) % 400.0 - 200.0
     ego_yaw = torch.cumsum(torch.randn(n_frames, generator=g) * 0.05, dim=0)
+    return xy, ego_yaw
+
+
+def make_rays(n_rays: int, seed: int = 42, n_frames: int = 200, n_videos: int = 10) -> Dict[str, torch.Tensor]:
+    """Host-side (CPU) batch: origins/directions [N,3], camera / video indices [N,1], and loss targets."""
+    g = torch.Generator().manual_seed(seed)
+    xy, ego_yaw = _trajectory(g, n_frames)                # cameras at z = 1.5 m
     frame = torch.randint(0, n_frames, (n_rays,), generator=g)
     cam = torch.randint(0, 6, (n_rays,), generator=g)
     u = torch.rand(n_rays, generator=g) * W
@@ -51,6 +56,25 @@ def make_rays(n_rays: int, seed: int = 42, n_frames: int = 200, n_videos: int = 
         "n_cameras": n_frames * 6,
         "n_videos": n_videos,
     }
+
+
+def make_cameras(seed: int = 42, n_frames: int = 200) -> Dict[str, torch.Tensor]:
+    """The cameras `make_rays(..., seed, n_frames)` draws its rays from, as a `RayGenerator` takes them (host tensors):
+    camera_to_worlds [6F,3,4] (OpenGL axes: x right, y up, looking along -z; camera index frame * 6 + camera, as in
+    make_rays), fx, fy, cx, cy [6F], and the image size H, W.  A pixel (row v, col u) of camera i gives the ray make_rays
+    draws for that camera at the continuous pixel (u + 0.5, v + 0.5)."""
+    g = torch.Generator().manual_seed(seed)
+    xy, ego_yaw = _trajectory(g, n_frames)
+    yaw = (ego_yaw[:, None] + torch.tensor(CAM_YAWS_DEG)[None, :] * (math.pi / 180.0)).reshape(-1)     # [6F]
+    C = yaw.shape[0]
+    right = torch.stack([torch.sin(yaw), -torch.cos(yaw), torch.zeros(C)], dim=-1)
+    up = torch.tensor([0.0, 0.0, 1.0]).expand(C, 3)
+    back = -torch.stack([torch.cos(yaw), torch.sin(yaw), torch.zeros(C)], dim=-1)
+    origin = torch.cat([xy, torch.full((n_frames, 1), 1.5)], dim=-1).repeat_interleave(6, dim=0) * POSE_SCALE
+    c2w = torch.stack([right, up, back, origin], dim=-1)                                             # [C,3,4]
+    full = lambda v: torch.full((C,), v)                                                             # noqa: E731
+    return {"camera_to_worlds": c2w.contiguous(), "fx": full(FX), "fy": full(FY), "cx": full(CX), "cy": full(CY),
+            "H": H, "W": W}
 
 
 def tile_aabb() -> torch.Tensor:
