@@ -425,6 +425,30 @@ int ps_image_metrics_workspace(int B, int H, int W, int64_t* bytes);
 int ps_image_metrics(const float* pred, const float* gt, int B, int H, int W, float data_range_psnr, void* workspace,
                      double* sse, float* psnr, double* ssim, void* stream);
 
+/* LPIPS of rendered images, the reference model's third evaluation metric: nerfacto's
+ * `LearnedPerceptualImagePatchSimilarity(normalize=True)` (AlexNet, LPIPS v0.1, mean reduction), as torchmetrics
+ * functional/image/lpips.py defines it after lpips 0.1 (`pretrained_networks.alexnet`, `normalize_tensor`).  Per pair:
+ *   x = (2 x - 1 - shift_c) / scale_c, shift (-0.030, -0.088, -0.188), scale (0.458, 0.448, 0.450);
+ *   AlexNet features cut after each ReLU (torchvision features.{0,3,6,8,10}, max-pool 3x3/2 floor before conv 2 and 3);
+ *   per layer k: f / (sqrt(sum_c f_c^2) + 1e-10) for both images, d = sum_c lin_k[c] (f0_c - f1_c)^2, mean over pixels;
+ *   out [B] f64 = sum of the five means, per_layer [B,5] f64 the means themselves (may be NULL).
+ * Convolutions in TF32 (operands rounded to nearest, fp32 accumulation), as cuDNN runs them for torchmetrics under
+ * PyTorch's default allow_tf32.  pred, gt [B,H,W,3] fp32 channels-last in [0,1] (not checked); H, W >= 31.
+ * net: device pointers packed by presight_b200.metrics.LPIPS: conv_w[k] [C_out][K_pad] fp32 with K = kh kw C_in in
+ * (ky, kx, ci) order, zero-padded to K_pad = a multiple of 32 and TF32-rounded (RNA); conv_b[k] [C_out]; lin[k] [C_k],
+ * C = 64, 192, 384, 256, 256.  workspace: device memory of ps_lpips_workspace(B, H, W) bytes (about 140 MB per pair at
+ * 1600 x 900).  Status 1 for B outside [1, 32767], H or W below 31, sizes whose per-image indices overflow 32 bits, or a
+ * null pointer.  No allocation, no host synchronisation and no floating-point atomics: repeated calls are bit-identical,
+ * and lpips(x, x) == 0 and lpips(a, b) == lpips(b, a) exactly. */
+typedef struct ps_lpips_net {
+    const float* conv_w[5];
+    const float* conv_b[5];
+    const float* lin[5];
+} ps_lpips_net;
+int ps_lpips_workspace(int B, int H, int W, int64_t* bytes);
+int ps_lpips(const float* pred, const float* gt, int B, int H, int W, const ps_lpips_net* net, void* workspace,
+             double* per_layer, double* out, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Sub-field routing and the sub-field mode of the fused levels (SURVEY §8 a10).  Replace the nearest-centroid routers
  * fields/PreSight/ingp_field_ms.py:80-126, prop_density_field_ms.py:86-105 (cdist().argmin, then per sub-field a

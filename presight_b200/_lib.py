@@ -96,6 +96,8 @@ SIGNATURES = {
     "ps_surface_hits": [_p, _p, _p, _i64, _f, _f, _f, _f, _p, _p, _p, _p],
     "ps_image_metrics_workspace": [_i, _i, _i, _p],
     "ps_image_metrics": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p, _p],
+    "ps_lpips_workspace": [_i, _i, _i, _p],
+    "ps_lpips": [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p],
 }
 _RESTYPES = {"ps_last_error": C.c_char_p, "ps_abi_version": C.c_int, "ps_launch_count": C.c_int64}
 
@@ -229,6 +231,11 @@ class FieldNetDev(C.Structure):
     """ps_field_net_dev of include/presight_b200.h."""
     _fields_ = [("W", C.c_void_p * 8), ("B", C.c_void_p * 8), ("dW", C.c_void_p * 8), ("dB", C.c_void_p * 8),
                 ("in_dim", C.c_int), ("app_dim", C.c_int)]
+
+
+class LpipsNet(C.Structure):
+    """ps_lpips_net of include/presight_b200.h."""
+    _fields_ = [("conv_w", C.c_void_p * 5), ("conv_b", C.c_void_p * 5), ("lin", C.c_void_p * 5)]
 
 
 _DEV_TABLES = {}

@@ -4,21 +4,22 @@ models/nerfacto.py `get_metrics_dict` / `get_image_metrics_and_images`, which Pr
     psnr(pred, gt)           PeakSignalNoiseRatio(data_range=1.0): 10 log10(1 / mean((pred - gt)^2)), fp64 sum
     ssim(pred, gt)           structural_similarity_index_measure with its defaults, one image at a time
     image_metrics(pred, gt)  both for a batch of images in one call
+    LPIPS                    LearnedPerceptualImagePatchSimilarity(normalize=True) (AlexNet, LPIPS v0.1) on `ps_lpips`
 
 Images are [H,W,3] or [B,H,W,3] fp32 channels-last, as `get_outputs_for_camera_ray_bundle` returns them.  Every result
 stays on the device (no host read), and repeated calls give bit-identical results.  The exact definitions, and the
-NaN SSIM of two constant images, are in csrc/metrics_core.h.  LPIPS, the reference's third evaluation metric, needs
-pretrained AlexNet weights and is not provided.
+NaN SSIM of two constant images, are in csrc/metrics_core.h.  LPIPS needs pretrained weights, which this project does
+not ship: the caller brings torchvision's AlexNet state dict and the LPIPS v0.1 linear layers (see `LPIPS`).
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import Tuple
+from typing import Dict, List, Mapping, Tuple
 
 import torch
 from torch import Tensor
 
-from ._lib import call, ptr, stream
+from ._lib import LpipsNet, call, ptr, stream
 
 
 def _images(pred: Tensor, gt: Tensor) -> Tuple[Tensor, Tensor]:
@@ -71,3 +72,143 @@ def ssim(pred: Tensor, gt: Tensor) -> Tensor:
     """SSIM of one [H,W,3] pair (a device scalar f64) or of each pair of [B,H,W,3] ([B] f64)."""
     out = image_metrics(pred, gt)[1]
     return out[0] if pred.dim() == 3 else out
+
+
+# ---- LPIPS ----------------------------------------------------------------------------------------------------------
+LPIPS_CHANNELS = (64, 192, 384, 256, 256)
+_LPIPS_CIN = (3, 64, 192, 384, 256)
+_LPIPS_CONV = ((11, 4, 2), (5, 1, 2), (3, 1, 1), (3, 1, 1), (3, 1, 1))   # kernel, stride, padding
+_ALEXNET_INDEX = (0, 3, 6, 8, 10)                                          # torchvision `features.{i}`
+_LPIPS_GROUP_BYTES = 1 << 30                 # workspace bound of one ps_lpips call (about 7 pairs at 1600 x 900)
+
+
+def lpips_layer_shapes(H: int, W: int) -> List[Tuple[int, int]]:
+    """(h, w) of the five AlexNet feature maps LPIPS compares for an H x W image; ValueError below 31 x 31, where the
+    second max-pool leaves nothing."""
+    if H < 31 or W < 31:
+        raise ValueError(f"LPIPS needs images of at least 31 x 31 pixels, got {H} x {W}")
+
+    def conv(n, k, s, p):
+        return (n + 2 * p - k) // s + 1
+
+    def pool(n):
+        return (n - 3) // 2 + 1
+
+    h1, w1 = conv(H, 11, 4, 2), conv(W, 11, 4, 2)
+    h2, w2 = pool(h1), pool(w1)
+    h3, w3 = pool(h2), pool(w2)
+    return [(h1, w1), (h2, w2), (h3, w3), (h3, w3), (h3, w3)]
+
+
+def lpips_flops(H: int, W: int) -> int:
+    """Multiply-adds x 2 of the five convolutions for one H x W image (a pair costs twice this)."""
+    return sum(2 * h * w * c * cin * k * k
+               for (h, w), c, cin, (k, _, _) in zip(lpips_layer_shapes(H, W), LPIPS_CHANNELS, _LPIPS_CIN, _LPIPS_CONV))
+
+
+def tf32_round(x: Tensor) -> Tensor:
+    """fp32 -> the nearest TF32 value (ties away from zero), as cvt.rna.tf32.f32 rounds finite values."""
+    bits = x.detach().to(torch.float32).contiguous().view(torch.int32)
+    return ((bits + 0x1000) & -0x2000).view(torch.float32)
+
+
+def _expected_keys() -> Dict[str, Tuple[int, ...]]:
+    exp = {}
+    for i, c, cin, (k, _, _) in zip(_ALEXNET_INDEX, LPIPS_CHANNELS, _LPIPS_CIN, _LPIPS_CONV):
+        exp[f"features.{i}.weight"] = (c, cin, k, k)
+        exp[f"features.{i}.bias"] = (c,)
+    for j, c in enumerate(LPIPS_CHANNELS):
+        exp[f"lin{j}.model.1.weight"] = (1, c, 1, 1)
+    return exp
+
+
+class LPIPS:
+    """LPIPS as nerfacto computes it: torchmetrics `LearnedPerceptualImagePatchSimilarity(net_type="alex",
+    normalize=True)`, LPIPS v0.1, mean over the batch's pairs in the reference (here one value per pair).  Definition in
+    include/presight_b200.h (`ps_lpips`); the convolutions run in TF32, as cuDNN runs torchmetrics' under PyTorch's
+    default `allow_tf32`.
+
+    A plain class, not an nn.Module: attached to a model it adds nothing to the model's state_dict.  The weights are the
+    caller's: `LPIPS.from_state_dicts(torchvision_alexnet.state_dict(), lpips_alex_lin_state_dict)`.
+
+        net = LPIPS.from_state_dicts(alexnet_sd, lin_sd)
+        value = net(pred, gt)                    # [H,W,3] -> device f64 scalar, [B,H,W,3] -> [B]
+    """
+
+    def __init__(self, conv_w: List[Tensor], conv_b: List[Tensor], lin: List[Tensor]):
+        """Packed tensors (see `from_state_dicts`): conv_w[k] [C_out][K_pad] TF32-rounded in (ky, kx, ci) order,
+        conv_b[k] [C_out], lin[k] [C_k], all fp32 on one device."""
+        self.conv_w, self.conv_b, self.lin = list(conv_w), list(conv_b), list(lin)
+        self.device = self.conv_w[0].device
+
+    @classmethod
+    def from_state_dicts(cls, alexnet_sd: Mapping[str, Tensor], lin_sd: Mapping[str, Tensor],
+                         device="cuda") -> "LPIPS":
+        """alexnet_sd: torchvision's AlexNet keys `features.{0,3,6,8,10}.{weight,bias}` (what
+        `torchvision.models.alexnet(...).state_dict()` and the `alexnet-owt-*.pth` file hold; `classifier.*` is
+        ignored).  lin_sd: the LPIPS v0.1 `alex.pth` keys `lin{k}.model.1.weight`, each [1,C_k,1,1].  A missing key or a
+        wrong shape raises a ValueError naming every expected key and shape.  Packing runs on CPU tensors as well."""
+        exp = _expected_keys()
+        got = {**{k: v for k, v in alexnet_sd.items() if k.startswith("features.")},
+               **{k: v for k, v in lin_sd.items()}}
+        bad = [f"missing {k}" for k in exp if k not in got]
+        bad += [f"{k} has shape {tuple(got[k].shape)}, expected {exp[k]}" for k in exp
+                if k in got and tuple(got[k].shape) != exp[k]]
+        if bad:
+            want = ", ".join(f"{k} {list(v)}" for k, v in exp.items())
+            raise ValueError(f"LPIPS weights: {'; '.join(bad)}.  Expected keys and shapes: {want}")
+        conv_w, conv_b, lin = [], [], []
+        for i, c in zip(_ALEXNET_INDEX, LPIPS_CHANNELS):
+            w = got[f"features.{i}.weight"].detach().to(torch.float32)
+            k = w.shape[1] * w.shape[2] * w.shape[3]
+            w = w.permute(0, 2, 3, 1).reshape(c, k)                       # (ky, kx, ci), the kernel's K order
+            w = torch.nn.functional.pad(w, (0, -k % 32))
+            conv_w.append(tf32_round(w).to(device).contiguous())
+            conv_b.append(got[f"features.{i}.bias"].detach().to(torch.float32).to(device).contiguous())
+        for j, c in enumerate(LPIPS_CHANNELS):
+            lin.append(got[f"lin{j}.model.1.weight"].detach().to(torch.float32).reshape(c).to(device).contiguous())
+        return cls(conv_w, conv_b, lin)
+
+    def unpack(self) -> Tuple[Dict[str, Tensor], Dict[str, Tensor]]:
+        """The packed weights back in the layouts `from_state_dicts` reads (convolution weights TF32-rounded)."""
+        alex, lin = {}, {}
+        for i, w, b, c, cin, (k, _, _) in zip(_ALEXNET_INDEX, self.conv_w, self.conv_b, LPIPS_CHANNELS, _LPIPS_CIN,
+                                              _LPIPS_CONV):
+            alex[f"features.{i}.weight"] = w[:, :k * k * cin].reshape(c, k, k, cin).permute(0, 3, 1, 2).contiguous()
+            alex[f"features.{i}.bias"] = b.clone()
+        for j, (v, c) in enumerate(zip(self.lin, LPIPS_CHANNELS)):
+            lin[f"lin{j}.model.1.weight"] = v.reshape(1, c, 1, 1).clone()
+        return alex, lin
+
+    def _net(self) -> LpipsNet:
+        net = LpipsNet()
+        for k in range(5):
+            net.conv_w[k], net.conv_b[k], net.lin[k] = ptr(self.conv_w[k]), ptr(self.conv_b[k]), ptr(self.lin[k])
+        return net
+
+    @torch.no_grad()
+    def __call__(self, pred: Tensor, gt: Tensor, per_layer: bool = False):
+        """pred, gt [H,W,3] or [B,H,W,3] fp32 in [0,1], H, W >= 31 -> LPIPS as a device f64 scalar (or [B]), plus the
+        five per-layer means [5] (or [B,5]) when `per_layer`.  No host read.  Values outside [0,1] are not checked
+        (that would need one); torchmetrics rejects them.  Large batches run in groups of bounded workspace; every pair
+        is computed alone, so the grouping does not change any value."""
+        p, g = _images(pred, gt)
+        if p.device != self.device:
+            raise ValueError(f"images on {p.device}, LPIPS weights on {self.device}")
+        B, H, W, _ = p.shape
+        lpips_layer_shapes(H, W)
+        out = torch.empty(B, dtype=torch.float64, device=p.device)
+        layers = torch.empty(B, 5, dtype=torch.float64, device=p.device)
+        net = self._net()
+        nbytes = C.c_int64(0)
+        call("ps_lpips_workspace", 1, H, W, C.byref(nbytes))
+        group = max(1, min(B, _LPIPS_GROUP_BYTES // int(nbytes.value)))
+        call("ps_lpips_workspace", group, H, W, C.byref(nbytes))
+        ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=p.device)
+        for i in range(0, B, group):
+            n = min(group, B - i)
+            call("ps_lpips", ptr(p[i:i + n]), ptr(g[i:i + n]), n, H, W, C.byref(net), ptr(ws), ptr(layers[i:i + n]),
+                 ptr(out[i:i + n]), stream())
+        if pred.dim() == 3:
+            out, layers = out[0], layers[0]
+        return (out, layers) if per_layer else out

@@ -8,7 +8,7 @@ scripts/extract_priors.py:130-138.  Module names (`field`, `proposal_networks`, 
 from __future__ import annotations
 
 from dataclasses import dataclass, field
-from typing import Dict, List, Literal, Optional, Tuple
+from typing import TYPE_CHECKING, Dict, List, Literal, Optional, Tuple
 
 import numpy as np
 import torch
@@ -23,6 +23,9 @@ from .fields.prop_density_field import PropNetDensityField
 from .fields.sky_field import SkyField
 from .model_components.ray_samplers import ProposalNetworkSampler, SpacedSampler
 from .model_components.renderers import AccumulationRenderer, DepthRenderer, RGBRenderer
+
+if TYPE_CHECKING:
+    from .metrics import LPIPS
 
 VIDEO_ID = "video_id"
 
@@ -164,6 +167,10 @@ class NearFarCollider:
 
 
 class NerfactoNuscMSModel(nn.Module):
+    # LPIPS of the evaluation images (`metrics.LPIPS`, built from the caller's pretrained weights); None leaves it out.
+    # A plain attribute, not a submodule, so state_dict() keeps the reference's keys.
+    lpips: Optional[LPIPS] = None
+
     def __init__(self, config: NerfactoNuscMSModelConfig, centroids: Tensor, aabbs: Tensor, num_train_cameras: int = 1,
                  num_train_videos: int = 1) -> None:
         super().__init__()
@@ -487,14 +494,20 @@ class NerfactoNuscMSModel(nn.Module):
     def get_image_metrics_and_images(self, outputs: Dict[str, Tensor], batch: Dict[str, Tensor]
                                      ) -> Tuple[Dict[str, float], Dict[str, Tensor]]:
         """nerfacto's get_image_metrics_and_images for one rendered image: outputs of `get_outputs_for_camera_ray_bundle`,
-        batch["rgb"] [H,W,3] in [0,1] -> ({"psnr", "ssim"} as floats, {"img": gt and prediction side by side [H,2W,3],
-        "accumulation" [H,W,1], "depth" [H,W,1]}).  One host read for the two numbers.  The images are raw: the reference's
-        colormaps (matplotlib) are not applied, and LPIPS is not computed (it needs pretrained AlexNet weights)."""
+        batch["rgb"] [H,W,3] in [0,1] -> ({"psnr", "ssim"} as floats, and "lpips" when `self.lpips` is set; {"img": gt and
+        prediction side by side [H,2W,3], "accumulation" [H,W,1], "depth" [H,W,1]}).  One host read for the numbers.
+        LPIPS scores the render clamped to [0,1], as the reference does.  The images are raw: the reference's colormaps
+        (matplotlib) are not applied."""
         from . import metrics
         gt, pred = batch["rgb"].to(outputs["rgb"].device), outputs["rgb"]
         psnr, ssim, _ = metrics.image_metrics(pred, gt)
-        vals = torch.stack([psnr[0].double(), ssim[0]]).tolist()
+        vals = [psnr[0].double(), ssim[0]]
+        if self.lpips is not None:
+            vals.append(self.lpips(pred.clamp(0.0, 1.0), gt))
+        vals = torch.stack(vals).tolist()
         metrics_dict = {"psnr": float(vals[0]), "ssim": float(vals[1])}
+        if self.lpips is not None:
+            metrics_dict["lpips"] = float(vals[2])
         images_dict = {"img": torch.cat([gt, pred], dim=1), "accumulation": outputs["accumulation"],
                        "depth": outputs["depth"]}
         return metrics_dict, images_dict
