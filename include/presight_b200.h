@@ -449,6 +449,21 @@ int ps_lpips_workspace(int B, int H, int W, int64_t* bytes);
 int ps_lpips(const float* pred, const float* gt, int B, int H, int W, const ps_lpips_net* net, void* workspace,
              double* per_layer, double* out, void* stream);
 
+/* Colormapped evaluation images, as the reference model's `get_image_metrics_and_images` (nerfstudio's
+ * models/nerfacto.py) builds them with utils/colormaps.py and default ColormapOptions, for one image of HW pixels:
+ *   out[0]     [HW,3] = lut[idx(acc)]                                         (apply_colormap(accumulation))
+ *   out[1 + m] [HW,3] = lut[idx(clip((d - near) / (far - near + 1e-10), 0, 1))] * acc + (1 - acc), d = maps[m]
+ *                                                                             (apply_depth_colormap(d, accumulation))
+ *   idx(x) = long(nan_to_num(clip(x, 0, 1)) * 255); near / far = min / max of the map, NaN if it holds one.
+ * Bit-identical to torch running that definition on the device (rounding of each step in csrc/colormap_core.h).
+ *   maps [M][HW] fp32 (M depth-like maps: depth, prop_depth_0, ...), acc [HW] fp32, lut [256][3] fp32 (e.g. matplotlib's
+ *   turbo colours), out [M+1][HW][3] fp32.  M in [0, 1024]; maps and workspace may be NULL when M == 0.
+ * workspace: device memory of ps_colormap_workspace(M, HW) bytes.  Status 1 for M outside [0, 1024], HW <= 0 or a null
+ * pointer.  No host synchronisation and no floating-point atomics: repeated calls are bit-identical. */
+int ps_colormap_workspace(int M, int64_t HW, int64_t* bytes);
+int ps_colormap(const float* maps, int M, int64_t HW, const float* acc, const float* lut, void* workspace, float* out,
+                void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Sub-field routing and the sub-field mode of the fused levels (SURVEY §8 a10).  Replace the nearest-centroid routers
  * fields/PreSight/ingp_field_ms.py:80-126, prop_density_field_ms.py:86-105 (cdist().argmin, then per sub-field a

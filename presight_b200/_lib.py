@@ -98,6 +98,8 @@ SIGNATURES = {
     "ps_image_metrics": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p, _p],
     "ps_lpips_workspace": [_i, _i, _i, _p],
     "ps_lpips": [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p],
+    "ps_colormap_workspace": [_i, _i64, _p],
+    "ps_colormap": [_p, _i, _i64, _p, _p, _p, _p, _p],
 }
 _RESTYPES = {"ps_last_error": C.c_char_p, "ps_abi_version": C.c_int, "ps_launch_count": C.c_int64}
 

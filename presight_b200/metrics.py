@@ -5,16 +5,20 @@ models/nerfacto.py `get_metrics_dict` / `get_image_metrics_and_images`, which Pr
     ssim(pred, gt)           structural_similarity_index_measure with its defaults, one image at a time
     image_metrics(pred, gt)  both for a batch of images in one call
     LPIPS                    LearnedPerceptualImagePatchSimilarity(normalize=True) (AlexNet, LPIPS v0.1) on `ps_lpips`
+    colormap_images          the colormapped accumulation and depth images of nerfacto (utils/colormaps.py) on
+                             `ps_colormap`
 
 Images are [H,W,3] or [B,H,W,3] fp32 channels-last, as `get_outputs_for_camera_ray_bundle` returns them.  Every result
 stays on the device (no host read), and repeated calls give bit-identical results.  The exact definitions, and the
 NaN SSIM of two constant images, are in csrc/metrics_core.h.  LPIPS needs pretrained weights, which this project does
-not ship: the caller brings torchvision's AlexNet state dict and the LPIPS v0.1 linear layers (see `LPIPS`).
+not ship: the caller brings torchvision's AlexNet state dict and the LPIPS v0.1 linear layers, or a reference checkpoint
+that holds them (see `LPIPS`).  Likewise the colormaps need the caller's [256,3] table (e.g. matplotlib's turbo).
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Mapping, Tuple
+import re
+from typing import Dict, List, Mapping, Sequence, Tuple
 
 import torch
 from torch import Tensor
@@ -74,6 +78,32 @@ def ssim(pred: Tensor, gt: Tensor) -> Tensor:
     return out[0] if pred.dim() == 3 else out
 
 
+@torch.no_grad()
+def colormap_images(depth_maps: Sequence[Tensor], accumulation: Tensor, lut: Tensor) -> Tuple[Tensor, List[Tensor]]:
+    """nerfacto's evaluation images in one `ps_colormap` call: depth_maps [H,W,1] each (depth, prop_depth_0, ...),
+    accumulation [H,W,1], lut [256,3] -> (apply_colormap(accumulation), [apply_depth_colormap(d, accumulation) for d]),
+    each [H,W,3] fp32, bit-identical to nerfstudio's utils/colormaps.py run by torch on the device with default
+    ColormapOptions and this table as the colormap.  No host read: the per-map min / max stay on the device."""
+    if accumulation.dim() != 3 or accumulation.shape[-1] != 1:
+        raise ValueError(f"accumulation must be [H,W,1], got {tuple(accumulation.shape)}")
+    for d in depth_maps:
+        if d.shape != accumulation.shape:
+            raise ValueError(f"depth map {tuple(d.shape)} and accumulation {tuple(accumulation.shape)} differ in shape")
+    if tuple(lut.shape) != (256, 3):
+        raise ValueError(f"lut must be [256,3], got {tuple(lut.shape)}")
+    H, W, _ = accumulation.shape
+    dev, M = accumulation.device, len(depth_maps)
+    acc = accumulation.detach().to(torch.float32).contiguous()
+    table = lut.detach().to(device=dev, dtype=torch.float32).contiguous()
+    maps = torch.stack([d.detach().reshape(H * W) for d in depth_maps]).to(torch.float32) if M else None
+    nbytes = C.c_int64(0)
+    call("ps_colormap_workspace", M, H * W, C.byref(nbytes))
+    ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=dev) if M else None
+    out = torch.empty(M + 1, H, W, 3, dtype=torch.float32, device=dev)
+    call("ps_colormap", ptr(maps), M, H * W, ptr(acc), ptr(table), ptr(ws), ptr(out), stream())
+    return out[0], list(out[1:])
+
+
 # ---- LPIPS ----------------------------------------------------------------------------------------------------------
 LPIPS_CHANNELS = (64, 192, 384, 256, 256)
 _LPIPS_CIN = (3, 64, 192, 384, 256)
@@ -122,6 +152,32 @@ def _expected_keys() -> Dict[str, Tuple[int, ...]]:
     return exp
 
 
+# where a reference checkpoint keeps the weights: torchmetrics' `_LPIPS` under the model's `lpips.net.`, its AlexNet
+# slices holding torchvision's `features.{i}` layers
+_REFERENCE_SLICES = {0: "net.slice1.0", 3: "net.slice2.3", 6: "net.slice3.6", 8: "net.slice4.8", 10: "net.slice5.10"}
+_REFERENCE_KEY = re.compile(r"^((?:[^.]*\.)*?)lpips\.net\.(.+)$")
+# the scaling layer `ps_lpips` applies (csrc/lpips.cu c_shift / c_scale)
+_SCALING_LAYER = {"scaling_layer.shift": (-0.030, -0.088, -0.188), "scaling_layer.scale": (0.458, 0.448, 0.450)}
+
+
+def _reference_names() -> Dict[str, str]:
+    """key after `lpips.net.` -> the key `from_state_dicts` reads"""
+    names = {}
+    for i, s in _REFERENCE_SLICES.items():
+        names[f"{s}.weight"], names[f"{s}.bias"] = f"features.{i}.weight", f"features.{i}.bias"
+    names.update({f"lin{j}.model.1.weight": f"lin{j}.model.1.weight" for j in range(len(LPIPS_CHANNELS))})
+    return names
+
+
+def _check_keys(got: Mapping[str, Tensor], exp: Mapping[str, Tuple[int, ...]], extra: Sequence[str] = ()) -> None:
+    bad = list(extra) + [f"missing {k}" for k in exp if k not in got]
+    bad += [f"{k} has shape {tuple(got[k].shape)}, expected {exp[k]}" for k in exp
+            if k in got and tuple(got[k].shape) != exp[k]]
+    if bad:
+        want = ", ".join(f"{k} {list(v)}" for k, v in exp.items())
+        raise ValueError(f"LPIPS weights: {'; '.join(bad)}.  Expected keys and shapes: {want}")
+
+
 class LPIPS:
     """LPIPS as nerfacto computes it: torchmetrics `LearnedPerceptualImagePatchSimilarity(net_type="alex",
     normalize=True)`, LPIPS v0.1, mean over the batch's pairs in the reference (here one value per pair).  Definition in
@@ -148,15 +204,9 @@ class LPIPS:
         `torchvision.models.alexnet(...).state_dict()` and the `alexnet-owt-*.pth` file hold; `classifier.*` is
         ignored).  lin_sd: the LPIPS v0.1 `alex.pth` keys `lin{k}.model.1.weight`, each [1,C_k,1,1].  A missing key or a
         wrong shape raises a ValueError naming every expected key and shape.  Packing runs on CPU tensors as well."""
-        exp = _expected_keys()
         got = {**{k: v for k, v in alexnet_sd.items() if k.startswith("features.")},
                **{k: v for k, v in lin_sd.items()}}
-        bad = [f"missing {k}" for k in exp if k not in got]
-        bad += [f"{k} has shape {tuple(got[k].shape)}, expected {exp[k]}" for k in exp
-                if k in got and tuple(got[k].shape) != exp[k]]
-        if bad:
-            want = ", ".join(f"{k} {list(v)}" for k, v in exp.items())
-            raise ValueError(f"LPIPS weights: {'; '.join(bad)}.  Expected keys and shapes: {want}")
+        _check_keys(got, _expected_keys())
         conv_w, conv_b, lin = [], [], []
         for i, c in zip(_ALEXNET_INDEX, LPIPS_CHANNELS):
             w = got[f"features.{i}.weight"].detach().to(torch.float32)
@@ -168,6 +218,38 @@ class LPIPS:
         for j, c in enumerate(LPIPS_CHANNELS):
             lin.append(got[f"lin{j}.model.1.weight"].detach().to(torch.float32).reshape(c).to(device).contiguous())
         return cls(conv_w, conv_b, lin)
+
+    @classmethod
+    def from_reference_state_dict(cls, sd: Mapping[str, Tensor], device="cuda") -> "LPIPS":
+        """The weights a reference checkpoint already holds: a model or pipeline state dict (the keys under any one
+        prefix, e.g. `_model.` or `_model.module.`) whose `lpips.net.*` entries are torchmetrics' `_LPIPS`:
+        `net.slice{1..5}.{0,3,6,8,10}.{weight,bias}` (torchvision's `features.{0,3,6,8,10}`) and
+        `lin{k}.model.1.weight`.  A missing key, a wrong shape or keys under two different prefixes raise a ValueError
+        naming every expected key and shape; so does a `scaling_layer.shift` / `scale`, when present, that differs from
+        the constants `ps_lpips` applies."""
+        found = {}
+        for k, v in sd.items():
+            m = _REFERENCE_KEY.match(k)
+            if m:
+                found.setdefault(m.group(1), {})[m.group(2)] = v
+        names = _reference_names()
+        shapes = _expected_keys()
+        prefix = next(iter(found), "")
+        exp = {f"{prefix}lpips.net.{k}": shapes[v] for k, v in names.items()}
+        extra = []
+        if len(found) > 1:
+            extra.append("keys under more than one prefix: " + ", ".join(repr(p + "lpips.net.") for p in found))
+        sub = found.get(prefix, {})
+        _check_keys({f"{prefix}lpips.net.{k}": v for k, v in sub.items()}, exp, extra)
+        for k, want in _SCALING_LAYER.items():
+            if k in sub:
+                v = sub[k].detach().to(device="cpu", dtype=torch.float32).reshape(-1)
+                if not torch.equal(v, torch.tensor(want, dtype=torch.float32)):
+                    raise ValueError(f"LPIPS weights: {prefix}lpips.net.{k} is {v.tolist()}, but ps_lpips applies "
+                                     f"{list(want)}")
+        got = {theirs: sub[k] for k, theirs in names.items()}
+        return cls.from_state_dicts({k: v for k, v in got.items() if k.startswith("features.")},
+                                    {k: v for k, v in got.items() if k.startswith("lin")}, device=device)
 
     def unpack(self) -> Tuple[Dict[str, Tensor], Dict[str, Tensor]]:
         """The packed weights back in the layouts `from_state_dicts` reads (convolution weights TF32-rounded)."""

@@ -170,6 +170,9 @@ class NerfactoNuscMSModel(nn.Module):
     # LPIPS of the evaluation images (`metrics.LPIPS`, built from the caller's pretrained weights); None leaves it out.
     # A plain attribute, not a submodule, so state_dict() keeps the reference's keys.
     lpips: Optional[LPIPS] = None
+    # [256,3] colormap table (e.g. matplotlib's turbo colours) for the evaluation images; None returns them raw.  A plain
+    # attribute as well, for the same reason.
+    colormap: Optional[Tensor] = None
 
     def __init__(self, config: NerfactoNuscMSModelConfig, centroids: Tensor, aabbs: Tensor, num_train_cameras: int = 1,
                  num_train_videos: int = 1) -> None:
@@ -495,21 +498,27 @@ class NerfactoNuscMSModel(nn.Module):
                                      ) -> Tuple[Dict[str, float], Dict[str, Tensor]]:
         """nerfacto's get_image_metrics_and_images for one rendered image: outputs of `get_outputs_for_camera_ray_bundle`,
         batch["rgb"] [H,W,3] in [0,1] -> ({"psnr", "ssim"} as floats, and "lpips" when `self.lpips` is set; {"img": gt and
-        prediction side by side [H,2W,3], "accumulation" [H,W,1], "depth" [H,W,1]}).  One host read for the numbers.
-        LPIPS scores the render clamped to [0,1], as the reference does.  The images are raw: the reference's colormaps
-        (matplotlib) are not applied."""
+        prediction side by side [H,2W,3], "accumulation", "depth"}).  One host read for the numbers.  LPIPS scores the
+        render clamped to [0,1], as the reference does.  With `self.colormap` unset the images are raw [H,W,1]; with it
+        set they are the reference's colormapped [H,W,3] images, `prop_depth_{i}` of every proposal iteration included,
+        all from one `ps_colormap` call (`metrics.colormap_images`)."""
         from . import metrics
         gt, pred = batch["rgb"].to(outputs["rgb"].device), outputs["rgb"]
         psnr, ssim, _ = metrics.image_metrics(pred, gt)
         vals = [psnr[0].double(), ssim[0]]
         if self.lpips is not None:
             vals.append(self.lpips(pred.clamp(0.0, 1.0), gt))
+        images_dict = {"img": torch.cat([gt, pred], dim=1), "accumulation": outputs["accumulation"],
+                       "depth": outputs["depth"]}
+        if self.colormap is not None:
+            props = [f"prop_depth_{i}" for i in range(self.config.num_proposal_iterations)]
+            acc_img, depth_imgs = metrics.colormap_images([outputs["depth"]] + [outputs[k] for k in props],
+                                                          outputs["accumulation"], self.colormap)
+            images_dict.update({"accumulation": acc_img, "depth": depth_imgs[0]}, **dict(zip(props, depth_imgs[1:])))
         vals = torch.stack(vals).tolist()
         metrics_dict = {"psnr": float(vals[0]), "ssim": float(vals[1])}
         if self.lpips is not None:
             metrics_dict["lpips"] = float(vals[2])
-        images_dict = {"img": torch.cat([gt, pred], dim=1), "accumulation": outputs["accumulation"],
-                       "depth": outputs["depth"]}
         return metrics_dict, images_dict
 
     @torch.no_grad()
