@@ -292,6 +292,35 @@ int ps_voxel_finalize(const int64_t* keys, int64_t capacity, const uint32_t* cou
 int ps_hits_quantile(const int64_t* hits, int64_t M, double q, uint32_t* hist, int64_t bins, double* out, int* status,
                      void* stream);
 
+/* The tile voxelizer: the per-voxel means of ps_voxel_accumulate / ps_voxel_finalize in memory that follows the number of
+ * voxels V, not of points.  Two passes over the points, with the same voxel key as ps_voxel_accumulate:
+ * ps_voxel_insert: pass 1, keys only.  Inserts the key of every point into keys [capacity] int64 (preset to -1, capacity
+ *   a power of two; the caller keeps capacity >= 2 * (V + N)) and adds the number of new voxels to *n_voxels.
+ * ps_voxel_rehash: moves the occupied keys of old_keys [old_capacity] into keys [capacity] (preset to -1, capacity >=
+ *   old_capacity, both powers of two).
+ * ps_voxel_assign_rows: rows[slot of sorted_keys[r]] = r for r < V (sorted_keys: the occupied keys in ascending order;
+ *   rows [capacity] int32 beside the table).
+ * ps_voxel_accumulate_rows: pass 2.  Looks each point's row up (no insertion) and adds the point to the dense rows:
+ *   counts [V] u32, sum_xyz / sum_col [V,3] and sum_feat [V,C] fp64, caller-zeroed.  features_f16 [N,C] / colors [N,3]
+ *   nullable together with their sums.
+ * ps_voxel_finalize_rows: row r's means -> out_xyz [V,3], out_col [V,3], out_feat_f16 [V,C], out_hits [V], as
+ *   ps_voxel_finalize writes them; the rows stay in ascending key order.
+ * status: |= 1 table full, |= 2 voxel index outside 21 bits per axis, |= 4 a point's voxel is not in the table (checked by
+ *   the caller after a sync).  No kernel allocates. */
+int ps_voxel_insert(const float* points, int64_t N, const float* min_point, double voxel_size, int64_t* keys,
+                    int64_t capacity, uint64_t* n_voxels, int* status, void* stream);
+int ps_voxel_rehash(const int64_t* old_keys, int64_t old_capacity, int64_t* keys, int64_t capacity, int* status,
+                    void* stream);
+int ps_voxel_assign_rows(const int64_t* sorted_keys, int64_t V, const int64_t* keys, int64_t capacity, int32_t* rows,
+                         int* status, void* stream);
+int ps_voxel_accumulate_rows(const float* points, const void* features_f16, const float* colors, int64_t N, int C,
+                             const float* min_point, double voxel_size, const int64_t* keys, const int32_t* rows,
+                             int64_t capacity, uint32_t* counts, double* sum_xyz, double* sum_col, double* sum_feat,
+                             int* status, void* stream);
+int ps_voxel_finalize_rows(const uint32_t* counts, const double* sum_xyz, const double* sum_col, const double* sum_feat,
+                           int64_t V, int C, float* out_xyz, float* out_col, void* out_feat_f16, int64_t* out_hits,
+                           void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Ray generation (SURVEY 8f-3): RayGenerator.forward + Cameras.generate_rays for PERSPECTIVE cameras without distortion
  * (model_components/ray_generators.py:43-61, cameras/cameras.py:497-880).
@@ -409,6 +438,17 @@ int ps_density_level_fwd_ms(const struct ps_prop_net_dev* nets_dev, int hidden, 
 int ps_surface_hits(const float* origins, const float* dirs, const float* depth, int64_t N, float pose_scale,
                     float max_range_m, float z_min_m, float z_max_m, float* points_scaled, float* points_m, uint8_t* keep,
                     void* stream);
+
+/* The kept hits of a chunk into the extractor's hit store, in ray order: the rows with keep[i] != 0 && density[i] > 1
+ * (extract_priors.py:157) are written to store_points / store_colors [capacity,3] from row *cursor on (colors nullable:
+ * zeros are stored), *cursor advances by their number, and the per-axis minimum of their points_m is folded into
+ * min_out[3] (preset to +inf, as ps_voxel_min_bound).  When they do not all fit below capacity, nothing is written,
+ * *cursor stays and status |= 1.  points_scaled / points_m [N,3], keep [N] u8 and density [N] as ps_surface_hits and
+ * query_priors give them.  workspace: device memory of ps_hits_append_workspace(N) bytes.  No host synchronisation. */
+int ps_hits_append_workspace(int64_t N, int64_t* bytes);
+int ps_hits_append(const float* points_scaled, const float* points_m, const uint8_t* keep, const float* density,
+                   const float* colors, int64_t N, float* store_points, float* store_colors, int64_t capacity,
+                   int64_t* cursor, float* min_out, int* status, void* workspace, void* stream);
 
 /* Image metrics of rendered images: replace the torchmetrics calls of the reference model's `get_metrics_dict` and
  * `get_image_metrics_and_images` (models/PreSight/nerfacto_nusc_ms.py, as nerfstudio's models/nerfacto.py):

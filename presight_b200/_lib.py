@@ -72,6 +72,11 @@ SIGNATURES = {
     "ps_voxel_accumulate": [_p, _p, _p, _p, _i64, _i, _p, C.c_double, _p, _i64, _p, _p, _p, _p, _p, _p],
     "ps_voxel_finalize": [_p, _i64, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p],
     "ps_hits_quantile": [_p, _i64, C.c_double, _p, _i64, _p, _p, _p],
+    "ps_voxel_insert": [_p, _i64, _p, C.c_double, _p, _i64, _p, _p, _p],
+    "ps_voxel_rehash": [_p, _i64, _p, _i64, _p, _p],
+    "ps_voxel_assign_rows": [_p, _i64, _p, _i64, _p, _p, _p],
+    "ps_voxel_accumulate_rows": [_p, _p, _p, _i64, _i, _p, C.c_double, _p, _p, _i64, _p, _p, _p, _p, _p, _p],
+    "ps_voxel_finalize_rows": [_p, _p, _p, _p, _i64, _i, _p, _p, _p, _p, _p],
     "ps_generate_rays": [_p, _p, _p, _p, _p, _i, _p, _i64, _f, _p, _p, _p, _p, _p],
     "ps_assemble_batch": [_p, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "ps_peer_alloc": [C.c_size_t, _p],
@@ -94,6 +99,8 @@ SIGNATURES = {
     "ps_density_level_fwd": [_p, _p, _p, _p, _i64, _i, _fp, _i, _p, _fp, _i, _i, _i, _p, _p],
     "ps_density_level_fwd_ms": [_p, _i, _p, _p, _p, _p, _i64, _p, _fp, _i, _i, _i, _p, _p],
     "ps_surface_hits": [_p, _p, _p, _i64, _f, _f, _f, _f, _p, _p, _p, _p],
+    "ps_hits_append_workspace": [_i64, _p],
+    "ps_hits_append": [_p, _p, _p, _p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _p],
     "ps_image_metrics_workspace": [_i, _i, _i, _p],
     "ps_image_metrics": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p, _p],
     "ps_lpips_workspace": [_i, _i, _i, _p],

@@ -101,8 +101,20 @@ __global__ void __launch_bounds__(256) voxel_accumulate_kernel(
     }
 }
 
-// occupied slots -> dense rows (arbitrary order; the caller orders them by key): key, centre of mass, colour mean,
-// feature mean (fp64 mean rounded once to fp16, as numpy's astype does), hits
+// centre of mass, colour mean, feature mean (fp64 mean rounded once to fp16, as numpy's astype does) of accumulator row
+// `s` into output row `row`; one warp
+__device__ __forceinline__ void write_means(uint64_t s, unsigned long long row, int lane, unsigned int count,
+                                           const double* __restrict__ sum_xyz, const double* __restrict__ sum_col,
+                                           const double* __restrict__ sum_feat, int C, float* __restrict__ out_xyz,
+                                           float* __restrict__ out_col, __half* __restrict__ out_feat) {
+    const double n = (double)count;
+    if (lane < 3) out_xyz[row * 3 + lane] = (float)(sum_xyz[s * 3 + lane] / n);
+    else if (lane < 6 && out_col) out_col[row * 3 + (lane - 3)] = (float)(sum_col[s * 3 + (lane - 3)] / n);
+    if (out_feat)
+        for (int c = lane; c < C; c += 32) out_feat[row * C + c] = __double2half(sum_feat[s * C + c] / n);
+}
+
+// occupied slots -> dense rows (arbitrary order; the caller orders them by key): key, means, hits
 __global__ void __launch_bounds__(256) voxel_finalize_kernel(
     const long long* __restrict__ keys, uint64_t cap, const unsigned int* __restrict__ cnt,
     const double* __restrict__ sum_xyz, const double* __restrict__ sum_col, const double* __restrict__ sum_feat, int C,
@@ -116,15 +128,126 @@ __global__ void __launch_bounds__(256) voxel_finalize_kernel(
         unsigned long long row = 0;
         if (lane == 0) row = atomicAdd(n_out, 1ull);
         row = __shfl_sync(0xffffffffu, row, 0);
-        const double n = (double)cnt[s];
         if (lane == 0) {
             out_keys[row] = key;
             out_hits[row] = (long long)cnt[s];
         }
-        if (lane < 3) out_xyz[row * 3 + lane] = (float)(sum_xyz[s * 3 + lane] / n);
-        else if (lane < 6 && out_col) out_col[row * 3 + (lane - 3)] = (float)(sum_col[s * 3 + (lane - 3)] / n);
-        if (out_feat)
-            for (int c = lane; c < C; c += 32) out_feat[row * C + c] = __double2half(sum_feat[s * C + c] / n);
+        write_means(s, row, lane, cnt[s], sum_xyz, sum_col, sum_feat, C, out_xyz, out_col, out_feat);
+    }
+}
+
+// ---- the tile voxelizer: a key table sized by the voxels, then dense rows in ascending key order ---------------------
+// Pass 1 inserts keys only (8 B per slot; the caller keeps the load factor <= 1/2 and grows the table with
+// ps_voxel_rehash).  Sealing ranks the sorted keys into a row array beside the table (4 B per slot).  Pass 2 looks each
+// point's row up and adds it to dense fp64 rows with the accumulate kernel's warp-per-point scheme.
+// status: |= 1 table full, |= 2 voxel index outside 21 bits per axis, |= 4 a point's voxel is not in the table.
+
+// slot of `key` (inserted if absent; *fresh = it was absent), or -1 when the table is full
+__device__ __forceinline__ long long table_insert(long long* __restrict__ keys, uint64_t cap_mask, long long key,
+                                                  bool& fresh) {
+    fresh = false;
+    uint64_t s = mix64((uint64_t)key) & cap_mask;
+    for (uint64_t probe = 0; probe <= cap_mask; ++probe) {
+        const long long seen = __ldcg(keys + s);                   // a set key never changes: no atomic needed to skip it
+        if (seen == key) return (long long)s;
+        if (seen == kEmptyKey) {
+            const long long prev = (long long)atomicCAS(reinterpret_cast<unsigned long long*>(keys + s),
+                                                        (unsigned long long)kEmptyKey, (unsigned long long)key);
+            if (prev == kEmptyKey) { fresh = true; return (long long)s; }
+            if (prev == key) return (long long)s;
+        }
+        s = (s + 1) & cap_mask;
+    }
+    return -1;
+}
+
+// slot of `key`, or -1 when it is not in the table
+__device__ __forceinline__ long long table_find(const long long* __restrict__ keys, uint64_t cap_mask, long long key) {
+    uint64_t s = mix64((uint64_t)key) & cap_mask;
+    for (uint64_t probe = 0; probe <= cap_mask; ++probe) {
+        const long long seen = keys[s];
+        if (seen == key) return (long long)s;
+        if (seen == kEmptyKey) return -1;
+        s = (s + 1) & cap_mask;
+    }
+    return -1;
+}
+
+__global__ void __launch_bounds__(256) voxel_insert_kernel(const float* __restrict__ pts, int64_t N,
+                                                           const float* __restrict__ min_pt, double voxel,
+                                                           long long* __restrict__ keys, uint64_t cap_mask,
+                                                           unsigned long long* __restrict__ n_voxels,
+                                                           int* __restrict__ status) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += stride) {
+        const float p[3] = {__ldg(pts + 3 * i), __ldg(pts + 3 * i + 1), __ldg(pts + 3 * i + 2)};
+        bool ok, fresh;
+        const long long key = voxel_key(p, min_pt, voxel, ok);
+        if (!ok) { atomicOr(status, 2); continue; }
+        if (table_insert(keys, cap_mask, key, fresh) < 0) atomicOr(status, 1);
+        else if (fresh) atomicAdd(n_voxels, 1ull);
+    }
+}
+
+__global__ void __launch_bounds__(256) voxel_rehash_kernel(const long long* __restrict__ old_keys, uint64_t old_cap,
+                                                           long long* __restrict__ keys, uint64_t cap_mask,
+                                                           int* __restrict__ status) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s < old_cap; s += stride) {
+        const long long key = old_keys[s];
+        bool fresh;
+        if (key != kEmptyKey && table_insert(keys, cap_mask, key, fresh) < 0) atomicOr(status, 1);
+    }
+}
+
+__global__ void __launch_bounds__(256) voxel_assign_rows_kernel(const long long* __restrict__ sorted_keys, int64_t V,
+                                                                const long long* __restrict__ keys, uint64_t cap_mask,
+                                                                int* __restrict__ rows, int* __restrict__ status) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < V; r += stride) {
+        const long long s = table_find(keys, cap_mask, sorted_keys[r]);
+        if (s < 0) atomicOr(status, 4);
+        else rows[s] = (int)r;
+    }
+}
+
+__global__ void __launch_bounds__(256) voxel_accumulate_rows_kernel(
+    const float* __restrict__ pts, const __half* __restrict__ feat, const float* __restrict__ col, int64_t N, int C,
+    const float* __restrict__ min_pt, double voxel, const long long* __restrict__ keys, const int* __restrict__ rows,
+    uint64_t cap_mask, unsigned int* __restrict__ cnt, double* __restrict__ sum_xyz, double* __restrict__ sum_col,
+    double* __restrict__ sum_feat, int* __restrict__ status) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < N; i += warps) {
+        const float p[3] = {__ldg(pts + 3 * i), __ldg(pts + 3 * i + 1), __ldg(pts + 3 * i + 2)};
+        long long row = -1;
+        if (lane == 0) {
+            bool ok;
+            const long long key = voxel_key(p, min_pt, voxel, ok);
+            const long long s = ok ? table_find(keys, cap_mask, key) : -1;
+            if (!ok) atomicOr(status, 2);
+            else if (s < 0) atomicOr(status, 4);
+            else row = rows[s];
+        }
+        row = __shfl_sync(0xffffffffu, row, 0);
+        if (row < 0) continue;
+        if (lane == 0) atomicAdd(cnt + row, 1u);
+        if (lane < 3) atomicAdd(sum_xyz + row * 3 + lane, (double)(lane == 0 ? p[0] : lane == 1 ? p[1] : p[2]));
+        else if (lane < 6 && col) atomicAdd(sum_col + row * 3 + (lane - 3), (double)__ldg(col + 3 * i + (lane - 3)));
+        if (feat)
+            for (int c = lane; c < C; c += 32) atomicAdd(sum_feat + row * C + c, (double)__half2float(feat[i * C + c]));
+    }
+}
+
+__global__ void __launch_bounds__(256) voxel_finalize_rows_kernel(
+    const unsigned int* __restrict__ cnt, const double* __restrict__ sum_xyz, const double* __restrict__ sum_col,
+    const double* __restrict__ sum_feat, int64_t V, int C, float* __restrict__ out_xyz, float* __restrict__ out_col,
+    __half* __restrict__ out_feat, long long* __restrict__ out_hits) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+    for (uint64_t r = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < (uint64_t)V; r += warps) {
+        if (lane == 0) out_hits[r] = (long long)cnt[r];
+        write_means(r, r, lane, cnt[r], sum_xyz, sum_col, sum_feat, C, out_xyz, out_col, out_feat);
     }
 }
 
@@ -210,6 +333,90 @@ extern "C" int ps_voxel_finalize(const int64_t* keys, int64_t capacity, const ui
         reinterpret_cast<unsigned long long*>(n_out), reinterpret_cast<long long*>(out_keys), out_xyz, out_col,
         reinterpret_cast<__half*>(out_feat_f16), reinterpret_cast<long long*>(out_hits));
     return check_launch("voxel_finalize");
+}
+
+static bool pow2_capacity(int64_t capacity) { return capacity >= 2 && (capacity & (capacity - 1)) == 0; }
+
+extern "C" int ps_voxel_insert(const float* points, int64_t N, const float* min_point, double voxel_size, int64_t* keys,
+                               int64_t capacity, uint64_t* n_voxels, int* status, void* stream) {
+    PS_REQUIRE(N >= 0, "voxel_insert: negative point count %lld", (long long)N);
+    if (N == 0) return 0;
+    PS_REQUIRE(points && min_point && keys && n_voxels && status, "voxel_insert: null pointer");
+    PS_REQUIRE(pow2_capacity(capacity), "voxel_insert: capacity %lld is not a power of two", (long long)capacity);
+    PS_REQUIRE(voxel_size > 0.0, "voxel_insert: voxel size must be positive");
+    int64_t blocks = cdiv(N, 256);
+    if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
+    voxel_insert_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        points, N, min_point, voxel_size, reinterpret_cast<long long*>(keys), (uint64_t)capacity - 1,
+        reinterpret_cast<unsigned long long*>(n_voxels), status);
+    return check_launch("voxel_insert");
+}
+
+extern "C" int ps_voxel_rehash(const int64_t* old_keys, int64_t old_capacity, int64_t* keys, int64_t capacity, int* status,
+                               void* stream) {
+    PS_REQUIRE(old_keys && keys && status, "voxel_rehash: null pointer");
+    PS_REQUIRE(pow2_capacity(old_capacity) && pow2_capacity(capacity) && capacity >= old_capacity,
+               "voxel_rehash: capacities %lld -> %lld must be powers of two that do not shrink", (long long)old_capacity,
+               (long long)capacity);
+    int64_t blocks = cdiv(old_capacity, 256);
+    if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
+    voxel_rehash_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const long long*>(old_keys), (uint64_t)old_capacity, reinterpret_cast<long long*>(keys),
+        (uint64_t)capacity - 1, status);
+    return check_launch("voxel_rehash");
+}
+
+extern "C" int ps_voxel_assign_rows(const int64_t* sorted_keys, int64_t V, const int64_t* keys, int64_t capacity,
+                                    int32_t* rows, int* status, void* stream) {
+    PS_REQUIRE(V >= 0 && V < (1ll << 31), "voxel_assign_rows: %lld voxels outside [0, 2^31)", (long long)V);
+    if (V == 0) return 0;
+    PS_REQUIRE(sorted_keys && keys && rows && status, "voxel_assign_rows: null pointer");
+    PS_REQUIRE(pow2_capacity(capacity) && capacity >= 2 * V, "voxel_assign_rows: capacity %lld for %lld voxels",
+               (long long)capacity, (long long)V);
+    int64_t blocks = cdiv(V, 256);
+    if (blocks > (int64_t)kNumSMs * 16) blocks = (int64_t)kNumSMs * 16;
+    voxel_assign_rows_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        reinterpret_cast<const long long*>(sorted_keys), V, reinterpret_cast<const long long*>(keys),
+        (uint64_t)capacity - 1, rows, status);
+    return check_launch("voxel_assign_rows");
+}
+
+extern "C" int ps_voxel_accumulate_rows(const float* points, const void* features_f16, const float* colors, int64_t N,
+                                        int C, const float* min_point, double voxel_size, const int64_t* keys,
+                                        const int32_t* rows, int64_t capacity, uint32_t* counts, double* sum_xyz,
+                                        double* sum_col, double* sum_feat, int* status, void* stream) {
+    PS_REQUIRE(N >= 0, "voxel_accumulate_rows: negative point count %lld", (long long)N);
+    if (N == 0) return 0;
+    PS_REQUIRE(points && min_point && keys && rows && counts && sum_xyz && status, "voxel_accumulate_rows: null pointer");
+    PS_REQUIRE(pow2_capacity(capacity), "voxel_accumulate_rows: capacity %lld is not a power of two", (long long)capacity);
+    PS_REQUIRE(voxel_size > 0.0, "voxel_accumulate_rows: voxel size must be positive");
+    PS_REQUIRE((features_f16 == nullptr) == (sum_feat == nullptr), "voxel_accumulate_rows: features and sum_feat go together");
+    PS_REQUIRE((colors == nullptr) == (sum_col == nullptr), "voxel_accumulate_rows: colors and sum_col go together");
+    PS_REQUIRE(features_f16 == nullptr || C >= 1, "voxel_accumulate_rows: bad feature width %d", C);
+    int64_t blocks = cdiv(N, 8);                                       // 8 warps (points) per CTA per pass
+    if (blocks > (int64_t)kNumSMs * 8) blocks = (int64_t)kNumSMs * 8;
+    voxel_accumulate_rows_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        points, reinterpret_cast<const __half*>(features_f16), colors, N, C, min_point, voxel_size,
+        reinterpret_cast<const long long*>(keys), rows, (uint64_t)capacity - 1, counts, sum_xyz, sum_col, sum_feat,
+        status);
+    return check_launch("voxel_accumulate_rows");
+}
+
+extern "C" int ps_voxel_finalize_rows(const uint32_t* counts, const double* sum_xyz, const double* sum_col,
+                                      const double* sum_feat, int64_t V, int C, float* out_xyz, float* out_col,
+                                      void* out_feat_f16, int64_t* out_hits, void* stream) {
+    PS_REQUIRE(V >= 0, "voxel_finalize_rows: negative row count %lld", (long long)V);
+    if (V == 0) return 0;
+    PS_REQUIRE(counts && sum_xyz && out_xyz && out_hits, "voxel_finalize_rows: null pointer");
+    PS_REQUIRE((sum_col == nullptr) == (out_col == nullptr) && (sum_feat == nullptr) == (out_feat_f16 == nullptr),
+               "voxel_finalize_rows: accumulators and outputs go together");
+    PS_REQUIRE(sum_feat == nullptr || C >= 1, "voxel_finalize_rows: bad feature width %d", C);
+    int64_t blocks = cdiv(V, 8);
+    if (blocks > (int64_t)kNumSMs * 8) blocks = (int64_t)kNumSMs * 8;
+    voxel_finalize_rows_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        counts, sum_xyz, sum_col, sum_feat, V, C, out_xyz, out_col, reinterpret_cast<__half*>(out_feat_f16),
+        reinterpret_cast<long long*>(out_hits));
+    return check_launch("voxel_finalize_rows");
 }
 
 extern "C" int ps_hits_quantile(const int64_t* hits, int64_t M, double q, uint32_t* hist, int64_t bins, double* out,

@@ -8,7 +8,9 @@ rounded to fp16, hit count, then the hit-quantile filter — and the result is w
 `{points f32, features f16, colors f32, hits, origin f32}` the occupancy / online-mapping plugins read.
 
 `PriorVoxelizer` is the streaming form (one `add()` per camera / chunk once the bound is known); `postprocess_priors`
-is the one-shot form over resident arrays.  CUDA tensors only — no CPU fallback (the CPU restatement is oracle/).
+is the one-shot form over resident arrays.  Both size their table by the number of points.  `TileVoxelizer` gives the
+same result in two passes with a table sized by the number of voxels, for a whole tile's hits (`extract.PriorExtractor`).
+CUDA tensors only — no CPU fallback (the CPU restatement is oracle/).
 """
 from __future__ import annotations
 
@@ -99,6 +101,117 @@ class PriorVoxelizer:
         sel = order[keep]
         return {"points": oxyz[:m][sel], "features": None if ofeat is None else ofeat[:m][sel],
                 "colors": None if ocol is None else ocol[:m][sel], "hits": hits[keep], "hit_thr": thr[0], "n_voxels": m}
+
+
+_TABLE_STATUS = {1: "the voxel key table is full", 2: "a voxel index exceeds 21 bits per axis (tile larger than 2^21 "
+                 "voxels across)", 4: "a point reached pass 2 whose voxel was not inserted in pass 1"}
+
+
+class TileVoxelizer:
+    """`PriorVoxelizer`'s result for a whole tile in memory that follows the number of voxels V, not of points.
+
+    Two passes over the same points (metres, f32), the lattice anchored at `min_point` as in `PriorVoxelizer`:
+        insert(points)                       pass 1, keys only (12 B per table slot, load factor <= 1/2): before each slice
+                                             of P points the table grows to >= 2 (V + P) slots (one host read per slice)
+        seal()                               sorts the V keys; row r of the accumulators is the r-th smallest key
+        accumulate(points, feats, colors)    pass 2: each point is added to its voxel's dense fp64 row (572 B per row)
+        finalize(hit_thr_ratio)              -> the dict of `PriorVoxelizer.finalize`, rows already in ascending key order
+    Peak device memory: the table, V accumulator rows and V output rows (168 B each), and the caller's slice."""
+
+    def __init__(self, min_point: Tensor, voxel_size: float = 0.4, feature_dim: int = 64, with_colors: bool = True,
+                 capacity: int = 1 << 16) -> None:
+        assert min_point.is_cuda and min_point.numel() == 3, "min_point: 3 floats on the GPU"
+        self.dev, self.voxel_size, self.C, self.with_colors = min_point.device, float(voxel_size), int(feature_dim), with_colors
+        self.min_point = min_point.detach().to(torch.float32).contiguous()
+        self.capacity = _next_pow2(capacity)
+        self.keys = torch.full((self.capacity,), -1, device=self.dev, dtype=torch.int64)
+        self._n_voxels = torch.zeros(1, device=self.dev, dtype=torch.int64)
+        self.status = torch.zeros(1, device=self.dev, dtype=torch.int32)
+        self.rows: Optional[Tensor] = None              # slot -> row, after seal()
+        self.row_keys: Optional[Tensor] = None          # the V keys in ascending order, after seal()
+        self.counts = self.sum_xyz = self.sum_col = self.sum_feat = None
+
+    def _check(self, what: str) -> None:
+        st = int(self.status.item())
+        for bit, msg in _TABLE_STATUS.items():
+            if st & bit:
+                raise RuntimeError(f"TileVoxelizer.{what}: {msg}")
+
+    def insert(self, points_m: Tensor) -> None:
+        """Pass 1: the voxel keys of points [P,3] f32 metres."""
+        assert self.rows is None, "TileVoxelizer.insert after seal()"
+        p = points_m.detach().to(torch.float32).contiguous()
+        P = p.shape[0]
+        if P == 0:
+            return
+        need = 2 * (int(self._n_voxels.item()) + P)
+        if self.capacity < need:
+            cap = _next_pow2(need)
+            keys = torch.full((cap,), -1, device=self.dev, dtype=torch.int64)
+            call("ps_voxel_rehash", ptr(self.keys), self.capacity, ptr(keys), cap, ptr(self.status), stream())
+            self.keys, self.capacity = keys, cap
+        call("ps_voxel_insert", ptr(p), P, ptr(self.min_point), self.voxel_size, ptr(self.keys), self.capacity,
+             ptr(self._n_voxels), ptr(self.status), stream())
+
+    @property
+    def n_voxels(self) -> int:
+        return int(self._n_voxels.item())
+
+    def seal(self) -> None:
+        """Ends pass 1: ranks the keys and allocates the V accumulator rows."""
+        assert self.rows is None, "TileVoxelizer.seal twice"
+        self._check("seal")
+        V = self.n_voxels
+        if V == 0:
+            raise RuntimeError("TileVoxelizer: no point was inserted")
+        self.row_keys = torch.sort(self.keys[self.keys >= 0]).values
+        assert self.row_keys.numel() == V
+        self.rows = torch.empty(self.capacity, device=self.dev, dtype=torch.int32)
+        call("ps_voxel_assign_rows", ptr(self.row_keys), V, ptr(self.keys), self.capacity, ptr(self.rows),
+             ptr(self.status), stream())
+        z = lambda *s: torch.zeros(*s, device=self.dev, dtype=torch.float64)
+        self.counts = torch.zeros(V, device=self.dev, dtype=torch.int32)          # u32 on the device
+        self.sum_xyz = z(V, 3)
+        self.sum_col = z(V, 3) if self.with_colors else None
+        self.sum_feat = z(V, self.C) if self.C else None
+
+    def accumulate(self, points_m: Tensor, features: Optional[Tensor], colors: Optional[Tensor]) -> None:
+        """Pass 2: points [P,3] f32 metres (each inserted in pass 1), features [P,C] f16, colors [P,3] f32."""
+        assert self.rows is not None, "TileVoxelizer.accumulate before seal()"
+        p = points_m.detach().to(torch.float32).contiguous()
+        f = None if self.sum_feat is None else features.detach().to(torch.float16).contiguous()
+        c = None if self.sum_col is None else colors.detach().to(torch.float32).contiguous()
+        assert f is None or f.shape == (p.shape[0], self.C)
+        assert c is None or c.shape == (p.shape[0], 3)
+        call("ps_voxel_accumulate_rows", ptr(p), ptr(f), ptr(c), p.shape[0], self.C, ptr(self.min_point),
+             self.voxel_size, ptr(self.keys), ptr(self.rows), self.capacity, ptr(self.counts), ptr(self.sum_xyz),
+             ptr(self.sum_col), ptr(self.sum_feat), ptr(self.status), stream())
+
+    def finalize(self, hit_thr_ratio: float = 0.2) -> Dict[str, Tensor]:
+        """-> the dict of `PriorVoxelizer.finalize` (voxels in ascending (ix, iy, iz) order, hit-quantile filtered).
+        Frees the table and the accumulators as it goes: the voxelizer is spent afterwards."""
+        assert self.rows is not None, "TileVoxelizer.finalize before seal()"
+        self._check("finalize")
+        self.keys = self.rows = None
+        dev, V, C = self.dev, self.row_keys.numel(), self.C
+        oxyz = torch.empty(V, 3, device=dev, dtype=torch.float32)
+        ocol = torch.empty(V, 3, device=dev, dtype=torch.float32) if self.sum_col is not None else None
+        ofeat = torch.empty(V, C, device=dev, dtype=torch.float16) if self.sum_feat is not None else None
+        hits = torch.empty(V, device=dev, dtype=torch.int64)
+        call("ps_voxel_finalize_rows", ptr(self.counts), ptr(self.sum_xyz), ptr(self.sum_col), ptr(self.sum_feat), V, C,
+             ptr(oxyz), ptr(ocol), ptr(ofeat), ptr(hits), stream())
+        self.counts = self.sum_xyz = self.sum_col = self.sum_feat = None
+        lo, hi = (int(v) for v in torch.stack(torch.aminmax(hits)).tolist())
+        if lo == 0:
+            raise RuntimeError("TileVoxelizer: a voxel of pass 1 received no point in pass 2")
+        bins = hi + 1
+        hist = torch.zeros(bins, device=dev, dtype=torch.int32)
+        thr = torch.zeros(1, device=dev, dtype=torch.float64)
+        status = torch.zeros(1, device=dev, dtype=torch.int32)
+        call("ps_hits_quantile", ptr(hits), V, float(hit_thr_ratio), ptr(hist), bins, ptr(thr), ptr(status), stream())
+        keep = hits.to(torch.float64) > thr                 # extract_priors.py:191
+        return {"points": oxyz[keep], "features": None if ofeat is None else ofeat[keep],
+                "colors": None if ocol is None else ocol[keep], "hits": hits[keep], "hit_thr": thr[0], "n_voxels": V}
 
 
 def postprocess_priors(points: Tensor, features: Tensor, colors: Tensor, densities: Optional[Tensor],
