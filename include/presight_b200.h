@@ -504,6 +504,64 @@ int ps_colormap_workspace(int M, int64_t HW, int64_t* bytes);
 int ps_colormap(const float* maps, int M, int64_t HW, const float* acc, const float* lut, void* workspace, float* out,
                 void* stream);
 
+/* Depth metrics of rendered depth maps against LiDAR depth (Eigen et al. / Monodepth convention), for one image of HW
+ * pixels and M in [1, 4] maps (e.g. the "depth" and "expected_depth" outputs):
+ *   pred_m = pred / pose_scale (fp32 IEEE division); valid pixels: min_m < target_m < max_m (0 = no LiDAR);
+ *   p = pred_m clamped to [min_m, max_m]; per map, over the valid pixels, terms in fp64 from the fp32 p and t:
+ *   out [M][8] f64 = abs_rel mean |p-t|/t, sq_rel mean (p-t)^2/t, rmse sqrt mean (p-t)^2, rmse_log sqrt mean (ln p -
+ *   ln t)^2, a1 / a2 / a3 the fraction with max(p/t, t/p) < 1.25^k, n_valid.  No valid pixel: NaN metrics, n_valid 0.
+ *   Definitions in presight_b200/csrc/depth_metrics_core.h.  pred [M][HW] fp32 (scene units), target_m [HW] fp32 metres.
+ *   pose_scale: host value, or pose_scale_dev (a device float, read on the device) when not NULL.
+ * workspace: device memory of ps_depth_metrics_workspace(M, HW) bytes.  Status 1 for M outside [1, 4], HW <= 0, a null
+ * pointer, pose_scale <= 0 (host value), or bounds outside 0 < min_m < max_m < inf.  No host synchronisation and no
+ * floating-point atomics: repeated calls are bit-identical. */
+int ps_depth_metrics_workspace(int M, int64_t HW, int64_t* bytes);
+int ps_depth_metrics(const float* pred, int M, int64_t HW, const float* target_m, float pose_scale,
+                     const float* pose_scale_dev, float min_m, float max_m, void* workspace, double* out, void* stream);
+
+/* Nearest-neighbour distances within a radius between two point clouds (accuracy / completeness of extracted priors
+ * against a LiDAR cloud), on a grid of cells of side r = `cell` over the reference set.  Build, per reference set
+ * points [M,3] f32 (M >= 1):
+ *   ps_nn_grid_bounds        bounds[6] (device; caller presets +inf x3, -inf x3) <- per-axis min, max
+ *   ps_nn_grid_cells_per_axis  cells[3] (host) <- floor((max - min) / r) + 1 per axis from bounds_host[6]; status 1 with
+ *                            a message when an axis needs more than 2^21 cells
+ *   ps_nn_grid_keys          keys [M] i64 <- (cx << 42) | (cy << 21) | cz, c = floor(((double)p - (double)min) / r); the
+ *                            same extent check
+ *   (the caller sorts the keys, keeping the permutation perm [M] i64)
+ *   ps_nn_grid_count_cells   *n_cells (device i64, caller presets 0) += the number of distinct sorted keys
+ *   ps_nn_grid_cells         cell_keys [capacity] i64 (caller presets -1), cell_ranges [capacity][2] i32 <- [start, end)
+ *                            of every cell in sorted order; points_sorted [M,3] <- points[perm]; capacity a power of two
+ *                            (>= 2 n_cells keeps probes short); status |= 1 table full, |= 2 a cell was lost.
+ * Query, for N query points [N,3] f32 (any N; chunks of one scoring run are consecutive calls):
+ *   ps_nn_grid_query         d = min over the grid's points of sqrt(((qx-px)^2 + (qy-py)^2) + (qz-pz)^2), every step in
+ *                            fp64 from the fp32 coordinates, or r when that is not < r; dist_out [N] f64 (nullable).  The
+ *                            call scores queries as blocks of PS_NN_BLOCK_QUERIES consecutive points: block_sums[first_block
+ *                            + b] f64 = sum of d, block_counts[(first_block + b) K + k] i64 = #(d < taus_host[k]),
+ *                            0 < taus_host[k] <= r, K <= PS_NN_MAX_TAUS.  A chunk that is not the last must hold a
+ *                            multiple of PS_NN_BLOCK_QUERIES points for the blocks to line up.
+ *   ps_nn_grid_reduce        mean[0] = sum of block_sums / n, counts[k] = sum of block_counts[.][k], fixed order.
+ * No floating-point atomics: repeated calls, and any chunking into whole blocks, give bit-identical results. */
+#define PS_NN_BLOCK_QUERIES 1024
+#define PS_NN_MAX_TAUS 8
+typedef struct ps_nn_grid {
+    const float* points;        /* [M,3] in cell order (points_sorted) */
+    const int64_t* cell_keys;   /* [capacity] */
+    const int32_t* cell_ranges; /* [capacity][2] */
+    int64_t capacity;
+    float origin[3];            /* the per-axis minimum the keys were computed from */
+    double cell;                /* r */
+} ps_nn_grid;
+int ps_nn_grid_bounds(const float* points, int64_t M, float* bounds, void* stream);
+int ps_nn_grid_cells_per_axis(const float* bounds_host, double cell, int64_t* cells);
+int ps_nn_grid_keys(const float* points, int64_t M, const float* bounds_host, double cell, int64_t* keys, void* stream);
+int ps_nn_grid_count_cells(const int64_t* sorted_keys, int64_t M, int64_t* n_cells, void* stream);
+int ps_nn_grid_cells(const float* points, const int64_t* perm, const int64_t* sorted_keys, int64_t M, int64_t* cell_keys,
+                     int32_t* cell_ranges, int64_t capacity, float* points_sorted, int* status, void* stream);
+int ps_nn_grid_query(const ps_nn_grid* grid, const float* queries, int64_t N, int64_t first_block, const double* taus_host,
+                     int K, double* dist_out, double* block_sums, int64_t* block_counts, void* stream);
+int ps_nn_grid_reduce(const double* block_sums, const int64_t* block_counts, int64_t nblocks, int K, int64_t n,
+                      double* mean, int64_t* counts, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Sub-field routing and the sub-field mode of the fused levels (SURVEY §8 a10).  Replace the nearest-centroid routers
  * fields/PreSight/ingp_field_ms.py:80-126, prop_density_field_ms.py:86-105 (cdist().argmin, then per sub-field a

@@ -107,6 +107,15 @@ SIGNATURES = {
     "ps_lpips": [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p],
     "ps_colormap_workspace": [_i, _i64, _p],
     "ps_colormap": [_p, _i, _i64, _p, _p, _p, _p, _p],
+    "ps_depth_metrics_workspace": [_i, _i64, _p],
+    "ps_depth_metrics": [_p, _i, _i64, _p, _f, _p, _f, _f, _p, _p, _p],
+    "ps_nn_grid_bounds": [_p, _i64, _p, _p],
+    "ps_nn_grid_cells_per_axis": [_fp, C.c_double, _p],
+    "ps_nn_grid_keys": [_p, _i64, _fp, C.c_double, _p, _p],
+    "ps_nn_grid_count_cells": [_p, _i64, _p, _p],
+    "ps_nn_grid_cells": [_p, _p, _p, _i64, _p, _p, _i64, _p, _p, _p],
+    "ps_nn_grid_query": [_p, _p, _i64, _i64, C.POINTER(C.c_double), _i, _p, _p, _p, _p],
+    "ps_nn_grid_reduce": [_p, _p, _i64, _i, _i64, _p, _p, _p],
 }
 _RESTYPES = {"ps_last_error": C.c_char_p, "ps_abi_version": C.c_int, "ps_launch_count": C.c_int64}
 
@@ -245,6 +254,16 @@ class FieldNetDev(C.Structure):
 class LpipsNet(C.Structure):
     """ps_lpips_net of include/presight_b200.h."""
     _fields_ = [("conv_w", C.c_void_p * 5), ("conv_b", C.c_void_p * 5), ("lin", C.c_void_p * 5)]
+
+
+NN_BLOCK_QUERIES = 1024    # PS_NN_BLOCK_QUERIES
+NN_MAX_TAUS = 8            # PS_NN_MAX_TAUS
+
+
+class NNGrid(C.Structure):
+    """ps_nn_grid of include/presight_b200.h."""
+    _fields_ = [("points", C.c_void_p), ("cell_keys", C.c_void_p), ("cell_ranges", C.c_void_p),
+                ("capacity", C.c_int64), ("origin", C.c_float * 3), ("cell", C.c_double)]
 
 
 _DEV_TABLES = {}

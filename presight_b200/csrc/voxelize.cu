@@ -11,13 +11,11 @@
 // and features to the slot's fp64 accumulators with native double atomics.  Sums of fp16 features in fp64 are exact
 // (11-bit mantissas, < 2^40 points), so the feature means are independent of the accumulation order; coordinates and
 // colours are order-independent to ~1e-16 relative.  The table lives in caller-owned buffers.
-#include "common.cuh"
+#include "key_table.cuh"
 
 #include <cuda_fp16.h>
 
 namespace ps {
-
-constexpr long long kEmptyKey = -1;
 
 __device__ __forceinline__ bool point_selected(const float* __restrict__ dens, int64_t i) {
     return dens == nullptr || __ldg(dens + i) > 1.0f;
@@ -38,13 +36,6 @@ __global__ void __launch_bounds__(256) voxel_min_kernel(const float* __restrict_
         m[a] = warp_min(m[a]);
         if ((threadIdx.x & 31) == 0 && m[a] != INFINITY) atomic_min_float(out + a, m[a]);
     }
-}
-
-__device__ __forceinline__ uint64_t mix64(uint64_t k) {   // splitmix64 finaliser
-    k ^= k >> 30; k *= 0xbf58476d1ce4e5b9ull;
-    k ^= k >> 27; k *= 0x94d049bb133111ebull;
-    k ^= k >> 31;
-    return k;
 }
 
 // voxel index of a point exactly as open3d computes it: doubles, bound shifted by half a voxel, floor
@@ -141,37 +132,6 @@ __global__ void __launch_bounds__(256) voxel_finalize_kernel(
 // ps_voxel_rehash).  Sealing ranks the sorted keys into a row array beside the table (4 B per slot).  Pass 2 looks each
 // point's row up and adds it to dense fp64 rows with the accumulate kernel's warp-per-point scheme.
 // status: |= 1 table full, |= 2 voxel index outside 21 bits per axis, |= 4 a point's voxel is not in the table.
-
-// slot of `key` (inserted if absent; *fresh = it was absent), or -1 when the table is full
-__device__ __forceinline__ long long table_insert(long long* __restrict__ keys, uint64_t cap_mask, long long key,
-                                                  bool& fresh) {
-    fresh = false;
-    uint64_t s = mix64((uint64_t)key) & cap_mask;
-    for (uint64_t probe = 0; probe <= cap_mask; ++probe) {
-        const long long seen = __ldcg(keys + s);                   // a set key never changes: no atomic needed to skip it
-        if (seen == key) return (long long)s;
-        if (seen == kEmptyKey) {
-            const long long prev = (long long)atomicCAS(reinterpret_cast<unsigned long long*>(keys + s),
-                                                        (unsigned long long)kEmptyKey, (unsigned long long)key);
-            if (prev == kEmptyKey) { fresh = true; return (long long)s; }
-            if (prev == key) return (long long)s;
-        }
-        s = (s + 1) & cap_mask;
-    }
-    return -1;
-}
-
-// slot of `key`, or -1 when it is not in the table
-__device__ __forceinline__ long long table_find(const long long* __restrict__ keys, uint64_t cap_mask, long long key) {
-    uint64_t s = mix64((uint64_t)key) & cap_mask;
-    for (uint64_t probe = 0; probe <= cap_mask; ++probe) {
-        const long long seen = keys[s];
-        if (seen == key) return (long long)s;
-        if (seen == kEmptyKey) return -1;
-        s = (s + 1) & cap_mask;
-    }
-    return -1;
-}
 
 __global__ void __launch_bounds__(256) voxel_insert_kernel(const float* __restrict__ pts, int64_t N,
                                                            const float* __restrict__ min_pt, double voxel,

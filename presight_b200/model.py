@@ -501,13 +501,27 @@ class NerfactoNuscMSModel(nn.Module):
         prediction side by side [H,2W,3], "accumulation", "depth"}).  One host read for the numbers.  LPIPS scores the
         render clamped to [0,1], as the reference does.  With `self.colormap` unset the images are raw [H,W,1]; with it
         set they are the reference's colormapped [H,W,3] images, `prop_depth_{i}` of every proposal iteration included,
-        all from one `ps_colormap` call (`metrics.colormap_images`)."""
+        all from one `ps_colormap` call (`metrics.colormap_images`).
+        When the batch holds a LiDAR depth image "depth" ([H,W] or [H,W,1], metres, 0 = no return), the numbers also
+        hold `depth_{m}` and `expected_depth_{m}` for m in abs_rel, sq_rel, rmse, rmse_log, a1, a2, a3: the depth errors
+        of the "depth" and "expected_depth" outputs (`geometry.depth_metrics` with 1 m < target <
+        `lidar_depth_upperbound`, NaN without a valid pixel).  They need `pose_scale_factor` in the batch (KeyError
+        otherwise)."""
         from . import metrics
         gt, pred = batch["rgb"].to(outputs["rgb"].device), outputs["rgb"]
         psnr, ssim, _ = metrics.image_metrics(pred, gt)
         vals = [psnr[0].double(), ssim[0]]
         if self.lpips is not None:
             vals.append(self.lpips(pred.clamp(0.0, 1.0), gt))
+        depth_names = []
+        if "depth" in batch:
+            from . import geometry
+            names = [n for n in geometry.DEPTH_METRICS if n != "n_valid"]
+            dm = geometry.depth_metrics([outputs["depth"], outputs["expected_depth"]],
+                                        batch["depth"].to(pred.device), self._pose_scale_factor(None, batch),
+                                        1.0, self.config.lidar_depth_upperbound)
+            depth_names = [f"{p}_{n}" for p in ("depth", "expected_depth") for n in names]
+            vals.extend(dm[:, :len(names)].reshape(-1))
         images_dict = {"img": torch.cat([gt, pred], dim=1), "accumulation": outputs["accumulation"],
                        "depth": outputs["depth"]}
         if self.colormap is not None:
@@ -519,6 +533,7 @@ class NerfactoNuscMSModel(nn.Module):
         metrics_dict = {"psnr": float(vals[0]), "ssim": float(vals[1])}
         if self.lpips is not None:
             metrics_dict["lpips"] = float(vals[2])
+        metrics_dict.update(zip(depth_names, (float(v) for v in vals[len(vals) - len(depth_names):])))
         return metrics_dict, images_dict
 
     @torch.no_grad()
