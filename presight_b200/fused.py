@@ -357,9 +357,11 @@ class _FieldLevel(torch.autograd.Function):
         d_rgb_s = torch.empty(P, 3, device=dev, dtype=torch.float32)
         d_sem_s = torch.empty(P, C, device=dev, dtype=torch.float32) if C else None
         with ops._probe("composite_bwd"):
+            # converted upstream gradients bound to names: ptr() keeps only an address, and a copy freed before the
+            # launch may be handed to the next one of the argument list
+            g = [_f32c(dw).view(N, S), _f32c(drgb), _f32c(dacc), _f32c(ddexp), _f32c(dsem) if C else None]
             call("ps_composite_bwd", ptr(eu), ptr(density), ptr(rgb_s), ptr(sem_s), None, ptr(acc), ptr(dexp), N, S, C,
-                 ptr(_f32c(dw).view(N, S)), ptr(_f32c(drgb)), ptr(_f32c(dacc)), ptr(_f32c(ddexp)),
-                 ptr(_f32c(dsem)) if C else None, ptr(d_density), ptr(d_rgb_s), ptr(d_sem_s), stream())
+                 *map(ptr, g), ptr(d_density), ptr(d_rgb_s), ptr(d_sem_s), stream())
         # dh: column 0 is driven by d_density inside the base backward; [1, 1+geo) by the colour head;
         # [1+geo, ...) by the semantic head (zero when there is none)
         dh = torch.empty(P, hd, device=dev, dtype=torch.float32) if sem is not None \
@@ -800,12 +802,14 @@ class _FieldLevelMS(torch.autograd.Function):
             t = _f32c(t)
             return t if shape is None else t.view(shape)
         d_density = torch.empty(P, device=dev, dtype=torch.float32)
-        d_rgb_s = torch.empty(P, 3, device=dev, dtype=torch.float32)
-        d_sem_s = torch.empty(P, 64, device=dev, dtype=torch.float32)
+        # the compositing backward writes d_rgb_s / d_sem_s only when their upstream gradient is given, and the sub-field
+        # kernel reads both: a loss without colour (or semantics) must hand it zeros
+        d_rgb_s = (torch.empty if drgb is not None else torch.zeros)(P, 3, device=dev, dtype=torch.float32)
+        d_sem_s = (torch.empty if dsem is not None else torch.zeros)(P, 64, device=dev, dtype=torch.float32)
         with ops._probe("composite_bwd"):
+            g = [opt(dw, (N, S)), opt(drgb), opt(dacc), opt(ddexp), opt(dsem)]     # alive until the launch
             call("ps_composite_bwd", ptr(eu), ptr(density), ptr(rgb_s), ptr(sem_s), None, ptr(acc), ptr(dexp), N, S, 64,
-                 ptr(opt(dw, (N, S))), ptr(opt(drgb)), ptr(opt(dacc)), ptr(opt(ddexp)), ptr(opt(dsem)), ptr(d_density),
-                 ptr(d_rgb_s), ptr(d_sem_s), stream())
+                 *map(ptr, g), ptr(d_density), ptr(d_rgb_s), ptr(d_sem_s), stream())
         grads = _zeros_like_many([t for s in subs for t in s])
         gsub = [grads[PER * k:PER * (k + 1)] for k in range(nf)]
         slot = ("field", subs[0][0].data_ptr())

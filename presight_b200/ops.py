@@ -161,7 +161,10 @@ def sample_positions(origins: Tensor, dirs: Tensor, eu_bins: Tensor) -> Tensor:
     """Frustum mid-points [N,S,3] (cameras/rays.py:49-58)."""
     N, S = eu_bins.shape[0], eu_bins.shape[1] - 1
     pos = torch.empty(N, S, 3, device=eu_bins.device, dtype=torch.float32)
-    call("ps_sample_positions", ptr(_f32c(origins)), ptr(_f32c(dirs)), ptr(_f32c(eu_bins)), N, S, ptr(pos), stream())
+    # converted copies bound to names: ptr() keeps only an address, and a copy freed before the launch may be handed to
+    # the next one of the argument list
+    o, d, eu = _f32c(origins), _f32c(dirs), _f32c(eu_bins)
+    call("ps_sample_positions", ptr(o), ptr(d), ptr(eu), N, S, ptr(pos), stream())
     return pos
 
 
@@ -344,9 +347,9 @@ def pdf_resample(weights: Tensor, sp_in: Tensor, num_samples: int, rand: Optiona
     cdf = torch.empty(N, S_in + 1, device=dev, dtype=torch.float32) if probes else None
     u = torch.empty(N, nb, device=dev, dtype=torch.float32) if probes else None
     r = None if rand is None else _f32c(rand).view(-1)
-    call("ps_pdf_resample", ptr(w), ptr(_f32c(sp_in.detach())), ptr(u_base), ptr(r), ptr(_f32c(nears).view(-1)),
-         ptr(_f32c(fars).view(-1)), N, S_in, num_samples, float(padding), float(eps), float(anneal), float(thr),
-         ptr(sp_out), ptr(eu_out), ptr(inds), ptr(cdf), ptr(u), stream())
+    sp, nr, fr = _f32c(sp_in.detach()), _f32c(nears).view(-1), _f32c(fars).view(-1)     # alive until the launch
+    call("ps_pdf_resample", ptr(w), ptr(sp), ptr(u_base), ptr(r), ptr(nr), ptr(fr), N, S_in, num_samples,
+         float(padding), float(eps), float(anneal), float(thr), ptr(sp_out), ptr(eu_out), ptr(inds), ptr(cdf), ptr(u), stream())
     return (sp_out, eu_out, inds, cdf, u) if probes else (sp_out, eu_out)
 
 
@@ -465,9 +468,10 @@ class _Composite(torch.autograd.Function):
 
         def opt(t):
             return None if t is None else _f32c(t)
-        call("ps_composite_bwd", ptr(b), ptr(s), ptr(r), ptr(m), None, ptr(acc), ptr(dexp), N, S, C,
-             ptr(opt(dw)), ptr(opt(drgb) if has_rgb else None), ptr(opt(dacc)), ptr(opt(ddexp)),
-             ptr(opt(dsem) if has_sem else None), ptr(d_density), ptr(d_rgb), ptr(d_sem), stream())
+        # converted upstream gradients bound to names: alive until the launch (see sample_positions)
+        g = [opt(dw), opt(drgb) if has_rgb else None, opt(dacc), opt(ddexp), opt(dsem) if has_sem else None]
+        call("ps_composite_bwd", ptr(b), ptr(s), ptr(r), ptr(m), None, ptr(acc), ptr(dexp), N, S, C, *map(ptr, g),
+             ptr(d_density), ptr(d_rgb), ptr(d_sem), stream())
         return None, d_density, d_rgb, d_sem, None
 
 

@@ -657,3 +657,24 @@ def test_tcgen05_operand_conventions(ops):
     want4 = torch.zeros(64, 16)
     want4[:, 3] = Xb.sum(0)
     assert_close(C4.cpu()[:64], want4, 1e-5, "column sums through a one-hot operand with zero K stride")
+
+
+def test_wrappers_keep_converted_inputs_alive():
+    """Inputs a wrapper converts (non-contiguous or not fp32) stay referenced until the kernel is enqueued: with several
+    conversions in one call, a copy freed early would have its block handed to the next one and be overwritten by it."""
+    from presight_b200 import ops
+    g = torch.Generator().manual_seed(0)
+    N, S = 4096, 32
+    o, d = torch.rand(N, 3, generator=g).to(DEV), torch.randn(N, 3, generator=g).to(DEV)
+    eu = (torch.rand(N, S + 1, generator=g) * 0.1 + 0.01).cumsum(-1).to(DEV)
+
+    def strided(t):                      # the same values as a column slice of a wider tensor: not contiguous
+        return torch.cat([t, t], dim=1)[:, :t.shape[1]]
+    assert torch.equal(ops.sample_positions(strided(o), strided(d), strided(eu)), ops.sample_positions(o, d, eu))
+    density = (torch.rand(N, S, generator=g) * 5).to(DEV).requires_grad_(True)
+    _, _, acc, dexp, _, _, _ = ops.composite(eu, density, None, None)
+    # expanded upstream gradients of equal shape (what `acc.sum()` hands back) are converted one after the other
+    ga, gd = torch.ones(1, 1, device=DEV).expand(N, 1), torch.full((1, 1), 0.5, device=DEV).expand(N, 1)
+    got = torch.autograd.grad([acc, dexp], density, [ga, gd], retain_graph=True)[0]
+    want = torch.autograd.grad([acc, dexp], density, [ga.contiguous(), gd.contiguous()])[0]
+    assert torch.equal(got, want)
