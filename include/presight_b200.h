@@ -281,7 +281,11 @@ int ps_depth_losses(const float* weights, const float* eu_bins, const float* ste
  * ps_voxel_finalize: occupied slots -> rows 0..*n_out-1 (caller-zeroed counter; row order arbitrary): out_keys (packed
  *   ix<<42 | iy<<21 | iz), out_xyz [.,3] = centre of mass, out_col [.,3], out_feat_f16 [.,C], out_hits.
  * ps_hits_quantile: out[0] = np.quantile(hits[0..M), q) (linear interpolation); hist [bins] u32 caller-zeroed scratch,
- *   bins > max(hits) (status |= 4 otherwise). */
+ *   bins > max(hits) (status |= 4 otherwise).  It is ps_hits_histogram followed by ps_hits_quantile_from_histogram.
+ * ps_hits_histogram: hist[h] += number of hits[i] == h, i < M (M may be 0); hist [bins] u32 caller-zeroed, bins >
+ *   max(hits) (status |= 4 otherwise).  Histograms of disjoint parts of a hit array may be summed.
+ * ps_hits_quantile_from_histogram: out[0] = np.quantile of the M >= 1 hit counts whose histogram is hist [bins] (the
+ *   result of ps_hits_quantile on them, bit for bit). */
 int ps_voxel_min_bound(const float* points, const float* densities, int64_t N, float* min_out, void* stream);
 int ps_voxel_accumulate(const float* points, const void* features_f16, const float* colors, const float* densities,
                         int64_t N, int C, const float* min_point, double voxel_size, int64_t* keys, int64_t capacity,
@@ -291,6 +295,8 @@ int ps_voxel_finalize(const int64_t* keys, int64_t capacity, const uint32_t* cou
                       float* out_xyz, float* out_col, void* out_feat_f16, int64_t* out_hits, void* stream);
 int ps_hits_quantile(const int64_t* hits, int64_t M, double q, uint32_t* hist, int64_t bins, double* out, int* status,
                      void* stream);
+int ps_hits_histogram(const int64_t* hits, int64_t M, uint32_t* hist, int64_t bins, int* status, void* stream);
+int ps_hits_quantile_from_histogram(const uint32_t* hist, int64_t bins, int64_t M, double q, double* out, void* stream);
 
 /* The tile voxelizer: the per-voxel means of ps_voxel_accumulate / ps_voxel_finalize in memory that follows the number of
  * voxels V, not of points.  Two passes over the points, with the same voxel key as ps_voxel_accumulate:
@@ -320,6 +326,21 @@ int ps_voxel_accumulate_rows(const float* points, const void* features_f16, cons
 int ps_voxel_finalize_rows(const uint32_t* counts, const double* sum_xyz, const double* sum_col, const double* sum_feat,
                            int64_t V, int C, float* out_xyz, float* out_col, void* out_feat_f16, int64_t* out_hits,
                            void* stream);
+
+/* Owner partition of an extractor's stored hits, for one tile's extraction over `world` GPUs: a stable counting sort by
+ * the rank that owns each hit's voxel.
+ *   points_scaled / colors [N,3] fp32: stored hits (scene units) and their colours.  The voxel key is ps_voxel_insert's,
+ *   of the metre point points_scaled / pose_scale (IEEE division per component), on the lattice anchored at min_point [3]
+ *   (device) with voxel_size.  Owner of a key k: (splitmix64(k) >> 32) % world, splitmix64 the finaliser
+ *   z ^= z >> 30; z *= 0xbf58476d1ce4e5b9; z ^= z >> 27; z *= 0x94d049bb133111eb; z ^= z >> 31 on uint64.
+ *   -> out_points / out_colors [N,3]: the hits of owner 0, then of owner 1, ..., each owner's in input order;
+ *   counts [world] int64: hits per owner (written).  A key outside 21 bits per axis sets status |= 2 (as ps_voxel_insert;
+ *   the hit is still placed, by its masked key).  1 <= world <= 64; N may be 0 (counts are zeroed).
+ *   workspace: device memory of ps_voxel_partition_workspace(N, world) bytes.  No host synchronisation. */
+int ps_voxel_partition_workspace(int64_t N, int world, int64_t* bytes);
+int ps_voxel_partition(const float* points_scaled, const float* colors, int64_t N, float pose_scale,
+                       const float* min_point, double voxel_size, int world, float* out_points, float* out_colors,
+                       int64_t* counts, int* status, void* workspace, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Ray generation (SURVEY 8f-3): RayGenerator.forward + Cameras.generate_rays for PERSPECTIVE cameras without distortion

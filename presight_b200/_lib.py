@@ -72,11 +72,15 @@ SIGNATURES = {
     "ps_voxel_accumulate": [_p, _p, _p, _p, _i64, _i, _p, C.c_double, _p, _i64, _p, _p, _p, _p, _p, _p],
     "ps_voxel_finalize": [_p, _i64, _p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _p, _p],
     "ps_hits_quantile": [_p, _i64, C.c_double, _p, _i64, _p, _p, _p],
+    "ps_hits_histogram": [_p, _i64, _p, _i64, _p, _p],
+    "ps_hits_quantile_from_histogram": [_p, _i64, _i64, C.c_double, _p, _p],
     "ps_voxel_insert": [_p, _i64, _p, C.c_double, _p, _i64, _p, _p, _p],
     "ps_voxel_rehash": [_p, _i64, _p, _i64, _p, _p],
     "ps_voxel_assign_rows": [_p, _i64, _p, _i64, _p, _p, _p],
     "ps_voxel_accumulate_rows": [_p, _p, _p, _i64, _i, _p, C.c_double, _p, _p, _i64, _p, _p, _p, _p, _p, _p],
     "ps_voxel_finalize_rows": [_p, _p, _p, _p, _i64, _i, _p, _p, _p, _p, _p],
+    "ps_voxel_partition_workspace": [_i64, _i, _p],
+    "ps_voxel_partition": [_p, _p, _i64, _f, _p, C.c_double, _i, _p, _p, _p, _p, _p, _p],
     "ps_generate_rays": [_p, _p, _p, _p, _p, _i, _p, _i64, _f, _p, _p, _p, _p, _p],
     "ps_assemble_batch": [_p, _p, _p, _p, _p, _i, _p, _p, _p, _p, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "ps_peer_alloc": [C.c_size_t, _p],

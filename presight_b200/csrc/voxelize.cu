@@ -13,6 +13,8 @@
 // colours are order-independent to ~1e-16 relative.  The table lives in caller-owned buffers.
 #include "key_table.cuh"
 
+#include <cmath>
+
 #include <cuda_fp16.h>
 
 namespace ps {
@@ -211,6 +213,124 @@ __global__ void __launch_bounds__(256) voxel_finalize_rows_kernel(
     }
 }
 
+// ---- owner partition of stored hits (one tile's extraction over several GPUs) ---------------------------------------
+// A stable counting sort of the extractor's stored hits by owner rank, in two launches over G <= kPartMaxBlocks blocks,
+// each owning one contiguous span of hits (the pattern of ps_hits_append): (1) every block counts its hits per owner
+// into ws[r * G + b]; (2) every block sums, per owner, the counts of all blocks (the segment sizes, which block 0 writes
+// out) and of the blocks before it, then walks its span in tiles of 256 hits, ranking each owner's hits within a tile by
+// a warp match and per-warp counts.  Nothing reads a value written by the same launch: no host round trip, no spin-wait.
+constexpr int kPartThreads = 256;
+constexpr int kPartWarps = kPartThreads / 32;
+constexpr int kPartMaxBlocks = 1024;
+constexpr int64_t kPartMinSpan = 2048;
+constexpr int kPartMaxWorld = 64;
+
+// Owner rank of a voxel key: the high 32 bits of splitmix64(key), mod world.  Not the low bits: every rank's key table
+// places its keys by the low bits of the same hash, and a rank owns only keys of one residue.
+__device__ __forceinline__ int owner_of(long long key, int world) {
+    return (int)((mix64((uint64_t)key) >> 32) % (uint64_t)world);
+}
+
+// owner of stored hit i: its voxel key from the metre value TileVoxelizer.insert receives (an IEEE division of the
+// scene-unit point by the pose scale, as PriorExtractor.finalize computes it)
+__device__ __forceinline__ int hit_owner(const float* __restrict__ pts, int64_t i, float pose_scale,
+                                         const float* __restrict__ min_pt, double voxel, int world, bool& ok) {
+    const float p[3] = {__fdiv_rn(__ldg(pts + 3 * i), pose_scale), __fdiv_rn(__ldg(pts + 3 * i + 1), pose_scale),
+                        __fdiv_rn(__ldg(pts + 3 * i + 2), pose_scale)};
+    return owner_of(voxel_key(p, min_pt, voxel, ok), world);
+}
+
+__global__ void __launch_bounds__(kPartThreads) partition_count_kernel(
+    const float* __restrict__ pts, int64_t N, int64_t span, float pose_scale, const float* __restrict__ min_pt,
+    double voxel, int world, long long* __restrict__ ws, int* __restrict__ status) {
+    __shared__ int s_cnt[kPartMaxWorld];
+    const int G = gridDim.x, b = blockIdx.x, lane = threadIdx.x & 31;
+    for (int r = threadIdx.x; r < world; r += kPartThreads) s_cnt[r] = 0;
+    __syncthreads();
+    const int64_t lo = (int64_t)b * span, hi = min(N, lo + span);
+    bool bad = false;
+    for (int64_t t0 = lo; t0 < hi; t0 += kPartThreads) {         // block-uniform trip count: full-warp matches
+        const int64_t i = t0 + threadIdx.x;
+        bool ok = true;
+        const int o = i < hi ? hit_owner(pts, i, pose_scale, min_pt, voxel, world, ok) : -1;
+        bad |= !ok;
+        const unsigned peers = __match_any_sync(0xffffffffu, o);
+        if (o >= 0 && lane == __ffs(peers) - 1) atomicAdd(s_cnt + o, __popc(peers));
+    }
+    if (bad) atomicOr(status, 2);                                  // voxel index outside 21 bits per axis
+    __syncthreads();
+    for (int r = threadIdx.x; r < world; r += kPartThreads) ws[(int64_t)r * G + b] = s_cnt[r];
+}
+
+__global__ void __launch_bounds__(kPartThreads) partition_scatter_kernel(
+    const float* __restrict__ pts, const float* __restrict__ cols, int64_t N, int64_t span, float pose_scale,
+    const float* __restrict__ min_pt, double voxel, int world, const long long* __restrict__ ws,
+    float* __restrict__ out_pts, float* __restrict__ out_cols, long long* __restrict__ counts) {
+    __shared__ long long s_pre[kPartMaxWorld], s_tot[kPartMaxWorld];
+    __shared__ long long s_base[kPartMaxWorld];                    // next output row of each owner in this block
+    __shared__ int s_warp[kPartWarps][kPartMaxWorld];              // hits of each owner in each warp of the tile
+    const int G = gridDim.x, b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int r = warp; r < world; r += kPartWarps) {               // one warp per owner: its column of the counts
+        long long pre = 0, tot = 0;
+        for (int j = lane; j < G; j += 32) {
+            const long long c = ws[(int64_t)r * G + j];
+            tot += c;
+            pre += j < b ? c : 0;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            pre += __shfl_xor_sync(0xffffffffu, pre, o);
+            tot += __shfl_xor_sync(0xffffffffu, tot, o);
+        }
+        if (lane == 0) s_pre[r] = pre, s_tot[r] = tot;
+    }
+    for (int k = threadIdx.x; k < kPartWarps * kPartMaxWorld; k += kPartThreads) (&s_warp[0][0])[k] = 0;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        long long seg = 0;                                         // owner r's segment starts after owners < r
+        for (int r = 0; r < world; ++r) {
+            s_base[r] = seg + s_pre[r];
+            if (b == 0) counts[r] = s_tot[r];
+            seg += s_tot[r];
+        }
+    }
+    __syncthreads();
+    const int64_t lo = (int64_t)b * span, hi = min(N, lo + span);
+    for (int64_t t0 = lo; t0 < hi; t0 += kPartThreads) {
+        const int64_t i = t0 + threadIdx.x;
+        bool ok = true;
+        const int o = i < hi ? hit_owner(pts, i, pose_scale, min_pt, voxel, world, ok) : -1;
+        const unsigned peers = __match_any_sync(0xffffffffu, o);
+        if (o >= 0 && lane == __ffs(peers) - 1) s_warp[warp][o] = __popc(peers);
+        __syncthreads();
+        if (o >= 0) {
+            long long row = s_base[o] + __popc(peers & ((1u << lane) - 1u));
+            for (int w = 0; w < warp; ++w) row += s_warp[w][o];
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                out_pts[3 * row + a] = __ldg(pts + 3 * i + a);
+                out_cols[3 * row + a] = __ldg(cols + 3 * i + a);
+            }
+        }
+        __syncthreads();
+        for (int r = threadIdx.x; r < world; r += kPartThreads) {
+            long long t = 0;
+#pragma unroll
+            for (int w = 0; w < kPartWarps; ++w) {
+                t += s_warp[w][r];
+                s_warp[w][r] = 0;
+            }
+            s_base[r] += t;
+        }
+        __syncthreads();
+    }
+}
+
+int64_t partition_blocks(int64_t N) {
+    const int64_t g = cdiv(N, kPartMinSpan);
+    return g < 1 ? 1 : (g > kPartMaxBlocks ? kPartMaxBlocks : g);
+}
+
 // np.quantile(hits, q) (linear interpolation, numpy's _lerp) from a histogram of the hit counts; one CTA.
 __global__ void __launch_bounds__(1024) hits_hist_kernel(const long long* __restrict__ hits, int64_t M,
                                                           unsigned int* __restrict__ hist, int64_t bins,
@@ -379,16 +499,65 @@ extern "C" int ps_voxel_finalize_rows(const uint32_t* counts, const double* sum_
     return check_launch("voxel_finalize_rows");
 }
 
+extern "C" int ps_hits_histogram(const int64_t* hits, int64_t M, uint32_t* hist, int64_t bins, int* status,
+                                 void* stream) {
+    PS_REQUIRE(M >= 0, "hits_histogram: negative count %lld", (long long)M);
+    if (M == 0) return 0;
+    PS_REQUIRE(hits && hist && status, "hits_histogram: null pointer");
+    PS_REQUIRE(bins >= 1, "hits_histogram: no bins");
+    int64_t blocks = cdiv(M, 1024);
+    if (blocks > kNumSMs * 2) blocks = kNumSMs * 2;
+    hits_hist_kernel<<<(unsigned)blocks, 1024, 0, (cudaStream_t)stream>>>(reinterpret_cast<const long long*>(hits), M, hist,
+                                                                        bins, status);
+    return check_launch("hits_histogram");
+}
+
+extern "C" int ps_hits_quantile_from_histogram(const uint32_t* hist, int64_t bins, int64_t M, double q, double* out,
+                                               void* stream) {
+    PS_REQUIRE(hist && out, "hits_quantile_from_histogram: null pointer");
+    PS_REQUIRE(M >= 1 && bins >= 1, "hits_quantile_from_histogram: empty input");
+    PS_REQUIRE(q >= 0.0 && q <= 1.0, "hits_quantile_from_histogram: q = %f outside [0, 1]", q);
+    hits_quantile_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(hist, bins, M, q, out);
+    return check_launch("hits_quantile_from_histogram");
+}
+
 extern "C" int ps_hits_quantile(const int64_t* hits, int64_t M, double q, uint32_t* hist, int64_t bins, double* out,
                                 int* status, void* stream) {
     PS_REQUIRE(hits && hist && out && status, "hits_quantile: null pointer");
     PS_REQUIRE(M >= 1 && bins >= 2, "hits_quantile: empty input");
     PS_REQUIRE(q >= 0.0 && q <= 1.0, "hits_quantile: q = %f outside [0, 1]", q);
-    int64_t blocks = cdiv(M, 1024);
-    if (blocks > kNumSMs * 2) blocks = kNumSMs * 2;
-    hits_hist_kernel<<<(unsigned)blocks, 1024, 0, (cudaStream_t)stream>>>(reinterpret_cast<const long long*>(hits), M, hist,
-                                                                        bins, status);
-    if (int e = check_launch("hits_quantile(hist)")) return e;
-    hits_quantile_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(hist, bins, M, q, out);
-    return check_launch("hits_quantile");
+    if (int e = ps_hits_histogram(hits, M, hist, bins, status, stream)) return e;
+    return ps_hits_quantile_from_histogram(hist, bins, M, q, out, stream);
+}
+
+extern "C" int ps_voxel_partition_workspace(int64_t N, int world, int64_t* bytes) {
+    PS_REQUIRE(bytes, "voxel_partition_workspace: null pointer");
+    PS_REQUIRE(N >= 0, "voxel_partition_workspace: negative hit count %lld", (long long)N);
+    PS_REQUIRE(world >= 1 && world <= kPartMaxWorld, "voxel_partition_workspace: world %d outside [1, %d]", world,
+               kPartMaxWorld);
+    *bytes = partition_blocks(N) * world * (int64_t)sizeof(long long);
+    return 0;
+}
+
+extern "C" int ps_voxel_partition(const float* points_scaled, const float* colors, int64_t N, float pose_scale,
+                                  const float* min_point, double voxel_size, int world, float* out_points,
+                                  float* out_colors, int64_t* counts, int* status, void* workspace, void* stream) {
+    PS_REQUIRE(N >= 0, "voxel_partition: negative hit count %lld", (long long)N);
+    PS_REQUIRE(world >= 1 && world <= kPartMaxWorld, "voxel_partition: world %d outside [1, %d]", world, kPartMaxWorld);
+    PS_REQUIRE(counts && status && workspace, "voxel_partition: null pointer");
+    PS_REQUIRE(N == 0 || (points_scaled && colors && min_point && out_points && out_colors),
+               "voxel_partition: null pointer");
+    PS_REQUIRE(pose_scale > 0.f && std::isfinite(pose_scale), "voxel_partition: pose scale factor %g is not a positive "
+               "number", (double)pose_scale);
+    PS_REQUIRE(voxel_size > 0.0, "voxel_partition: voxel size must be positive");
+    const int64_t G = partition_blocks(N);                          // N == 0: one block writes zero counts
+    const int64_t span = cdiv(cdiv(N, G), kPartThreads) * kPartThreads;
+    auto* ws = reinterpret_cast<long long*>(workspace);
+    partition_count_kernel<<<(unsigned)G, kPartThreads, 0, (cudaStream_t)stream>>>(
+        points_scaled, N, span, pose_scale, min_point, voxel_size, world, ws, status);
+    if (int e = check_launch("voxel_partition(count)")) return e;
+    partition_scatter_kernel<<<(unsigned)G, kPartThreads, 0, (cudaStream_t)stream>>>(
+        points_scaled, colors, N, span, pose_scale, min_point, voxel_size, world, ws, out_points, out_colors,
+        reinterpret_cast<long long*>(counts));
+    return check_launch("voxel_partition");
 }

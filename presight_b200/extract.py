@@ -15,6 +15,10 @@ and height window, queries density and semantics there, drops hits with mean den
                 writes.  The 64-d features (128 B per hit) are never stored, and nothing grows with the number of hits
                 but the store itself.
 
+`ShardedPriorExtractor` spreads one tile's extraction over the GPUs of a process group: each rank adds its share of the
+rays, and finalize() moves every stored hit to the rank that owns its voxel (ps_voxel_partition + all_to_all_single),
+voxelises there, applies the hit threshold of all ranks' voxels and gathers the kept voxels on one rank.
+
 Pixel selection (image decoding, seg-mask filtering) stays with the caller, who hands rays built by
 `cameras.RayGenerator` from (camera, row, col) indices.
 """
@@ -24,6 +28,7 @@ import ctypes as C
 from typing import Dict, List, Optional, Tuple
 
 import torch
+import torch.distributed as dist
 from torch import Tensor
 
 from ._lib import call, check, load, ptr, stream
@@ -158,13 +163,16 @@ class PriorExtractor:
             raise RuntimeError("PriorExtractor: no surface hit passed the selector and the density filter")
         if int(self._status.item()) & 1:
             raise RuntimeError("PriorExtractor: a chunk's hits did not fit their store block")
-        filled = self._filled()
-        blocks = [(p[:k], c[:k]) for (p, c), k in zip(self._blocks, filled)]
-        vox = TileVoxelizer(self._min, self.voxel_size, self.model.config.semantic_dim,
-                            capacity=2 * min(self.insert_slice, sum(filled)))
+        blocks = [(p[:k], c[:k]) for (p, c), k in zip(self._blocks, self._filled())]
+        return self._voxelize(blocks, self._min).finalize(self.hit_thr_ratio)
+
+    def _voxelize(self, blocks: List[Tuple[Tensor, Tensor]], anchor: Tensor) -> TileVoxelizer:
+        """TileVoxelizer over stored hits (scene-unit points, colours), both passes done: ready to finalize."""
+        vox = TileVoxelizer(anchor, self.voxel_size, self.model.config.semantic_dim,
+                            capacity=2 * min(self.insert_slice, sum(p.shape[0] for p, _ in blocks)))
         # metres exactly as ps_surface_hits computes them: an element-wise IEEE division (torch turns a division by a
         # Python scalar into a multiplication by its reciprocal, which can differ in the last bit)
-        scale = torch.full((1, 3), self.pose_scale, device=self._min.device, dtype=torch.float32)
+        scale = torch.full((1, 3), self.pose_scale, device=anchor.device, dtype=torch.float32)
         for pts, _ in blocks:
             for i in range(0, pts.shape[0], self.insert_slice):
                 vox.insert(pts[i:i + self.insert_slice] / scale)
@@ -174,4 +182,176 @@ class PriorExtractor:
                 p = pts[i:i + self.chunk_rays]
                 _, feats = self.model.query_priors(p)
                 vox.accumulate(p / scale, feats, cols[i:i + self.chunk_rays])
-        return vox.finalize(self.hit_thr_ratio)
+        return vox
+
+
+class ShardedPriorExtractor(PriorExtractor):
+    """`PriorExtractor` for one tile over the GPUs of a `torch.distributed` group (NCCL, one GPU per rank).
+
+    Each rank `add()`s its own share of the tile's rays, in any split (`parallel.shard_range`, round-robin, or none at
+    all on some ranks).  `finalize(dst)` then returns, on rank `dst`, what `PriorExtractor.finalize` returns for all the
+    ranks' rays on one GPU -- the same voxels, hit counts, threshold and features; centres and colours up to the
+    rounding of their fp64 sums -- and None on the other ranks:
+        anchor      all-reduce MIN of the ranks' running minima (the lattice anchor is a per-axis minimum)
+        exchange    per store block: ps_voxel_partition packs the hits by the rank that owns their voxel (a hash of the
+                    voxel key), the counts are swapped (one host read) and the hits move with all_to_all_single; the
+                    block is freed.  `max over ranks` rounds of one block each, so a rank holds its store, one block's
+                    send buffer and the hits it owns
+        voxelize    TileVoxelizer over the owned hits: the ranks' voxel sets are disjoint, and each voxel gets all its
+                    hits on its owner
+        threshold   the hit quantile over the sum of the ranks' histograms of per-voxel hit counts
+        gather      the kept rows of every rank to `dst`, ordered by voxel key
+    group: the process group (None: the default one; world 1 when no process group is initialised).  The store is
+    released as it is exchanged: the extractor is spent after finalize()."""
+
+    def __init__(self, model, pose_scale_factor: float, voxel_size: float = 0.4, hit_thr_ratio: float = 0.2,
+                 max_range_m: Optional[float] = None, z_range_m: Optional[Tuple[Optional[float], Optional[float]]] = None,
+                 chunk_rays: int = 1 << 17, block_hits: int = 1 << 24, insert_slice: int = 1 << 24, group=None) -> None:
+        super().__init__(model, pose_scale_factor, voxel_size, hit_thr_ratio, max_range_m, z_range_m, chunk_rays,
+                         block_hits, insert_slice)
+        on = dist.is_available() and dist.is_initialized()
+        self.group = group
+        self.world = dist.get_world_size(group) if on else 1
+        self.rank = dist.get_rank(group) if on else 0
+        self.exchanged_bytes = 0                         # hits this rank sent to other ranks in finalize(), 24 B each
+
+    def _all_reduce(self, t: Tensor, op) -> Tensor:
+        if self.world > 1:
+            dist.all_reduce(t, op=op, group=self.group)
+        return t
+
+    def _all_gather(self, t: Tensor) -> List[int]:
+        """The ranks' int64 vectors `t`, concatenated in rank order, on the host."""
+        if self.world == 1:
+            return t.tolist()
+        out = torch.empty(self.world * t.numel(), device=t.device, dtype=t.dtype)
+        dist.all_gather_into_tensor(out, t, group=self.group)
+        return out.tolist()
+
+    def _peer(self, r: int) -> int:
+        return r if self.group is None else dist.get_global_rank(self.group, r)
+
+    @torch.no_grad()
+    def finalize(self, dst: int = 0) -> Optional[Dict[str, Tensor]]:
+        """-> on rank `dst`, the result dict of `PriorExtractor.finalize` for the rays of every rank; None elsewhere.
+        Every rank of the group calls it."""
+        assert 0 <= dst < self.world, f"dst {dst} is not a rank of a group of {self.world}"
+        anchor, rounds = self._anchor()
+        owned = self._exchange(anchor, rounds)
+        kept, n_voxels, thr = self._voxelize_owned(owned, anchor)
+        return self._gather(kept, n_voxels, thr, dst)
+
+    def _anchor(self) -> Tuple[Tensor, int]:
+        """The global lattice anchor and the number of exchange rounds; the same error on every rank when there is
+        nothing to voxelise or a store overflowed."""
+        dev = self._min.device if self._min is not None else torch.device("cuda", torch.cuda.current_device())
+        anchor = self._min.clone() if self._min is not None else torch.full((3,), float("inf"), device=dev)
+        self._all_reduce(anchor, dist.ReduceOp.MIN)
+        flags = torch.zeros(2, device=dev, dtype=torch.int64)          # store blocks, store status
+        flags[0] = len(self._blocks)
+        if self._status is not None:
+            flags[1] = self._status[0]
+        self._all_reduce(flags, dist.ReduceOp.MAX)
+        rounds, st = flags.tolist()
+        if bool(torch.isinf(anchor).any()):
+            raise RuntimeError("PriorExtractor: no surface hit passed the selector and the density filter")
+        if st & 1:
+            raise RuntimeError("PriorExtractor: a chunk's hits did not fit their store block")
+        return anchor, rounds
+
+    def _exchange(self, anchor: Tensor, rounds: int) -> List[Tuple[Tensor, Tensor]]:
+        """Moves every stored hit to the rank that owns its voxel -> the hits this rank owns (points, colours)."""
+        dev, W = anchor.device, self.world
+        filled = self._filled()
+        nbytes = C.c_int64()
+        check(load().ps_voxel_partition_workspace(self.block_hits, W, C.byref(nbytes)), "ps_voxel_partition_workspace")
+        ws = torch.empty(nbytes.value, device=dev, dtype=torch.uint8)
+        counts = torch.empty(W, device=dev, dtype=torch.int64)
+        recv_counts = torch.empty(W, device=dev, dtype=torch.int64)
+        status = torch.zeros(1, device=dev, dtype=torch.int32)
+        owned: List[Tuple[Tensor, Tensor]] = []
+        self.exchanged_bytes = 0
+        for i in range(rounds):
+            if i < len(self._blocks):                   # ranks with fewer blocks send empty rounds
+                n = filled[i]
+                pts, cols = (t[:n] for t in self._blocks[i])
+                self._blocks[i] = None
+            else:
+                n = 0
+                pts = cols = torch.empty(0, 3, device=dev)
+            send_p = torch.empty(n, 3, device=dev)
+            send_c = torch.empty(n, 3, device=dev)
+            call("ps_voxel_partition", ptr(pts), ptr(cols), n, self.pose_scale, ptr(anchor), self.voxel_size, W,
+                 ptr(send_p), ptr(send_c), ptr(counts), ptr(status), ptr(ws), stream())
+            del pts, cols                               # the store block goes back to the allocator
+            if W == 1:
+                owned.append((send_p, send_c))
+                continue
+            dist.all_to_all_single(recv_counts, counts, group=self.group)
+            split = torch.cat([counts, recv_counts]).tolist()
+            sent, recv = split[:W], split[W:]
+            recv_p = torch.empty(sum(recv), 3, device=dev)
+            recv_c = torch.empty(sum(recv), 3, device=dev)
+            dist.all_to_all_single(recv_p, send_p, recv, sent, group=self.group)
+            dist.all_to_all_single(recv_c, send_c, recv, sent, group=self.group)
+            self.exchanged_bytes += (sum(sent) - sent[self.rank]) * self.HIT_BYTES
+            owned.append((recv_p, recv_c))
+            del send_p, send_c
+        self._blocks, self._sealed = [], []
+        if int(self._all_reduce(status, dist.ReduceOp.MAX).item()) & 2:
+            raise RuntimeError("PriorExtractor: a voxel index exceeds 21 bits per axis (tile larger than 2^21 voxels "
+                               "across)")
+        return owned
+
+    def _voxelize_owned(self, owned: List[Tuple[Tensor, Tensor]], anchor: Tensor):
+        """TileVoxelizer over this rank's hits, filtered by the hit threshold of all ranks' voxels -> (kept rows,
+        voxels of all ranks, threshold [1] f64)."""
+        dev = anchor.device
+        if sum(p.shape[0] for p, _ in owned):
+            rows = self._voxelize(owned, anchor).finalize_rows()
+        else:                                           # this rank owns no voxel
+            C_ = self.model.config.semantic_dim
+            rows = {"keys": torch.empty(0, device=dev, dtype=torch.int64), "points": torch.empty(0, 3, device=dev),
+                    "features": torch.empty(0, C_, device=dev, dtype=torch.float16),
+                    "colors": torch.empty(0, 3, device=dev), "hits": torch.empty(0, device=dev, dtype=torch.int64)}
+        del owned
+        hits = rows["hits"]
+        V = hits.numel()
+        lo, hi = (int(v) for v in torch.stack(torch.aminmax(hits)).tolist()) if V else (1, 0)
+        if lo == 0:
+            raise RuntimeError("TileVoxelizer: a voxel of pass 1 received no point in pass 2")
+        per_rank = self._all_gather(torch.tensor([V, hi], device=dev, dtype=torch.int64))
+        n_voxels, bins = sum(per_rank[0::2]), max(per_rank[1::2]) + 1
+        hist = torch.zeros(bins, device=dev, dtype=torch.int32)        # u32 on the device
+        status = torch.zeros(1, device=dev, dtype=torch.int32)
+        call("ps_hits_histogram", ptr(hits), V, ptr(hist), bins, ptr(status), stream())
+        self._all_reduce(hist, dist.ReduceOp.SUM)
+        thr = torch.zeros(1, device=dev, dtype=torch.float64)
+        call("ps_hits_quantile_from_histogram", ptr(hist), bins, n_voxels, float(self.hit_thr_ratio), ptr(thr),
+             stream())
+        keep = hits.to(torch.float64) > thr             # extract_priors.py:191
+        return {k: v[keep] for k, v in rows.items()}, n_voxels, thr
+
+    def _gather(self, kept: Dict[str, Tensor], n_voxels: int, thr: Tensor, dst: int) -> Optional[Dict[str, Tensor]]:
+        """The kept rows of every rank -> rank `dst`, in ascending key order (None on the other ranks)."""
+        if self.world > 1:
+            K = self._all_gather(torch.tensor([kept["keys"].numel()], device=thr.device, dtype=torch.int64))
+            ops, parts = [], {}
+            for name, t in kept.items():
+                if self.rank == dst:
+                    parts[name] = [t if r == dst else torch.empty((K[r],) + tuple(t.shape[1:]), device=t.device,
+                                                                  dtype=t.dtype) for r in range(self.world)]
+                    ops += [dist.P2POp(dist.irecv, parts[name][r], self._peer(r), self.group)
+                            for r in range(self.world) if r != dst and K[r]]
+                elif K[self.rank]:
+                    ops.append(dist.P2POp(dist.isend, t, self._peer(dst), self.group))
+            if ops:
+                for req in dist.batch_isend_irecv(ops):
+                    req.wait()
+            if self.rank != dst:
+                return None
+            kept = {name: torch.cat(p) for name, p in parts.items()}
+            order = torch.argsort(kept["keys"])         # owners hold disjoint keys: a total order
+            kept = {name: t[order] for name, t in kept.items()}
+        return {"points": kept["points"], "features": kept["features"], "colors": kept["colors"],
+                "hits": kept["hits"], "hit_thr": thr[0], "n_voxels": n_voxels}

@@ -9,7 +9,8 @@ rounded to fp16, hit count, then the hit-quantile filter — and the result is w
 
 `PriorVoxelizer` is the streaming form (one `add()` per camera / chunk once the bound is known); `postprocess_priors`
 is the one-shot form over resident arrays.  Both size their table by the number of points.  `TileVoxelizer` gives the
-same result in two passes with a table sized by the number of voxels, for a whole tile's hits (`extract.PriorExtractor`).
+same result in two passes with a table sized by the number of voxels, for a whole tile's hits (`extract.PriorExtractor`;
+`finalize_rows` gives its rows before the filter, which `extract.ShardedPriorExtractor` applies across GPUs).
 CUDA tensors only — no CPU fallback (the CPU restatement is oracle/).
 """
 from __future__ import annotations
@@ -187,9 +188,10 @@ class TileVoxelizer:
              self.voxel_size, ptr(self.keys), ptr(self.rows), self.capacity, ptr(self.counts), ptr(self.sum_xyz),
              ptr(self.sum_col), ptr(self.sum_feat), ptr(self.status), stream())
 
-    def finalize(self, hit_thr_ratio: float = 0.2) -> Dict[str, Tensor]:
-        """-> the dict of `PriorVoxelizer.finalize` (voxels in ascending (ix, iy, iz) order, hit-quantile filtered).
-        Frees the table and the accumulators as it goes: the voxelizer is spent afterwards."""
+    def finalize_rows(self) -> Dict[str, Tensor]:
+        """-> every voxel's row before the hit-quantile filter, in ascending key order: {"keys" [V] i64 (packed
+        ix<<42 | iy<<21 | iz), "points", "features", "colors", "hits"} as `finalize` gives them.  Frees the table and
+        the accumulators as it goes: the voxelizer is spent afterwards."""
         assert self.rows is not None, "TileVoxelizer.finalize before seal()"
         self._check("finalize")
         self.keys = self.rows = None
@@ -201,6 +203,14 @@ class TileVoxelizer:
         call("ps_voxel_finalize_rows", ptr(self.counts), ptr(self.sum_xyz), ptr(self.sum_col), ptr(self.sum_feat), V, C,
              ptr(oxyz), ptr(ocol), ptr(ofeat), ptr(hits), stream())
         self.counts = self.sum_xyz = self.sum_col = self.sum_feat = None
+        return {"keys": self.row_keys, "points": oxyz, "features": ofeat, "colors": ocol, "hits": hits}
+
+    def finalize(self, hit_thr_ratio: float = 0.2) -> Dict[str, Tensor]:
+        """-> the dict of `PriorVoxelizer.finalize` (voxels in ascending (ix, iy, iz) order, hit-quantile filtered).
+        Frees the table and the accumulators as it goes: the voxelizer is spent afterwards."""
+        r = self.finalize_rows()
+        dev, hits, oxyz, ocol, ofeat = self.dev, r["hits"], r["points"], r["colors"], r["features"]
+        V = hits.numel()
         lo, hi = (int(v) for v in torch.stack(torch.aminmax(hits)).tolist())
         if lo == 0:
             raise RuntimeError("TileVoxelizer: a voxel of pass 1 received no point in pass 2")
