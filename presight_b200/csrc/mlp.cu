@@ -22,17 +22,7 @@ static int resolve(const int* dims, int n_layers, int& K0, int& H, int& NHID, in
 
 static int run(int K0, int H, int NHID, int NOUT, int prec, bool bwd, const MlpArgs& a, cudaStream_t s,
                const int* dims, int n_layers) {
-    if (a.lm_F > 0 && prec == 2) prec = 1;   // the tcgen05 forward reads row-major inputs only
-    PS_REQUIRE(prec >= 0 && prec <= 2, "mlp: precision %d (0 = tf32x3 fp32-grade, 1 = bf16 mma.sync, 2 = bf16 tcgen05)",
-               prec);
-    if (prec == 2) {
-        // Blackwell-native forward (tcgen05.mma + TMEM); the backward of this mode runs the bf16 mma.sync kernels
-        if (!bwd) {
-            const int r5 = dispatch_tc5_fwd(K0, H, NHID, NOUT, a, s);
-            if (r5 >= 0) return r5;
-        }
-        prec = 1;
-    }
+    PS_REQUIRE(prec >= 0 && prec <= 1, "mlp: precision %d (0 = tf32x3 fp32-grade, 1 = bf16 mma.sync)", prec);
     int r = dispatch_group0(K0, H, NHID, NOUT, prec, bwd, a, s);
     if (r < 0) r = dispatch_group1(K0, H, NHID, NOUT, prec, bwd, a, s);
     if (r < 0) r = dispatch_group2(K0, H, NHID, NOUT, prec, bwd, a, s);

@@ -21,9 +21,6 @@ int dispatch_group0(int K0, int H, int NHID, int NOUT, int prec, bool bwd, const
 int dispatch_group1(int K0, int H, int NHID, int NOUT, int prec, bool bwd, const MlpArgs& a, cudaStream_t s);
 int dispatch_group2(int K0, int H, int NHID, int NOUT, int prec, bool bwd, const MlpArgs& a, cudaStream_t s);
 
-// tcgen05 / TMEM forward (mlp_tc5.cu); -1 when the shape is not instantiated
-int dispatch_tc5_fwd(int K0, int H, int NHID, int NOUT, const MlpArgs& a, cudaStream_t s);
-
 #define PS_MLP_CASE(k0, h, nhid, nout)                                                       \
     if (K0 == k0 && H == h && NHID == nhid && NOUT == nout) {                                \
         using S = Shape<k0, h, nhid, nout>;                                                  \

@@ -576,12 +576,6 @@ static int launch(const PropArgs& a, bool bwd, cudaStream_t stream, const char* 
         if (occ > 8) occ = 8;
         if (occ < 1) occ = 1;
         ctas = occ < by_tmem ? occ : by_tmem;
-        // PS_PROP_BWD_MAX_CTAS: fewer resident CTAs per SM for the (persistent) backward, i.e. room for another kernel's
-        // CTAs on every SM for as long as it runs (data-parallel runs: the gradient exchange's kernels)
-        if (const char* cap = bwd ? getenv("PS_PROP_BWD_MAX_CTAS") : nullptr) {
-            const int c = atoi(cap);
-            if (c >= 1 && c < ctas) ctas = c;
-        }
         if (getenv("PS_DEBUG"))
             fprintf(stderr, "[prop_level %s H=%d F=%d K0=%d] smem %zu occ %d (%s) by_tmem %d -> %d CTAs/SM\n",
                     bwd ? "bwd" : "fwd", H, F, K0, smem, occ, cudaGetErrorString(e), by_tmem, ctas);

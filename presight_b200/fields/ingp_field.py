@@ -148,7 +148,7 @@ class iNGPField(Field):
         head fits the fused density kernels (fused.tc5_density_supported: bf16 class, hidden 64, L*F <= 48)."""
         from .. import fused
         ls = list(self.mlp_base_mlp.layers)
-        return (fused.USE_TC5_FIELD and len(ls) == 2 and all(l.bias is not None for l in ls)
+        return (len(ls) == 2 and all(l.bias is not None for l in ls)
                 and fused.tc5_density_supported(self._grid_meta(), ls[0].weight.shape[0], self.mlp_base_mlp.precision, S))
 
     def level_depth(self, origins: Tensor, directions: Tensor, eu_bins: Tensor, threshold: float = 0.5) -> Tensor:

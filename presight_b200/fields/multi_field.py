@@ -94,8 +94,7 @@ class iNGPFieldMS(nn.Module):
         base = fused.MlpMeta(dims(f0.mlp_base_mlp), f0.mlp_base_mlp._out_act)
         sem = fused.MlpMeta(dims(f0.semantic_head), f0.semantic_head._out_act)
         rgb = fused.MlpMeta(dims(f0.rgb_head), f0.rgb_head._out_act)
-        if not (fused.USE_TC5_FIELD and fused.tc5_field_supported(grid, base, sem, rgb, f0.geo_feat_dim,
-                                                                    f0.mlp_base_mlp.precision, 64, A)):
+        if not fused.tc5_field_supported(grid, base, sem, rgb, f0.geo_feat_dim, f0.mlp_base_mlp.precision, 64, A):
             return None
         for f in self.fields[1:]:
             e = f.mlp_base_grid
@@ -197,7 +196,7 @@ class PropNetDensityFieldMS(nn.Module):
         enc = f0.encoding
         grid = fused.GridMeta(enc._scalings_host, enc.log2_hashmap_size, enc.features_per_level)
         layers = list(f0.mlp_base[1].layers)
-        if not (fused.USE_TC5_PROP and len(layers) == 2 and layers[1].weight.shape[0] == 1
+        if not (len(layers) == 2 and layers[1].weight.shape[0] == 1
                 and all(l.bias is not None for l in layers)
                 and fused.tc5_ms_prop_supported(grid, layers[0].weight.shape[0], f0._precision)):
             return None

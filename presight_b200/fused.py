@@ -13,7 +13,6 @@ written straight into the matching windows of one `dh` buffer (the appearance gr
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
@@ -24,10 +23,7 @@ from . import ops
 from ._lib import call, host_floats, host_ints, host_ptrs, host_segments, ptr, stream
 
 _f32c = ops._f32c
-# PS_TC5_FIELD=0 keeps the final level on the chain of stand-alone kernels (hash / 3 MLPs / compositing)
-USE_TC5_FIELD = os.environ.get("PS_TC5_FIELD", "1") == "1"
-USE_TC5_PROP = os.environ.get("PS_TC5_PROP", "1") == "1"
-OVERLAP_PROP_BWD = os.environ.get("PS_OVERLAP_PROP_BWD", "1") == "1"
+OVERLAP_PROP_BWD = True
 
 
 def set_overlap_prop_bwd(on: bool) -> bool:
@@ -38,21 +34,17 @@ def set_overlap_prop_bwd(on: bool) -> bool:
     global OVERLAP_PROP_BWD
     prev, OVERLAP_PROP_BWD = OVERLAP_PROP_BWD, bool(on)
     return prev
-FIELD_CHUNKS = max(1, int(os.environ.get("PS_FIELD_CHUNKS", "1")))
 
 # Partial-gradient sinks (data-parallel training, presight_b200/parallel.py): the main hash table is ONE parameter of 512 MiB
 # whose gradient is complete only when the last level has been scattered — the last kernel of the backward.  A sink registered
 # for the table receives every level group's rows as soon as that group's scatter has been launched (called with the scatter's
 # stream current, so a collective issued inside it is ordered behind exactly that kernel) and can start reducing them while
 # the remaining levels and the proposal networks are still being differentiated.
-# device index -> [event recorded behind the step's (last) field backward kernel, proposal backwards launched since]
-# (autograd runs the field level's backward first).  PS_PROP_BWD_ORDER: "second" = the first proposal backward of a step starts
-# at once, later ones wait for the field kernel; "all" = all wait; "before" = they wait for the point where the field kernel
-# becomes launchable (and so queue behind it without waiting for its end); "free" = no ordering (which of two kernels
-# launched microseconds apart on different streams gets the SMs first is then a race).
+# device index -> [event recorded where the step's field backward kernel becomes launchable, proposal backwards launched
+# since] (autograd runs the field level's backward first).  The first proposal backward of a step starts at once; later ones
+# wait for that event, so they queue behind the field kernel without waiting for its end (two kernels launched microseconds
+# apart on different streams would otherwise race for the SMs).
 _FIELD_BWD_ORDER = {}
-PROP_BWD_ORDER = os.environ.get("PS_PROP_BWD_ORDER", "before")
-PROP_BWD_PRIO = os.environ.get("PS_PROP_BWD_PRIO", "0") == "1"      # proposal backwards on a high-priority stream
 
 _PARTIAL_SINKS = {}          # table.data_ptr() -> (callable(dtable, row_lo, row_hi), level groups [(l0, l1), ...], alloc)
 
@@ -98,7 +90,7 @@ class MlpMeta:
 def _mlp_fwd(segs, P, ws, bs, meta: MlpMeta, prec, y, sel=None, density_out=None, name="mlp"):
     with ops._probe(f"mlp_fwd_{name}"):
         call("ps_mlp_fwd_ex", host_segments(segs), len(segs), P, host_ptrs(ws), host_ptrs(bs), host_ints(meta.dims),
-             meta.n_layers, meta.out_act, ops.fwd_precision(prec), ptr(y), ptr(sel), ptr(density_out), stream())
+             meta.n_layers, meta.out_act, prec, ptr(y), ptr(sel), ptr(density_out), stream())
 
 
 def _mlp_bwd(segs, dy, P, ws, bs, meta: MlpMeta, prec, dW, db, sel=None, d_density=None, name="mlp"):
@@ -117,13 +109,14 @@ def _ray_points(origins, dirs, eu, aabb, contract):
     return x01, sel
 
 
-def _hash_fwd(x01, table, g: GridMeta):
-    """-> features as a flat tensor of P*L*F floats: level-major [L][P][F] (ps_hash_fwd_lm) when `g.level_major`,
-    else the reference's row-major [P][L*F]."""
+def _hash_fwd(x01, table, g: GridMeta, level_major: Optional[bool] = None):
+    """-> features as a flat tensor of P*L*F floats: level-major [L][P][F] (ps_hash_fwd_lm) when `level_major`
+    (default `g.level_major`; the fused field kernels read only this layout), else the reference's row-major [P][L*F]."""
+    lm = g.level_major if level_major is None else level_major
     P = x01.shape[0]
     out = torch.empty(P * g.L * g.F, device=x01.device, dtype=torch.float32)
     with ops._probe(f"hash_fwd_L{g.L}F{g.F}T{g.log2_T}"):
-        call("ps_hash_fwd_lm" if g.level_major else "ps_hash_fwd", ptr(x01), P, ptr(table), host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(out), stream())
+        call("ps_hash_fwd_lm" if lm else "ps_hash_fwd", ptr(x01), P, ptr(table), host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(out), stream())
     return out
 
 
@@ -132,10 +125,12 @@ def _feat_seg(feat, dfeat, g: GridMeta):
     return (feat, dfeat, g.L * g.F, 0, g.L * g.F, 1, g.F if g.level_major else 0)
 
 
-def _hash_bwd(x01, dfeat, table, g: GridMeta):
+def _hash_bwd(x01, dfeat, table, g: GridMeta, level_major: Optional[bool] = None):
+    """-> the table gradient of features `dfeat` laid out as `_hash_fwd` writes them."""
+    lm = g.level_major if level_major is None else level_major
     dtable = torch.zeros_like(table)
     with ops._probe(f"hash_bwd_L{g.L}F{g.F}T{g.log2_T}"):
-        call("ps_hash_bwd_lm" if g.level_major else "ps_hash_bwd", ptr(x01), x01.shape[0], None, host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(dfeat),
+        call("ps_hash_bwd_lm" if lm else "ps_hash_bwd", ptr(x01), x01.shape[0], None, host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(dfeat),
              ptr(dtable), None, stream())
     return dtable
 
@@ -229,18 +224,17 @@ class _PropLevelTc5(torch.autograd.Function):
         # the producer of `dw` published its completion event, run this backward on a side stream so that it overlaps
         # the field kernels / main hash scatter already queued on the main stream.
         ev_in = ops.pop_grad_event(dw, ctx.grad_key) if OVERLAP_PROP_BWD else None
-        run_on = ops.side_stream(eu.device, 1, high_priority=PROP_BWD_PRIO) if ev_in is not None else main
+        run_on = ops.side_stream(eu.device) if ev_in is not None else main
         with torch.cuda.stream(run_on):
             if ev_in is not None:
                 run_on.wait_event(ev_in)
-                # Order against the final level's backward (see _FIELD_BWD_ORDER): a proposal backward that autograd runs
-                # before the field level's (it finds the SMs idle while the main stream is still busy with the loss
-                # gradients) starts at once; one that comes after it starts when the field kernel — which needs whole SMs
-                # and all of tensor memory, so cannot share them with this kernel's persistent CTAs — has finished, and then
-                # co-runs with the main hash scatter.
+                # Order against the final level's backward (see _FIELD_BWD_ORDER): the first proposal backward since then
+                # starts at once; a later one queues behind the field kernel — which needs whole SMs and all of tensor
+                # memory, so cannot share them with this kernel's persistent CTAs — and co-runs with the main hash
+                # scatter once the field kernel retires.
                 order = _FIELD_BWD_ORDER.get(eu.device.index)
-                if order is not None and PROP_BWD_ORDER != "free":
-                    if order[1] >= 1 or PROP_BWD_ORDER == "all":
+                if order is not None:
+                    if order[1] >= 1:
                         run_on.wait_event(order[0])
                     order[1] += 1
             dwc = _f32c(dw).view(N, S)
@@ -267,7 +261,7 @@ class _PropLevelTc5(torch.autograd.Function):
 
 def prop_level_weights(origins, dirs, eu_bins, table, aabb, contract, grid: GridMeta, net: MlpMeta, prec,
                        weights: Sequence[Tensor], biases: Sequence[Tensor]) -> Tensor:
-    if USE_TC5_PROP and tc5_prop_supported(grid, net, prec, eu_bins.shape[1] - 1) and all(b is not None for b in biases):
+    if tc5_prop_supported(grid, net, prec, eu_bins.shape[1] - 1) and all(b is not None for b in biases):
         # hand-off key: a loss that consumes this tensor publishes its gradient's completion event under it (ops.py)
         key = ops.new_grad_key() if (OVERLAP_PROP_BWD and torch.is_grad_enabled()) else None
         out = _PropLevelTc5.apply(origins, dirs, eu_bins, table, aabb, contract, grid, key, weights[0], biases[0],
@@ -403,22 +397,6 @@ def tc5_field_supported(grid: GridMeta, base: MlpMeta, sem: Optional[MlpMeta], r
             and base.out_act == ops.ACT_NONE and sem.out_act == ops.ACT_NONE)
 
 
-def _hash_fwd_lm(x01, table, g: GridMeta):
-    P = x01.shape[0]
-    out = torch.empty(P * g.L * g.F, device=x01.device, dtype=torch.float32)
-    with ops._probe(f"hash_fwd_L{g.L}F{g.F}T{g.log2_T}"):
-        call("ps_hash_fwd_lm", ptr(x01), P, ptr(table), host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(out), stream())
-    return out
-
-
-def _hash_bwd_lm(x01, dfeat, table, g: GridMeta):
-    dtable = torch.zeros_like(table)
-    with ops._probe(f"hash_bwd_L{g.L}F{g.F}T{g.log2_T}"):
-        call("ps_hash_bwd_lm", ptr(x01), x01.shape[0], None, host_floats(g.scalings), g.L, g.F, g.log2_T, ptr(dfeat),
-             ptr(dtable), None, stream())
-    return dtable
-
-
 def tc5_field_forward(o, d, eu, app_c, table, aabb, contract, grid: GridMeta, ws, bs, A, threshold):
     """-> (x01, sel, feat, w [N,S], rgb [N,3], acc [N,1], dexp [N,1], dthr [N,1], sem [N,64], tmm [2])."""
     from ._lib import host_field_net
@@ -426,7 +404,6 @@ def tc5_field_forward(o, d, eu, app_c, table, aabb, contract, grid: GridMeta, ws
     N, S = eu.shape[0], eu.shape[1] - 1
     dev = eu.device
     x01, sel = _ray_points(o, d, eu, aabb, contract)
-    feat = _hash_fwd_lm(x01, table, grid)
     w = torch.empty(N, S, device=dev, dtype=torch.float32)
     rgb_out = torch.empty(N, 3, device=dev, dtype=torch.float32)
     acc = torch.empty(N, 1, device=dev, dtype=torch.float32)
@@ -435,6 +412,7 @@ def tc5_field_forward(o, d, eu, app_c, table, aabb, contract, grid: GridMeta, ws
     sem_out = torch.empty(N, 64, device=dev, dtype=torch.float32)
     tmm = ops.new_tminmax(dev)
     net = host_field_net(ws, bs, A)
+    feat = _hash_fwd(x01, table, grid, level_major=True)
     with ops._probe("field_level_fwd"):
         call("ps_field_level_fwd", C.byref(net), ptr(feat), grid.L, grid.F, ptr(sel), ptr(eu), ptr(d), ptr(app_c), N, S,
              float(threshold), ptr(w), ptr(rgb_out), ptr(acc), ptr(dexp), ptr(dthr), ptr(sem_out), ptr(tmm), stream())
@@ -445,62 +423,32 @@ _zeros_like_many = ops.zeros_like_many
 
 
 def _chunk_bounds(N: int, S: int) -> List[Tuple[int, int]]:
-    """Ray ranges of the software pipeline between the hash kernels and the field kernels: FIELD_CHUNKS equal slices
-    (multiples of 128 rays) for large batches, one slice otherwise."""
-    k = FIELD_CHUNKS if N * S >= (1 << 21) else 1
-    step = ((N + k - 1) // k + 127) // 128 * 128
-    return [(c0, min(c0 + step, N)) for c0 in range(0, N, step)]
+    """Ray ranges of the final level's hash and field kernels: the whole batch, one range.  bench.py's timing of the
+    main-grid scatter alone reads it, so that the scatter is launched over the same ranges as in the step."""
+    return [(0, N)]
 
 
 class _FieldLevelTc5(torch.autograd.Function):
     """Final level on the fused tcgen05 kernels: ray_points -> hash gather -> ONE field+compositing kernel; backward =
     ONE kernel (recompute + all gradients) -> hash scatter.  Saved for backward: bins, unit-cube points, selector and
-    the hash features only.
-
-    The hash kernels (bound by L2 gather / atomic throughput, few registers, no shared memory) and the field kernels
-    (bound by the latency of their GEMM -> epilogue chain, one CTA per SM) use disjoint resources, so the batch is cut
-    into ray slices and in the backward the two kernel families run as a two-stage pipeline on two streams: the scatter
-    of slice c overlaps the field backward of slice c+1 (tools/overlap_probe.py: 2.66 ms -> 2.01 ms for 32k rays)."""
+    the hash features only."""
 
     @staticmethod
     def forward(ctx, origins, dirs, eu_bins, app, table, aabb, contract, grid: GridMeta, threshold, *params):
-        import ctypes as C
-        from ._lib import host_field_net
         o, d, eu = _f32c(origins.detach()), _f32c(dirs.detach()), _f32c(eu_bins.detach())
         N, S = eu.shape[0], eu.shape[1] - 1
-        dev = eu.device
         ws = [p.detach() for p in params[:8]]
         bs = [p.detach() for p in params[8:]]
         A = 0 if app is None else app.shape[1]
         app_c = None if app is None else _f32c(app.detach())
-        tab = table.detach()
-        x01, sel = _ray_points(o, d, eu, aabb, contract)
-        w = torch.empty(N, S, device=dev, dtype=torch.float32)
-        rgb_out = torch.empty(N, 3, device=dev, dtype=torch.float32)
-        acc = torch.empty(N, 1, device=dev, dtype=torch.float32)
-        dexp = torch.empty(N, 1, device=dev, dtype=torch.float32)
-        dthr = torch.empty(N, 1, device=dev, dtype=torch.float32)
-        sem_out = torch.empty(N, 64, device=dev, dtype=torch.float32)
-        tmm = ops.new_tminmax(dev)
-        net = host_field_net(ws, bs, A)
-        bounds = _chunk_bounds(N, S)
-        feats = []
-        for (c0, c1) in bounds:
-            # (forward: the gather wants the L1 carve-out, the field kernel the shared-memory one — the two do not
-            # co-run, measured with tools/overlap_probe.py — so the slices simply alternate on one stream)
-            f = _hash_fwd_lm(x01[c0 * S:c1 * S], tab, grid)
-            feats.append(f)
-            with ops._probe("field_level_fwd"):
-                call("ps_field_level_fwd", C.byref(net), ptr(f), grid.L, grid.F, ptr(sel[c0 * S:c1 * S]),
-                     ptr(eu[c0:c1]), ptr(d[c0:c1]), None if app_c is None else ptr(app_c[c0:c1]), c1 - c0, S,
-                     float(threshold), ptr(w[c0:c1]), ptr(rgb_out[c0:c1]), ptr(acc[c0:c1]), ptr(dexp[c0:c1]),
-                     ptr(dthr[c0:c1]), ptr(sem_out[c0:c1]), ptr(tmm), stream())
-        saved = [eu, d, x01, sel, acc, dexp, table]
+        x01, sel, feat, w, rgb_out, acc, dexp, dthr, sem_out, tmm = tc5_field_forward(
+            o, d, eu, app_c, table.detach(), aabb, contract, grid, ws, bs, A, threshold)
+        saved = [eu, d, x01, sel, feat, acc, dexp, table]
         if app_c is not None:
             saved.append(app_c)
         ctx.n_fixed = len(saved)
-        ctx.save_for_backward(*saved, *feats, *params)
-        ctx.meta = (grid, N, S, A, bounds, app is not None and app.requires_grad)
+        ctx.save_for_backward(*saved, *params)
+        ctx.meta = (grid, N, S, A, app is not None and app.requires_grad)
         ctx.mark_non_differentiable(dthr, tmm)
         ctx.set_materialize_grads(False)
         return w.view(N, S, 1), rgb_out, acc, dexp, dthr, sem_out, tmm
@@ -509,13 +457,11 @@ class _FieldLevelTc5(torch.autograd.Function):
     def backward(ctx, dw, drgb, dacc, ddexp, _dthr, dsem, _dtmm):
         import ctypes as C
         from ._lib import host_field_net
-        grid, N, S, A, bounds, app_grad = ctx.meta
+        grid, N, S, A, app_grad = ctx.meta
         saved = list(ctx.saved_tensors)
-        nf, nc = ctx.n_fixed, len(bounds)
-        eu, d, x01, sel, acc, dexp, table = saved[:7]
-        app_c = saved[7] if A else None
-        feats = saved[nf:nf + nc]
-        params = saved[nf + nc:]
+        eu, d, x01, sel, feat, acc, dexp, table = saved[:8]
+        app_c = saved[8] if A else None
+        params = saved[ctx.n_fixed:]
         dev = eu.device
         ws = [p.detach() for p in params[:8]]
         bs = [p.detach() for p in params[8:]]
@@ -531,58 +477,27 @@ class _FieldLevelTc5(torch.autograd.Function):
             return t if shape is None else t.view(shape)
         dwc, drgbc, daccc, ddexpc, dsemc = opt(dw, (N, S)), opt(drgb), opt(dacc), opt(ddexp), opt(dsem)
 
-        def sl(t, c0, c1):
-            return None if t is None else ptr(t[c0:c1])
-        main = torch.cuda.current_stream()
-        piped = nc > 1
-        side = ops.side_stream(dev, 0) if piped else main
-        if piped:
-            side.wait_stream(main)                    # fork (also what makes the side stream part of a graph capture)
-        sink = _PARTIAL_SINKS.get(table.data_ptr()) if nc == 1 else None
-        with torch.cuda.stream(side):
-            # (the 512 MiB memset runs under the first field slice)
-            dtable = sink[2]() if (sink is not None and sink[2] is not None) else torch.zeros_like(table)
-        keep = []            # main-stream buffers read on the side stream: alive until the join below
-        ev_ready = None
-        if PROP_BWD_ORDER == "before":
-            # recorded where the field kernel's inputs are complete: a proposal backward launched later this step waits for it,
-            # i.e. it cannot reach the GPU before the field kernel is launchable and queues behind it
-            ev_ready = torch.cuda.Event()
-            ev_ready.record(main)
-        for i, (c0, c1) in enumerate(bounds):
-            dfeat = torch.empty_like(feats[i])
-            keep.append(dfeat)
-            with ops._probe("field_level_bwd"):
-                call("ps_field_level_bwd", C.byref(net), ptr(feats[i]), grid.L, grid.F, ptr(sel[c0 * S:c1 * S]),
-                     ptr(eu[c0:c1]), ptr(d[c0:c1]), None if app_c is None else ptr(app_c[c0:c1]), c1 - c0, S,
-                     ptr(acc[c0:c1]), ptr(dexp[c0:c1]), sl(dwc, c0, c1), sl(drgbc, c0, c1), sl(daccc, c0, c1),
-                     sl(ddexpc, c0, c1), sl(dsemc, c0, c1), ptr(dfeat), sl(dapp, c0, c1), stream())
-            if piped or i == nc - 1:
-                ev = torch.cuda.Event()
-                ev.record(main)
-                if piped:
-                    side.wait_event(ev)
-                if i == nc - 1:
-                    # [field backward done (or, "before": launchable), proposal backwards launched since]
-                    _FIELD_BWD_ORDER[dev.index] = [ev if ev_ready is None else ev_ready, 0]
-            with torch.cuda.stream(side):
-                if sink is None:
-                    with ops._probe(f"hash_bwd_L{grid.L}F{grid.F}T{grid.log2_T}"):
-                        call("ps_hash_bwd_lm", ptr(x01[c0 * S:c1 * S]), (c1 - c0) * S, None, host_floats(grid.scalings),
-                             grid.L, grid.F, grid.log2_T, ptr(dfeat), ptr(dtable), None, side.cuda_stream)
-                else:
-                    # one scatter per level group (the kernel is level-major anyway), each handed to the sink at once
-                    fn, groups = sink[0], sink[1]
-                    T, Pc = 1 << grid.log2_T, (c1 - c0) * S
-                    dfl, dtl = dfeat.view(grid.L, Pc * grid.F), dtable.view(grid.L, T * grid.F)
-                    for (l0, l1) in groups:
-                        with ops._probe(f"hash_bwd_L{grid.L}F{grid.F}T{grid.log2_T}"):
-                            call("ps_hash_bwd_lm", ptr(x01[c0 * S:c1 * S]), Pc, None, host_floats(grid.scalings[l0:l1]),
-                                 l1 - l0, grid.F, grid.log2_T, ptr(dfl[l0:l1]), ptr(dtl[l0:l1]), None, side.cuda_stream)
-                        fn(dtable, l0 * T, l1 * T)
-        if piped:
-            main.wait_stream(side)   # join (see _PropLevelTc5.backward for why no record_stream is needed)
-        del keep
+        sink = _PARTIAL_SINKS.get(table.data_ptr())
+        dtable = sink[2]() if (sink is not None and sink[2] is not None) else torch.zeros_like(table)
+        # recorded where the field kernel's inputs are complete: a proposal backward launched later this step waits for it,
+        # i.e. it cannot reach the GPU before the field kernel is launchable and queues behind it
+        ev_ready = torch.cuda.Event()
+        ev_ready.record()
+        dfeat = torch.empty_like(feat)
+        with ops._probe("field_level_bwd"):
+            call("ps_field_level_bwd", C.byref(net), ptr(feat), grid.L, grid.F, ptr(sel), ptr(eu), ptr(d), ptr(app_c), N, S,
+                 ptr(acc), ptr(dexp), ptr(dwc), ptr(drgbc), ptr(daccc), ptr(ddexpc), ptr(dsemc), ptr(dfeat), ptr(dapp),
+                 stream())
+        _FIELD_BWD_ORDER[dev.index] = [ev_ready, 0]      # [field kernel launchable, proposal backwards launched since]
+        # with a sink: one scatter per level group (the kernel is level-major anyway), each handed to the sink at once
+        T, P = 1 << grid.log2_T, N * S
+        dfl, dtl = dfeat.view(grid.L, P * grid.F), dtable.view(grid.L, T * grid.F)
+        for (l0, l1) in (sink[1] if sink is not None else [(0, grid.L)]):
+            with ops._probe(f"hash_bwd_L{grid.L}F{grid.F}T{grid.log2_T}"):
+                call("ps_hash_bwd_lm", ptr(x01), P, None, host_floats(grid.scalings[l0:l1]), l1 - l0, grid.F, grid.log2_T,
+                     ptr(dfl[l0:l1]), ptr(dtl[l0:l1]), None, stream())
+            if sink is not None:
+                sink[0](dtable, l0 * T, l1 * T)
         return (None, None, None, dapp, dtable, None, None, None, None, *dW, *dB)
 
 
@@ -592,7 +507,7 @@ def field_level(origins, dirs, eu_bins, app, table, aabb, contract, grid: GridMe
     """-> (weights [N,S,1], rgb [N,3], acc [N,1], depth_expected_unclipped [N,1], depth_threshold [N,1],
     semantics [N,C], tminmax [2]).  *_params = (weights list, biases list)."""
     A = 0 if app is None else app.shape[1]
-    if USE_TC5_FIELD and tc5_field_supported(grid, base, sem, rgb, geo_dim, prec, eu_bins.shape[1] - 1, A):
+    if tc5_field_supported(grid, base, sem, rgb, geo_dim, prec, eu_bins.shape[1] - 1, A):
         ws = [*base_params[0], *sem_params[0], *rgb_params[0]]
         bs = [*base_params[1], *sem_params[1], *rgb_params[1]]
         return _FieldLevelTc5.apply(origins, dirs, eu_bins, app, table, aabb, contract, grid, threshold, *ws, *bs)

@@ -6,7 +6,6 @@ There is no CPU / PyTorch fallback.
 """
 from __future__ import annotations
 
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -16,16 +15,7 @@ from . import _lib
 from ._lib import call, host_floats, host_ints, host_ptrs, ptr, stream
 
 ACT_NONE, ACT_RELU, ACT_SIGMOID = 0, 1, 2
-PREC_TF32X3, PREC_BF16, PREC_BF16_TCGEN05 = 0, 1, 2
-# PS_TCGEN05_FWD=1 routes bf16 forward passes through the tcgen05 / TMEM kernel (csrc/mlp_tc5.cu).  It is correct
-# (tests/test_gpu_kernels.py::test_mlp_tcgen05_forward) but, un-pipelined as it is, 0.7 ms/step slower than the
-# register-chained mma.sync kernel on C2 (profiles/r1_d_*), so it is opt-in for now.
-TCGEN05_FWD = os.environ.get("PS_TCGEN05_FWD", "0") == "1"
-
-
-def fwd_precision(precision: int) -> int:
-    return PREC_BF16_TCGEN05 if (precision == PREC_BF16 and TCGEN05_FWD) else precision
-
+PREC_TF32X3, PREC_BF16 = 0, 1
 
 
 class KernelProbe:
@@ -204,7 +194,7 @@ class _Mlp(torch.autograd.Function):
         bd = [None if b is None else b.detach().contiguous() for b in bs]
         with _probe("mlp_fwd_" + "x".join(map(str, dims))):
             call("ps_mlp_fwd", ptr(x2), x2.shape[0], host_ptrs(wd), host_ptrs(bd), host_ints(dims), n_layers, out_act,
-                 fwd_precision(precision), ptr(y), stream())
+                 precision, ptr(y), stream())
         ctx.save_for_backward(x2, *wd, *[b for b in bd if b is not None])
         ctx.meta = (out_act, precision, n_layers, dims, [b is not None for b in bd], x.shape)
         return y.view(*lead, dims[-1])
@@ -245,7 +235,7 @@ class _MlpSelect(torch.autograd.Function):
         hd, st = host_ints(dims), stream()
         with _probe("mlp_fwd_" + "x".join(map(str, dims))):
             for k, (ws, bs) in enumerate(nets):
-                call("ps_mlp_fwd", ptr(x2), N, host_ptrs(ws), host_ptrs(bs), hd, n_layers, out_act, fwd_precision(precision),
+                call("ps_mlp_fwd", ptr(x2), N, host_ptrs(ws), host_ptrs(bs), hd, n_layers, out_act, precision,
                      ptr(Y[k]), st)
         idx = sf.view(1, N, 1).expand(1, N, dims[-1])
         y = Y.gather(0, idx).squeeze(0)
@@ -530,13 +520,11 @@ def pop_grad_event(t: Tensor, key):
 _SIDE_STREAMS = {}
 
 
-def side_stream(device, idx: int = 0, high_priority: bool = False) -> "torch.cuda.Stream":
-    """Cached side streams.  `high_priority` (honoured when the stream is first created): among kernels that become runnable
-    at the same moment the block scheduler serves the older launch first and a later one only gets what is left — a kernel
-    meant to co-run from the start has to outrank the one launched before it."""
-    key = (torch.device(device).index, idx)
+def side_stream(device) -> "torch.cuda.Stream":
+    """The device's cached side stream (created on first use)."""
+    key = torch.device(device).index
     if key not in _SIDE_STREAMS:
-        _SIDE_STREAMS[key] = torch.cuda.Stream(device=device, priority=-1 if high_priority else 0)
+        _SIDE_STREAMS[key] = torch.cuda.Stream(device=device)
     return _SIDE_STREAMS[key]
 
 

@@ -141,7 +141,7 @@ def test_fused_matches_oracle_fp32():
                   props[1][0].net.weights[0].grad) < 5e-3
 
 
-def test_tc5_model_matches_oracle_bf16():
+def test_fused_model_matches_oracle_bf16():
     """The default path — both proposal levels and the final level on the fused tcgen05 kernels — against the CPU
     oracle on the same weights and jitters: 1e-2 (bf16 parity class) on every output, gradients by rel-L2."""
     from presight_b200 import fused
@@ -160,7 +160,7 @@ def test_tc5_model_matches_oracle_bf16():
     sky = [OS.sky_from_state(sd, "sky_model.fields.0.", True, True)]
     # the fused kernels must actually be the ones that ran
     f0, p0 = model.field.fields[0], model.proposal_networks[0].fields[0]
-    assert fused.USE_TC5_FIELD and fused.USE_TC5_PROP
+    assert model.field.supports_fused() and all(p.supports_fused() for p in model.proposal_networks)
     assert f0.mlp_base_mlp.layers[0].weight.shape[1] <= 48 and p0.encoding.features_per_level in (1, 2)
     ocfg = O.ModelCfg(num_proposal_samples=(64, 32), num_nerf_samples=32, near=NEAR, far=FAR, piecewise_thr=THR)
     om = O.Model(ocfg, torch.zeros(1, 3), [field], props, sky)

@@ -379,31 +379,6 @@ def test_composite_long_rays_against_oracle(ops):
         assert float(acc.max()) <= 1.0 + 1e-5       # sum of weights never exceeds 1
 
 
-@pytest.mark.parametrize("shape", SHAPES)
-def test_mlp_tcgen05_forward(ops, shape):
-    """precision 2 = tcgen05.mma + TMEM forward: agrees with the mma.sync bf16 kernel to fp32 summation order (values
-    on a bf16 rounding boundary may flip, hence 3e-3) and with the fp32 oracle to the bf16 class (1e-2)."""
-    n_in, hidden, n_layers, n_out, act = shape
-    g = torch.Generator().manual_seed(n_in * 131 + n_out)
-    ws, bs = _make_mlp(g, n_in, hidden, n_layers, n_out)
-    for P in (1, 777, 128 * 600 + 3):
-        x = torch.randn(P, n_in, generator=g)
-        wg, bg = [w.to(DEV) for w in ws], [b.to(DEV) for b in bs]
-        y_tc5 = ops.mlp(x.to(DEV), wg, bg, act, 2)
-        y32 = O.mlp_forward(x, O.Mlp(ws, bs, "sigmoid" if act == 2 else None))
-        y16 = O.mlp_forward_bf16_emulated(x, O.Mlp(ws, bs, "sigmoid" if act == 2 else None))
-        assert_close(y_tc5.cpu(), y16, 3e-3, f"tcgen05 vs bf16 emulation P={P}")
-        if P >= 100:      # a single bf16-MLP output can be >1 % off; the 1e-2 class is a statement about batches
-            assert_close(y_tc5.cpu(), y32, TOL16, f"tcgen05 vs fp32 oracle P={P}")
-        old = ops.TCGEN05_FWD
-        try:
-            ops.TCGEN05_FWD = False
-            y_sync = ops.mlp(x.to(DEV), wg, bg, act, 1)
-        finally:
-            ops.TCGEN05_FWD = old
-        assert_close(y_tc5, y_sync, 3e-3, f"tcgen05 vs mma.sync P={P}")
-
-
 # ------------------------------------------------------------------------------------------ loss stack (8f-1)
 @pytest.mark.parametrize("case", ["a", "b", "c"])
 def test_interlevel_loss_kernel_golden(ops, case):

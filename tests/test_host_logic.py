@@ -17,16 +17,9 @@ def test_algorithmic_bytes_match_survey():
     assert synthetic.step_bytes_per_ray(c1, False) == 291840 and synthetic.step_bytes_per_ray(c2, False) == 272128
 
 
-def test_chunk_bounds_cover_the_batch_in_multiples_of_128():
+def test_chunk_bounds_are_the_whole_batch():
     for n, s in [(65536, 64), (65536, 128), (21846, 64), (100, 64), (40000, 64), (32768 + 5, 96)]:
-        b = fused._chunk_bounds(n, s)
-        assert b[0][0] == 0 and b[-1][1] == n
-        for (a0, a1), (b0, _) in zip(b, b[1:]):
-            assert a1 == b0 and (a1 - a0) % 128 == 0 and a1 > a0
-        if n * s < (1 << 21):
-            assert len(b) == 1                      # small batches are not sliced
-        else:
-            assert len(b) <= fused.FIELD_CHUNKS
+        assert fused._chunk_bounds(n, s) == [(0, n)]            # the final level is never sliced
 
 
 def test_fused_kernel_eligibility():
@@ -37,7 +30,7 @@ def test_fused_kernel_eligibility():
     ok = dict(grid=g_main, base=base, sem=sem, rgb=rgb, geo_dim=15, prec=ops.PREC_BF16, S=64, A=16)
     assert fused.tc5_field_supported(**ok)
     assert not fused.tc5_field_supported(**{**ok, "S": 48})                      # C1's final level
-    assert not fused.tc5_field_supported(**{**ok, "prec": ops.PREC_BF16 + 1})    # fp32 class -> stand-alone kernels
+    assert not fused.tc5_field_supported(**{**ok, "prec": ops.PREC_TF32X3})      # fp32 class -> stand-alone kernels
     assert not fused.tc5_field_supported(**{**ok, "sem": None})
     assert not fused.tc5_field_supported(**{**ok, "A": 32, "rgb": fused.MlpMeta((63, 64, 64, 3), ops.ACT_SIGMOID)})
     g_prop = fused.GridMeta(tuple(float(i) for i in range(8)), 20, 1)

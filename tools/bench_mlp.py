@@ -16,7 +16,7 @@ def timeit(fn, iters=5):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--points", type=int, default=65536 * 64)
-    ap.add_argument("--precs", default="1,2")
+    ap.add_argument("--precs", default="0,1")
     ap.add_argument("--bwd", action="store_true")
     args = ap.parse_args()
     P = args.points

@@ -24,7 +24,7 @@ for dd in dims:
 eu = (torch.rand(n, S + 1, generator=g) * (40.0 / S) + 0.001).cumsum(-1).to(dev)
 app = torch.randn(n, A, generator=g).to(dev)
 x01, sel = fused._ray_points(o, d, eu, aabb, True)
-feat = fused._hash_fwd_lm(x01, table, grid)
+feat = fused._hash_fwd(x01, table, grid, level_major=True)
 P = n * S
 w = torch.empty(n, S, device=dev); rgb = torch.empty(n, 3, device=dev); acc = torch.empty(n, 1, device=dev)
 dexp = torch.empty(n, 1, device=dev); dthr = torch.empty(n, 1, device=dev); sem = torch.empty(n, 64, device=dev)
